@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- full-grid delay-and-sum power maps per second on B200 (BASELINE.json's metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--config cfg3] [--frames B] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--config cfg3] [--frames B] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of B synthetic frames (C channels x (B+3)*N samples, larger than
 L2) for every direction of the grid.  N = 1 runs the configuration the target is quoted on (cfg3: 512 microphones x
@@ -27,6 +27,11 @@ kernel against the FP32-FMA roofline (nominal, and against an in-job packed-FMA 
 the measured copy bandwidth.  `sustained`: >= 2 s of back-to-back steps with clocks and board power.  `other_configs`:
 cfg1 / cfg2 / cfg5 (and cfg4 MISO latency) in the same run.  `cpu_baseline`: the compiled reference delay() loop
 (oracle/_ref) on the host.  --config cfg4 benchmarks the dynamic-steering (MISO) path on its own.
+
+--dump-outputs DIR writes what the timed path delivered in its last timed step (power-map configurations: the [B][D]
+maps as DIR/power_maps.npy; cfg4: DIR/audio.npy and DIR/power.npy) so that two builds can be compared output for output:
+the input is synthesised from a fixed seed, so the same arguments give the same input on every run.  The benchmark
+writes nothing into the source tree (it may be read-only); DIR is the caller's.
 """
 import argparse
 import json
@@ -36,6 +41,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True      # no __pycache__ in the source tree
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (ROOT, os.path.join(ROOT, "beamforming-lk_b200"), os.path.join(ROOT, "tests")):
     if p not in sys.path:
@@ -66,7 +72,14 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip bit_identical / sustained / other_configs / latency / grid_shard")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step delivered as DIR/<name>.npy (float32, at most 64 MB in all)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs is defined for --impl ours")
+    return args
 
 
 def default_frames(c):
@@ -95,6 +108,23 @@ def workload(c, name, B):
 
 def flops_per_map(C, D, N):
     return D * N * (4 * C + 6)          # SURVEY.md 8d: 4 FLOP per (dir, ch, sample) + 6 per (dir, sample)
+
+
+DUMP_BYTES = 60_000_000      # stays under 64 MB with the .npy headers
+
+
+def dump_outputs(path, **arrays):
+    """--dump-outputs: each array (a torch tensor [rows][...] on the device) as path/<name>.npy in float32.  When the arrays
+    together exceed DUMP_BYTES, each keeps a fixed, seeded, sorted sample of its rows (frames)."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    total = sum(a.numel() * 4 for a in arrays.values())
+    for name, a in arrays.items():
+        if total > DUMP_BYTES:
+            keep = max(1, int(a.shape[0] * DUMP_BYTES / total))
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))
+            a = a.index_select(0, torch.from_numpy(rows).to(a.device))
+        np.save(os.path.join(path, f"{name}.npy"), a.float().cpu().numpy())
 
 
 def peaks():
@@ -336,10 +366,11 @@ def small_config_run(bflk, torch, name, dev, local, steps=8, warmup=3, kernel=0)
     return res
 
 
-def miso_bench(bflk, torch, dev, local, calls=300):
+def miso_bench(bflk, torch, dev, local, calls=300, steps=None, warmup=20, dump=None):
     """cfg4: 16 tracked targets x 512 microphones, enhanced audio + beam power per frame.  Latency of the host call on a
-    window kept on the device (what a tracker iterating on one frame pays), of the call that uploads the frame first, and
-    the device-side throughput of back-to-back asynchronous calls."""
+    window kept on the device (what a tracker iterating on one frame pays) and of the call that uploads the frame first,
+    sampled over `calls` calls each; the device-side throughput of `steps` (default `calls`) timed back-to-back
+    asynchronous calls after `warmup` untimed ones (the last call's audio and power go to `dump`, if given)."""
     import ctypes as C
     from bflk import synth
     c = cases.CFG4
@@ -376,16 +407,19 @@ def miso_bench(bflk, torch, dev, local, calls=300):
         rc = m._L.bflk_miso_dev(m._h, tt.ctypes.data_as(C.c_void_p), pp.ctypes.data_as(C.c_void_p), T, C.c_void_p(wd.data_ptr()),
                                 C.c_void_p(audio.data_ptr()), C.c_void_p(power.data_ptr()), C.c_void_p(st.cuda_stream))
         assert rc == 0
-    for _ in range(20):
+    steps = steps or calls
+    for _ in range(warmup):
         call()
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record(st)
-    for _ in range(calls):
+    for _ in range(steps):
         call()
     e1.record(st)
     torch.cuda.synchronize()
-    us = e0.elapsed_time(e1) * 1e3 / calls
+    us = e0.elapsed_time(e1) * 1e3 / steps
+    if dump:
+        dump_outputs(dump, audio=audio, power=power)
     flop = T * N * 4 * Cn
     # CPU: Particle::das + beam for the same targets = the reference delay() loop over T directions
     cpu = None
@@ -458,11 +492,13 @@ def run_miso_only(args):
     dev = torch.device("cuda", local)
     with ClockSampler(local) as clk:
         clk.begin()
-        r = miso_bench(bflk, torch, dev, local, calls=max(100, args.steps))
+        # latency percentiles want at least 100 samples; the timed throughput region runs exactly --steps calls
+        r = miso_bench(bflk, torch, dev, local, calls=max(100, args.steps), steps=args.steps, warmup=args.warmup,
+                       dump=args.dump_outputs)
         clk.end()
     c = cases.CFG4
     line = {"metric": "miso_target_samples_per_sec", "value": r["target_samples_per_sec"], "unit": "target-samples/s", "n_gpus": 1,
-            "steps": max(100, args.steps), "warmup": 20, "ms_per_step": r["device_us_per_call"] / 1e3, "higher_is_better": True,
+            "steps": args.steps, "warmup": args.warmup, "ms_per_step": r["device_us_per_call"] / 1e3, "higher_is_better": True,
             "scaling": "replicas only", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": {"workload": r["workload"], "targets": c["T"], "channels": 64 * c["nx"] * c["ny"], "frame_len": c["N"]},
             "clocks": clk.summary(), "e2e": {"value": c["T"] * c["N"] / (r["latency_with_upload"]["p50_us"] * 1e-6), "unit": "target-samples/s",
@@ -564,6 +600,8 @@ def run_ours(args, c, name):
         ms, launches, das_ms, das_n, pack_ms, pack_n = measure_resident(w, tm, step, args.steps, fl_launch)
         clk.end()
         value = B * args.steps / (ms / 1e3)
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, power_maps=out_all)     # the complete [B][D] maps of the last timed step
         # the dominant kernel's OWN launch duration (roofline.achieved) is timed with one synchronous call per step: in
         # continuous operation consecutive launches overlap, and an event pair around a launch then also spans its wait
         # for the SMs the previous launch still holds
