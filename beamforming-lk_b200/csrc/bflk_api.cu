@@ -9,6 +9,7 @@
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 
 #include "bflk_internal.h"
 
@@ -71,11 +72,9 @@ int bflk_create(const bflk_config *cfg, bflk_handle **out) {
     h->tuning.tile_pairs = env_int("BFLK_TILE_PAIRS", 0);
     h->tuning.tile_mode = env_int("BFLK_TILE_MODE", -1);
     h->tuning.no_ksplit = env_int("BFLK_NO_KSPLIT", 0);
-    h->tuning.sharded_overlap_compute = env_int("BFLK_SHARDED_OVERLAP_COMPUTE", 0);
     h->tuning.lat_warps = env_int("BFLK_LAT_WARPS", 0);
     h->tuning.lat_split = env_int("BFLK_LAT_SPLIT", 0);
     h->tuning.chunk_mib = env_int("BFLK_CHUNK_MIB", 0);
-    h->tuning.chunk_one_stream = env_int("BFLK_CHUNK_ONE_STREAM", 0);
     if ((e = cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking)) != cudaSuccess) {
         delete h;
         return create_fail(BFLK_ERR_CUDA, std::string("cudaStreamCreate: ") + cudaGetErrorString(e));
@@ -94,14 +93,15 @@ int bflk_destroy(bflk_handle *h) {
     }
     if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
     for (int k = 0; k < 2; k++) {
-        if (h->chunk_stream[k]) { cudaStreamSynchronize(h->chunk_stream[k]); cudaStreamDestroy(h->chunk_stream[k]); }
-        if (h->chunk_join[k]) cudaEventDestroy(h->chunk_join[k]);
+        if (h->lane[k]) { cudaStreamSynchronize(h->lane[k]); cudaStreamDestroy(h->lane[k]); }
+        if (h->lane_done[k]) cudaEventDestroy(h->lane_done[k]);
         if (h->dev_in[k]) cudaEventDestroy(h->dev_in[k]);
+        h->scratch[k].packed.release();
+        h->scratch[k].partial.release();
     }
-    h->d_packed_alt.release(); h->d_partial_alt.release();
     for (cudaEvent_t e : h->chunk_events) cudaEventDestroy(e);
     h->d_fir.release(); h->d_xyz.release(); h->d_index.release(); h->d_off.release(); h->d_frac.release(); h->d_tiles.release();
-    h->d_tile_dirs.release(); h->d_packed.release(); h->d_bcast_table.release(); h->d_bcast_dirs.release(); h->d_bcast_globals.release(); h->d_window.release(); h->d_power.release(); h->d_audio.release(); h->d_partial.release();
+    h->d_tile_dirs.release(); h->d_bcast_table.release(); h->d_bcast_dirs.release(); h->d_bcast_globals.release(); h->d_window.release(); h->d_power.release(); h->d_audio.release();
     h->d_trig.release(); h->d_soff.release(); h->d_sfrac.release(); h->d_misc.release();
     h->p_in.release(); h->p_out.release(); h->p_trig.release(); h->p_misc.release(); h->p_stage.release();
     for (int k = 0; k < 2; k++) {
@@ -626,7 +626,6 @@ static int ensure_bcast(bflk_handle *h) {
     return BFLK_OK;
 }
 
-// stream_dev: first sample of frame 0; rows are row_stride floats apart and hold row_len valid samples
 }  // extern "C"
 
 // CTA shape of a call that cannot fill two waves of 16-warp CTAs (a live worker's single frame).  One CTA per SM (the stage
@@ -659,33 +658,69 @@ void bflk::latency_shape(long long n_tiles, long long pair_ctas, int sms, int n_
     if (*warps == 16 && *split == 1) *warps = 0;
 }
 
+int bflk::tiled_form(const bflk_handle *h) {
+    if (h->fir_phases > 0 || h->kernel_choice == 1 || h->kernel_choice == 3) return -1;
+    return h->kernel_choice != 2 ? 1 : 0;
+}
+
+int bflk::note_use(bflk_handle *h, cudaStream_t st, bool overlapped) {
+    if (!h->caller_event) BFLK_CUDA(h, cudaEventCreateWithFlags(&h->caller_event, cudaEventDisableTiming));
+    BFLK_CUDA(h, cudaEventRecord(h->caller_event, st));
+    h->last_stream = st;
+    h->caller_event_is_overlapped = overlapped;
+    return BFLK_OK;
+}
+
+int bflk::lanes_fork(bflk_handle *h, cudaEvent_t after, int only) {
+    for (int i = 0; i < 2; i++) {
+        if (!h->lane[i]) BFLK_CUDA(h, cudaStreamCreateWithFlags(&h->lane[i], cudaStreamNonBlocking));
+        if (!h->lane_done[i]) BFLK_CUDA(h, cudaEventCreateWithFlags(&h->lane_done[i], cudaEventDisableTiming));
+    }
+    // tables first (ensure_tiles synchronises the handle's stream when it has to build them), before anything is queued
+    const int form = tiled_form(h);
+    if (form >= 0) {
+        int rc = ensure_tiles(h, form, 0);
+        if (rc) return rc;
+    }
+    const bool wait_caller = h->caller_event && !(only >= 0 && h->caller_event_is_overlapped);
+    for (int i = 0; i < 2; i++) {
+        if (only >= 0 && i != only) continue;
+        if (after) BFLK_CUDA(h, cudaStreamWaitEvent(h->lane[i], after, 0));
+        if (wait_caller) BFLK_CUDA(h, cudaStreamWaitEvent(h->lane[i], h->caller_event, 0));
+    }
+    return BFLK_OK;
+}
+
+int bflk::lanes_join(bflk_handle *h, int only) {
+    for (int i = 0; i < 2; i++) {
+        if (only >= 0 && i != only) continue;
+        BFLK_CUDA(h, cudaEventRecord(h->lane_done[i], h->lane[i]));
+        BFLK_CUDA(h, cudaStreamWaitEvent(h->stream, h->lane_done[i], 0));
+    }
+    return note_use(h, h->stream, only >= 0);
+}
+
 int bflk::power_map_dev(bflk_handle *h, const float *stream_dev, int64_t row_stride, int64_t n_samples, int32_t n_frames,
-                        float *power_dev, void *cuda_stream) {
+                        float *power_dev, const Launch &launch) {
     if (!h) return BFLK_ERR_INVALID;
     if (!h->have_grid) return h->fail(BFLK_ERR_STATE, "bflk_power_map: set geometry and grid first");
-    const int32_t *wire = h->wire_src;   // wire-format call: stream_dev is null, the samples are h->wire_src[n_samples][C]
+    const int32_t *wire = launch.wire;   // wire-format call: stream_dev is null, the samples are wire[n_samples][C]
     if ((!stream_dev && !wire) || !power_dev || n_frames <= 0) return h->fail(BFLK_ERR_INVALID, "bflk_power_map: null buffer or no frames");
     if (n_samples < min_stream_samples(h, n_frames))
         return h->fail(BFLK_ERR_INVALID, "bflk_power_map: %lld samples per channel cannot hold %d frames (need %lld)",
                        (long long)n_samples, n_frames, (long long)min_stream_samples(h, n_frames));
     BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
-    cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : h->stream;
+    cudaStream_t st = launch.st ? launch.st : h->stream;
     // the packed rows, partial sums and tables are the handle's: a call on another stream than the previous one waits for it
-    // (the chunk loop of a host batch orders its two streams and scratch sets itself and leaves the event behind at its end)
-    if (!h->chunk_mode && h->caller_event && h->last_stream != st) BFLK_CUDA(h, cudaStreamWaitEvent(st, h->caller_event, 0));
+    if (!launch.pipelined && h->caller_event && h->last_stream != st) BFLK_CUDA(h, cudaStreamWaitEvent(st, h->caller_event, 0));
     struct Mark {   // every exit after this point leaves an event behind on the stream the call used
         bflk_handle *h;
         cudaStream_t st;
-        ~Mark() {
-            if (h->chunk_mode) return;
-            if (!h->caller_event && cudaEventCreateWithFlags(&h->caller_event, cudaEventDisableTiming) != cudaSuccess) return;
-            cudaEventRecord(h->caller_event, st);
-            h->last_stream = st;
-            h->caller_event_is_overlapped = false;
-        }
-    } mark{h, st};
-    DevBuf<char> &d_packed = h->scratch_slot ? h->d_packed_alt : h->d_packed;
-    DevBuf<float> &d_partial = h->scratch_slot ? h->d_partial_alt : h->d_partial;
+        bool on;
+        ~Mark() { if (on) note_use(h, st, false); }
+    } mark{h, st, !launch.pipelined};
+    DevBuf<char> &d_packed = h->scratch[launch.scratch].packed;
+    DevBuf<float> &d_partial = h->scratch[launch.scratch].partial;
     const int N = h->cfg.frame_len, C = h->cfg.n_channels, usable = (int)h->index.size();
     const float norm = static_cast<float>(N * usable);  // power /= float(N_SAMPLES * count), mimo.cpp:137
     // automatic choice: register-tiled kernel when the grid tiles (2x2 direction tiles with small offset
@@ -695,7 +730,8 @@ int bflk::power_map_dev(bflk_handle *h, const float *stream_dev, int64_t row_str
     if (fir && h->kernel_choice > 1) return h->fail(BFLK_ERR_STATE, "bflk_power_map: FIR interpolation needs kernel 0 or 1");
     if (fir && n_samples < min_stream_samples(h, n_frames) + h->fir_taps - 2)
         return h->fail(BFLK_ERR_INVALID, "bflk_power_map: the FIR reads %d samples past a frame's last tap", h->fir_taps - 2);
-    if (!fir && (h->kernel_choice == 0 || h->kernel_choice == 2 || h->kernel_choice == 4)) {
+    const int form = tiled_form(h);
+    if (form >= 0) {
         // automatic choice = the two-FMA variant (power within the 1e-4 bar); 2 asks for bit-identical delayed sums
         // a call with few block pairs cannot fill the SMs with 16-warp CTAs (one cfg3 frame: 16 CTAs, each walking 512
         // channels with four warps per scheduler): smaller CTAs trade per-SM efficiency for latency.  The shape is part of
@@ -713,8 +749,8 @@ int bflk::power_map_dev(bflk_handle *h, const float *stream_dev, int64_t row_str
         }
         if (want_warps > 0 && h->tuning.lat_warps >= 2 && h->tuning.lat_warps <= 16) want_warps = h->tuning.lat_warps;   // experiments
         if (want_warps > 0 && h->tuning.lat_split >= 1 && h->allow_ksplit) want_split = h->tuning.lat_split;
-        if (h->chunk_mode) { want_warps = 0; want_split = 1; }   // the chunk loop built the throughput-shape tables before it queued anything
-        int rc = ensure_tiles(h, h->kernel_choice != 2 ? 1 : 0, want_warps);
+        if (launch.pipelined) { want_warps = 0; want_split = 1; }   // lanes_fork built the throughput-shape tables
+        int rc = ensure_tiles(h, form, want_warps);
         if (rc) return rc;
         h->tile_geom.ksplit = das_tile_ksplit_ok(h->tile_geom, want_split) ? want_split : 1;
         tiled = h->tiles_usable && (wire || (!(row_stride & 1) && !((uintptr_t)stream_dev & 7)));  // packed rows: 8-byte loads
@@ -827,41 +863,27 @@ int bflk::power_map_dev_overlapped(bflk_handle *h, const float *stream_dev, int6
     *used = caller;
     if (!h->have_grid) return h->fail(BFLK_ERR_STATE, "bflk_power_map: set geometry and grid first");
     BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
-    const bool tiled_choice = !h->fir_phases && !h->wire_src && (h->kernel_choice == 0 || h->kernel_choice == 2 || h->kernel_choice == 4);
-    if (tiled_choice) {
-        // tables first (ensure_tiles synchronises the handle's stream when it has to build them), before anything is queued
-        int rc = ensure_tiles(h, h->kernel_choice != 2 ? 1 : 0, 0);
+    const int form = tiled_form(h);
+    if (form >= 0) {
+        int rc = ensure_tiles(h, form, 0);
         if (rc) return rc;
     }
-    if (!tiled_choice || !h->tiles_usable || (row_stride & 1) || ((uintptr_t)stream_dev & 7))
-        return power_map_dev(h, stream_dev, row_stride, n_samples, n_frames, power_dev, caller);
+    if (form < 0 || !h->tiles_usable || (row_stride & 1) || ((uintptr_t)stream_dev & 7))
+        return power_map_dev(h, stream_dev, row_stride, n_samples, n_frames, power_dev, Launch{caller});
     const int slot = (int)(h->dev_seq++ & 1);
-    for (int i = 0; i < 2; i++) {
-        if (!h->chunk_stream[i]) BFLK_CUDA(h, cudaStreamCreateWithFlags(&h->chunk_stream[i], cudaStreamNonBlocking));
-        if (!h->chunk_join[i]) BFLK_CUDA(h, cudaEventCreateWithFlags(&h->chunk_join[i], cudaEventDisableTiming));
+    for (int i = 0; i < 2; i++)
         if (!h->dev_in[i]) BFLK_CUDA(h, cudaEventCreateWithFlags(&h->dev_in[i], cudaEventDisableTiming));
-    }
-    if (!h->caller_event) BFLK_CUDA(h, cudaEventCreateWithFlags(&h->caller_event, cudaEventDisableTiming));
-    cudaStream_t cs = h->chunk_stream[slot];
     // this batch's kernels wait for (a) the caller's stream having reached this call (its inputs), (b) whatever used the handle's
     // scratch on another stream before the overlapped batches began.  Earlier overlapped batches need no wait: the same
-    // set's previous batch ran on this very stream, the other set's batch shares nothing with this one.
+    // set's previous batch ran on this very lane, the other set's batch shares nothing with this one.
     BFLK_CUDA(h, cudaEventRecord(h->dev_in[slot], caller));
-    BFLK_CUDA(h, cudaStreamWaitEvent(cs, h->dev_in[slot], 0));
-    if (!h->caller_event_is_overlapped && h->last_stream) BFLK_CUDA(h, cudaStreamWaitEvent(cs, h->caller_event, 0));
-    h->chunk_mode = true;
-    h->scratch_slot = slot;
-    const int rc = power_map_dev(h, stream_dev, row_stride, n_samples, n_frames, power_dev, cs);
-    h->chunk_mode = false;
-    h->scratch_slot = 0;
+    int rc = lanes_fork(h, h->dev_in[slot], slot);
     if (rc) return rc;
+    if ((rc = power_map_dev(h, stream_dev, row_stride, n_samples, n_frames, power_dev, Launch{h->lane[slot], slot, true})))
+        return rc;
     // the handle's own stream collects the ends of all overlapped batches: caller_event then covers everything enqueued so far
-    BFLK_CUDA(h, cudaEventRecord(h->chunk_join[slot], cs));
-    BFLK_CUDA(h, cudaStreamWaitEvent(h->stream, h->chunk_join[slot], 0));
-    BFLK_CUDA(h, cudaEventRecord(h->caller_event, h->stream));
-    h->last_stream = h->stream;
-    h->caller_event_is_overlapped = true;
-    *used = cs;
+    if ((rc = lanes_join(h, slot))) return rc;
+    *used = h->lane[slot];
     return BFLK_OK;
 }
 
@@ -869,7 +891,7 @@ extern "C" {
 
 int bflk_power_map_batch_dev(bflk_handle *h, const float *stream_dev, int64_t n_samples, int32_t n_frames,
                              float *power_dev, void *cuda_stream) {
-    return power_map_dev(h, stream_dev, n_samples, n_samples, n_frames, power_dev, cuda_stream);
+    return power_map_dev(h, stream_dev, n_samples, n_samples, n_frames, power_dev, Launch{(cudaStream_t)cuda_stream});
 }
 
 int bflk_power_map_batch_dev_submit(bflk_handle *h, const float *stream_dev, int64_t n_samples, int32_t n_frames,
@@ -929,26 +951,76 @@ int host_chunk_frames(bflk_handle *h, int n_frames, int *chunk_frames_out) {
 
 extern "C" {
 
-// Enqueues one host batch: chunked uploads on the copy stream, pack + delay-and-sum per chunk on the handle's stream, D2H
-// of each chunk's maps.  Does not synchronise.  d_in / d_out: the device buffers of this batch.
-static int host_batch_enqueue(bflk_handle *h, const float *stream, int64_t n_samples, int32_t n_frames, float *power_out,
-                              DevBuf<float> &d_in, DevBuf<float> &d_out, cudaEvent_t reuse_after) {
-    const int C = h->cfg.n_channels, N = h->cfg.frame_len;
-    const size_t n_in = (size_t)C * n_samples, n_out = (size_t)n_frames * h->dir_count;
-    BFLK_CUDA(h, d_in.reserve(n_in));
-    BFLK_CUDA(h, d_out.reserve(n_out));
-    const int64_t tail = frame_tail_samples(h);
-    int chunk_frames = n_frames;
-    int rc = host_chunk_frames(h, n_frames, &chunk_frames);
-    if (rc) return rc;
+// A host batch's samples as the chunk loop moves them: what differs between channel-major float rows and sample-major wire
+// rows is data here, plus the copy.
+struct HostSamples {
+    const float *dev = nullptr;       // device copy: channel-major float rows [C][n_samples] ...
+    const int32_t *wire = nullptr;    // ... or sample-major wire rows [n_samples][C]
+    int64_t frame_elems = 0;          // elements from one frame's first sample to the next's: N, or N * C (wire)
+    int64_t first = 0, last = 0;      // samples [first, last) of each channel travel; the frames read nothing outside them
+    bool lanes = false;               // several chunks may alternate between the two lanes
+    bool sync_upload_on_compute = false;   // a synchronous single-chunk batch uploads on the compute stream itself
+    std::function<cudaError_t(int64_t t0, int64_t t1, cudaStream_t st)> upload;   // samples [t0, t1) of every channel
+};
+
+// Enqueues a host batch chunk by chunk: the samples of chunk k go up on the copy stream while chunk k - 1 is packed and
+// beamformed, and each chunk's maps come back on its compute stream.  Several chunks alternate between the two lanes (each
+// with its own scratch set), so the CTAs of chunk k + 1 fill the SMs that the last CTAs of chunk k leave idle one by one;
+// the lanes wait for reuse_after (the batch that used these device buffers before), and everything ordered after the
+// handle's stream sees the whole batch.  Does not synchronise.
+static int host_chunks(bflk_handle *h, const HostSamples &in, int64_t n_samples, int32_t n_frames, int chunk_frames,
+                       float *d_out, float *power_out, cudaEvent_t reuse_after) {
+    const int N = h->cfg.frame_len;
     const int n_chunks = (n_frames + chunk_frames - 1) / chunk_frames;
+    const int64_t tail = frame_tail_samples(h);
     if (!h->copy_stream) BFLK_CUDA(h, cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking));
     while ((int)h->chunk_events.size() < n_chunks) {
         cudaEvent_t e;
         BFLK_CUDA(h, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
         h->chunk_events.push_back(e);
     }
-    if (reuse_after) BFLK_CUDA(h, cudaStreamWaitEvent(h->copy_stream, reuse_after, 0));   // the batch that used d_in before is done
+    if (reuse_after) BFLK_CUDA(h, cudaStreamWaitEvent(h->copy_stream, reuse_after, 0));
+    const bool lanes = in.lanes && n_chunks > 1;
+    if (lanes) {
+        int rc = lanes_fork(h, reuse_after);
+        if (rc) return rc;
+    }
+    int64_t copied = in.first;
+    for (int k = 0; k < n_chunks; k++) {
+        const int f0 = k * chunk_frames, nf = std::min(chunk_frames, n_frames - f0);
+        const int64_t need = k == n_chunks - 1 ? in.last : std::min<int64_t>(in.last, (int64_t)(f0 + nf) * N + tail);
+        cudaStream_t cs = lanes ? h->lane[k & 1] : h->stream;
+        // a synchronous single-chunk call (one live frame) has nothing to overlap: no event hop between two streams
+        cudaStream_t up = (n_chunks == 1 && !reuse_after && in.sync_upload_on_compute) ? cs : h->copy_stream;
+        if (need > copied) {
+            BFLK_CUDA(h, in.upload(copied, need, up));
+            copied = need;
+        }
+        if (up != cs) {
+            BFLK_CUDA(h, cudaEventRecord(h->chunk_events[k], h->copy_stream));
+            BFLK_CUDA(h, cudaStreamWaitEvent(cs, h->chunk_events[k], 0));
+        }
+        const int64_t off = (int64_t)f0 * in.frame_elems;
+        float *pk = d_out + (size_t)f0 * h->dir_count;
+        int rc = power_map_dev(h, in.dev ? in.dev + off : nullptr, n_samples, copied - (int64_t)f0 * N, nf, pk,
+                               Launch{cs, lanes ? (k & 1) : 0, lanes, in.wire ? in.wire + off : nullptr});
+        if (rc) return rc;
+        BFLK_CUDA(h, cudaMemcpyAsync(power_out + (size_t)f0 * h->dir_count, pk, (size_t)nf * h->dir_count * sizeof(float),
+                                     cudaMemcpyDeviceToHost, cs));
+    }
+    return lanes ? lanes_join(h) : BFLK_OK;
+}
+
+// One float host batch into the device buffers d_in / d_out of this batch.  Does not synchronise.
+static int host_batch_enqueue(bflk_handle *h, const float *stream, int64_t n_samples, int32_t n_frames, float *power_out,
+                              DevBuf<float> &d_in, DevBuf<float> &d_out, cudaEvent_t reuse_after) {
+    const int C = h->cfg.n_channels, N = h->cfg.frame_len;
+    const size_t n_in = (size_t)C * n_samples, n_out = (size_t)n_frames * h->dir_count;
+    BFLK_CUDA(h, d_in.reserve(n_in));
+    BFLK_CUDA(h, d_out.reserve(n_out));
+    int chunk_frames = n_frames;
+    int rc = host_chunk_frames(h, n_frames, &chunk_frames);
+    if (rc) return rc;
     // only the samples a frame can touch travel: [history - largest delay, last frame's last tap] -- a third of the
     // reference's 1024-sample window for a single frame (the rest of d_in is never read)
     // (a strided copy out of PAGEABLE memory is staged row by row by the driver and loses more than it saves -- measured
@@ -956,78 +1028,27 @@ static int host_batch_enqueue(bflk_handle *h, const float *stream, int64_t n_sam
     cudaPointerAttributes attr{};
     const bool pageable = cudaPointerGetAttributes(&attr, stream) != cudaSuccess || attr.type == cudaMemoryTypeUnregistered;
     cudaGetLastError();
-    if (pageable && n_chunks == 1) {
+    if (pageable && chunk_frames >= n_frames) {
         if (reuse_after) BFLK_CUDA(h, cudaStreamWaitEvent(h->stream, reuse_after, 0));
         BFLK_CUDA(h, cudaMemcpyAsync(d_in.p, stream, n_in * sizeof(float), cudaMemcpyHostToDevice, h->stream));
-        rc = power_map_dev(h, d_in.p, n_samples, n_samples, n_frames, d_out.p, h->stream);
+        rc = power_map_dev(h, d_in.p, n_samples, n_samples, n_frames, d_out.p, Launch{h->stream});
         if (rc) return rc;
         BFLK_CUDA(h, cudaMemcpyAsync(power_out, d_out.p, n_out * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
         return BFLK_OK;
     }
-    int64_t copied = pageable ? 0 : std::max<int64_t>(0, (int64_t)(h->cfg.history - h->max_delay) & ~(int64_t)3);  // samples per row already "on the device"
-    const int64_t last_needed = std::min<int64_t>(n_samples, (int64_t)(n_frames - 1) * N + tail + N);
-    // several chunks: their kernels alternate between two compute streams (each with its own scratch), so the CTAs of
-    // chunk k + 1 fill the SMs that the last CTAs of chunk k leave idle one by one.  Ordering: a stream's chunks follow
-    // each other; both streams wait for whatever the handle's stream had queued before this batch (tables, a previous
-    // synchronous call) and for the batch that used these device buffers before (reuse_after); at the end the handle's
-    // stream waits for both, so everything ordered after it (async_done, later calls) sees the whole batch.
-    const bool two_streams = n_chunks > 1 && !h->tuning.chunk_one_stream;
-    if (two_streams) {
-        for (int i = 0; i < 2; i++) {
-            if (!h->chunk_stream[i]) BFLK_CUDA(h, cudaStreamCreateWithFlags(&h->chunk_stream[i], cudaStreamNonBlocking));
-            if (!h->chunk_join[i]) BFLK_CUDA(h, cudaEventCreateWithFlags(&h->chunk_join[i], cudaEventDisableTiming));
-        }
-        // tables first (ensure_tiles synchronises the handle's stream when it has to build them), before any chunk is queued
-        if (!h->fir_phases && (h->kernel_choice == 0 || h->kernel_choice == 2 || h->kernel_choice == 4)) {
-            rc = ensure_tiles(h, h->kernel_choice != 2 ? 1 : 0, 0);
-            if (rc) return rc;
-        }
-        if (h->caller_event)
-            for (int i = 0; i < 2; i++) BFLK_CUDA(h, cudaStreamWaitEvent(h->chunk_stream[i], h->caller_event, 0));
-        if (reuse_after)
-            for (int i = 0; i < 2; i++) BFLK_CUDA(h, cudaStreamWaitEvent(h->chunk_stream[i], reuse_after, 0));
-    }
-    struct ChunkMode {   // power_map_dev leaves the stream ordering to this loop while it runs
-        bflk_handle *h;
-        bool on;
-        ~ChunkMode() { if (on) { h->chunk_mode = false; h->scratch_slot = 0; } }
-    } mode{h, two_streams};
-    h->chunk_mode = two_streams;
-    for (int k = 0; k < n_chunks; k++) {
-        const int f0 = k * chunk_frames, nf = std::min(chunk_frames, n_frames - f0);
-        const int64_t need = k == n_chunks - 1 ? last_needed : std::min<int64_t>(last_needed, (int64_t)(f0 + nf) * N + tail);
-        cudaStream_t cs = two_streams ? h->chunk_stream[k & 1] : h->stream;
-        // a synchronous single-chunk call (one live frame) has nothing to overlap: its upload goes on the compute stream
-        // itself, no event hop between two streams on the latency path
-        cudaStream_t up = (n_chunks == 1 && !reuse_after) ? cs : h->copy_stream;
-        if (need > copied) {
-            BFLK_CUDA(h, cudaMemcpy2DAsync(d_in.p + copied, n_samples * sizeof(float), stream + copied,
-                                           n_samples * sizeof(float), (need - copied) * sizeof(float), C,
-                                           cudaMemcpyHostToDevice, up));
-            copied = need;
-        }
-        h->scratch_slot = two_streams ? (k & 1) : 0;
-        if (up != cs) {
-            BFLK_CUDA(h, cudaEventRecord(h->chunk_events[k], h->copy_stream));
-            BFLK_CUDA(h, cudaStreamWaitEvent(cs, h->chunk_events[k], 0));
-        }
-        float *pk = d_out.p + (size_t)f0 * h->dir_count;
-        rc = power_map_dev(h, d_in.p + (size_t)f0 * N, n_samples, copied - (int64_t)f0 * N, nf, pk, cs);
-        if (rc) return rc;
-        BFLK_CUDA(h, cudaMemcpyAsync(power_out + (size_t)f0 * h->dir_count, pk, (size_t)nf * h->dir_count * sizeof(float),
-                                     cudaMemcpyDeviceToHost, cs));
-    }
-    if (two_streams) {
-        for (int i = 0; i < 2; i++) {
-            BFLK_CUDA(h, cudaEventRecord(h->chunk_join[i], h->chunk_stream[i]));
-            BFLK_CUDA(h, cudaStreamWaitEvent(h->stream, h->chunk_join[i], 0));
-        }
-        if (!h->caller_event) BFLK_CUDA(h, cudaEventCreateWithFlags(&h->caller_event, cudaEventDisableTiming));
-        BFLK_CUDA(h, cudaEventRecord(h->caller_event, h->stream));
-        h->last_stream = h->stream;
-        h->caller_event_is_overlapped = false;
-    }
-    return BFLK_OK;
+    HostSamples in;
+    in.dev = d_in.p;
+    in.frame_elems = N;
+    in.first = pageable ? 0 : std::max<int64_t>(0, (int64_t)(h->cfg.history - h->max_delay) & ~(int64_t)3);
+    in.last = std::min<int64_t>(n_samples, (int64_t)(n_frames - 1) * N + frame_tail_samples(h) + N);
+    in.lanes = true;
+    in.sync_upload_on_compute = true;
+    float *dev = d_in.p;
+    in.upload = [=](int64_t t0, int64_t t1, cudaStream_t st) {
+        return cudaMemcpy2DAsync(dev + t0, n_samples * sizeof(float), stream + t0, n_samples * sizeof(float),
+                                 (t1 - t0) * sizeof(float), C, cudaMemcpyHostToDevice, st);
+    };
+    return host_chunks(h, in, n_samples, n_frames, chunk_frames, d_out.p, power_out, reuse_after);
 }
 
 static int host_batch_check(bflk_handle *h, const float *stream, int64_t n_samples, int32_t n_frames, const float *power_out) {
@@ -1083,17 +1104,20 @@ int bflk_power_map_batch(bflk_handle *h, const float *stream, int64_t n_samples,
     return BFLK_OK;
 }
 
+static int wire_check(bflk_handle *h, int64_t n_samples) {
+    if (h->cfg.n_channels % 8) return h->fail(BFLK_ERR_INVALID, "bflk_power_map_batch_i32: n_channels must be a multiple of 8 (serpentine rows)");
+    if (n_samples > 0x7fffffff) return h->fail(BFLK_ERR_INVALID, "bflk_power_map_batch_i32: more than 2^31 samples per call");
+    return BFLK_OK;
+}
+
 // frames[n_samples][C] int32 on the DEVICE, frame b = rows [b * N, b * N + H + N + 1): asynchronous on cuda_stream
 int bflk_power_map_batch_i32_dev(bflk_handle *h, const int32_t *frames_dev, int64_t n_samples, int32_t n_frames,
                                  float *power_dev, void *cuda_stream) {
     if (!h) return BFLK_ERR_INVALID;
     if (!frames_dev) return h->fail(BFLK_ERR_INVALID, "bflk_power_map_batch_i32: null buffer");
-    if (h->cfg.n_channels % 8) return h->fail(BFLK_ERR_INVALID, "bflk_power_map_batch_i32: n_channels must be a multiple of 8 (serpentine rows)");
-    if (n_samples > 0x7fffffff) return h->fail(BFLK_ERR_INVALID, "bflk_power_map_batch_i32: more than 2^31 samples per call");
-    h->wire_src = frames_dev;
-    const int rc = power_map_dev(h, nullptr, n_samples, n_samples, n_frames, power_dev, cuda_stream);
-    h->wire_src = nullptr;
-    return rc;
+    int rc = wire_check(h, n_samples);
+    if (rc) return rc;
+    return power_map_dev(h, nullptr, n_samples, n_samples, n_frames, power_dev, Launch{(cudaStream_t)cuda_stream, 0, false, frames_dev});
 }
 
 // Host buffers: the wire samples go up in chunks of frames (contiguous rows of the sample-major layout) on the copy
@@ -1105,72 +1129,31 @@ int bflk_power_map_batch_i32(bflk_handle *h, const int32_t *frames, int64_t n_sa
     if (n_samples < min_stream_samples(h, n_frames))
         return h->fail(BFLK_ERR_INVALID, "bflk_power_map_batch_i32: %lld samples cannot hold %d frames (need %lld)",
                        (long long)n_samples, n_frames, (long long)min_stream_samples(h, n_frames));
+    int rc = wire_check(h, n_samples);
+    if (rc) return rc;
     BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
     const int C = h->cfg.n_channels, N = h->cfg.frame_len;
     BFLK_CUDA(h, h->d_wire.reserve((size_t)C * n_samples));
     BFLK_CUDA(h, h->d_power.reserve((size_t)n_frames * h->dir_count));
-    const int64_t tail = frame_tail_samples(h);
     int chunk_frames = n_frames;
-    int rc = host_chunk_frames(h, n_frames, &chunk_frames);
-    if (rc) return rc;
-    const int n_chunks = (n_frames + chunk_frames - 1) / chunk_frames;
-    if (!h->copy_stream) BFLK_CUDA(h, cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking));
-    while ((int)h->chunk_events.size() < n_chunks) {
-        cudaEvent_t e;
-        BFLK_CUDA(h, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-        h->chunk_events.push_back(e);
+    if ((rc = host_chunk_frames(h, n_frames, &chunk_frames))) return rc;
+    HostSamples in;
+    in.wire = h->d_wire.p;
+    in.frame_elems = (int64_t)N * C;
+    in.last = n_samples;
+    // two lanes only when the register-tiled kernel takes the wire samples directly: the other kernels convert them into
+    // the handle's one float window first (ingest_kernel)
+    const int form = tiled_form(h);
+    if (chunk_frames < n_frames && form >= 0) {
+        if ((rc = ensure_tiles(h, form, 0))) return rc;
+        in.lanes = h->tiles_usable;
     }
-    int64_t copied = 0;  // samples (rows) already on the device
-    // chunks alternate between two compute streams like host_batch_enqueue's -- when the register-tiled kernel takes the
-    // wire samples directly (the other kernels go through the handle's one float window, ingest_kernel)
-    bool two_streams = n_chunks > 1 && !h->tuning.chunk_one_stream && !h->fir_phases &&
-                       (h->kernel_choice == 0 || h->kernel_choice == 2 || h->kernel_choice == 4);
-    if (two_streams) {
-        rc = ensure_tiles(h, h->kernel_choice != 2 ? 1 : 0, 0);
-        if (rc) return rc;
-        two_streams = h->tiles_usable;
-    }
-    if (two_streams) {
-        for (int i = 0; i < 2; i++) {
-            if (!h->chunk_stream[i]) BFLK_CUDA(h, cudaStreamCreateWithFlags(&h->chunk_stream[i], cudaStreamNonBlocking));
-            if (!h->chunk_join[i]) BFLK_CUDA(h, cudaEventCreateWithFlags(&h->chunk_join[i], cudaEventDisableTiming));
-            if (h->caller_event) BFLK_CUDA(h, cudaStreamWaitEvent(h->chunk_stream[i], h->caller_event, 0));
-        }
-    }
-    struct ChunkMode {
-        bflk_handle *h;
-        bool on;
-        ~ChunkMode() { if (on) { h->chunk_mode = false; h->scratch_slot = 0; } }
-    } mode{h, two_streams};
-    h->chunk_mode = two_streams;
-    for (int k = 0; k < n_chunks; k++) {
-        const int f0 = k * chunk_frames, nf = std::min(chunk_frames, n_frames - f0);
-        const int64_t need = std::min<int64_t>(n_samples, k == n_chunks - 1 ? n_samples : (int64_t)(f0 + nf) * N + tail);
-        if (need > copied) {
-            BFLK_CUDA(h, cudaMemcpyAsync(h->d_wire.p + (size_t)copied * C, frames + (size_t)copied * C, (size_t)(need - copied) * C * sizeof(int32_t),
-                                         cudaMemcpyHostToDevice, h->copy_stream));
-            copied = need;
-        }
-        cudaStream_t cs = two_streams ? h->chunk_stream[k & 1] : h->stream;
-        h->scratch_slot = two_streams ? (k & 1) : 0;
-        BFLK_CUDA(h, cudaEventRecord(h->chunk_events[k], h->copy_stream));
-        BFLK_CUDA(h, cudaStreamWaitEvent(cs, h->chunk_events[k], 0));
-        float *pk = h->d_power.p + (size_t)f0 * h->dir_count;
-        rc = bflk_power_map_batch_i32_dev(h, h->d_wire.p + (size_t)f0 * N * C, copied - (int64_t)f0 * N, nf, pk, cs);
-        if (rc) return rc;
-        BFLK_CUDA(h, cudaMemcpyAsync(power_out + (size_t)f0 * h->dir_count, pk, (size_t)nf * h->dir_count * sizeof(float),
-                                     cudaMemcpyDeviceToHost, cs));
-    }
-    if (two_streams) {
-        for (int i = 0; i < 2; i++) {
-            BFLK_CUDA(h, cudaEventRecord(h->chunk_join[i], h->chunk_stream[i]));
-            BFLK_CUDA(h, cudaStreamWaitEvent(h->stream, h->chunk_join[i], 0));
-        }
-        if (!h->caller_event) BFLK_CUDA(h, cudaEventCreateWithFlags(&h->caller_event, cudaEventDisableTiming));
-        BFLK_CUDA(h, cudaEventRecord(h->caller_event, h->stream));
-        h->last_stream = h->stream;
-        h->caller_event_is_overlapped = false;
-    }
+    int32_t *dev = h->d_wire.p;
+    in.upload = [=](int64_t t0, int64_t t1, cudaStream_t st) {
+        return cudaMemcpyAsync(dev + (size_t)t0 * C, frames + (size_t)t0 * C, (size_t)(t1 - t0) * C * sizeof(int32_t),
+                               cudaMemcpyHostToDevice, st);
+    };
+    if ((rc = host_chunks(h, in, n_samples, n_frames, chunk_frames, h->d_power.p, power_out, nullptr))) return rc;
     BFLK_CUDA(h, cudaStreamSynchronize(h->stream));
     return BFLK_OK;
 }
@@ -1216,7 +1199,6 @@ int bflk_set_window_dev(bflk_handle *h, const float *window_dev) {
 static int miso_launch(bflk_handle *h, const double *theta, const double *phi, int n_targets, const float *window_dev,
                        float *audio_dev, float *power_dev, int32_t *flag_dev, cudaStream_t st) {
     const int C = h->cfg.n_channels, N = h->cfg.frame_len;
-    if (!h->caller_event) BFLK_CUDA(h, cudaEventCreateWithFlags(&h->caller_event, cudaEventDisableTiming));
     MisoArgs a{};
     if (n_targets <= kMisoInline) {
         for (int i = 0; i < n_targets; i++) a.trig_inline[i] = make_trig(theta[i], phi[i]);
@@ -1224,7 +1206,7 @@ static int miso_launch(bflk_handle *h, const double *theta, const double *phi, i
     } else {
         BFLK_CUDA(h, h->p_trig.reserve(n_targets));
         BFLK_CUDA(h, h->d_trig.reserve(n_targets));
-        BFLK_CUDA(h, cudaEventSynchronize(h->caller_event));   // the previous call's copy is done with the staging
+        if (h->caller_event) BFLK_CUDA(h, cudaEventSynchronize(h->caller_event));   // the previous call's copy is done with the staging
         for (int i = 0; i < n_targets; i++) h->p_trig.p[i] = make_trig(theta[i], phi[i]);
         BFLK_CUDA(h, cudaMemcpyAsync(h->d_trig.p, h->p_trig.p, n_targets * sizeof(DirTrig), cudaMemcpyHostToDevice, st));
         a.trig = h->d_trig.p;
@@ -1232,7 +1214,7 @@ static int miso_launch(bflk_handle *h, const double *theta, const double *phi, i
     if (power_dev) {
         const size_t slots = (size_t)n_targets * das_miso_slices(N);
         if (slots > h->d_miso_partial.n || (size_t)n_targets > h->d_miso_counters.n) {
-            BFLK_CUDA(h, cudaEventSynchronize(h->caller_event));
+            if (h->caller_event) BFLK_CUDA(h, cudaEventSynchronize(h->caller_event));
             BFLK_CUDA(h, h->d_miso_partial.reserve(slots));
             const size_t had = h->d_miso_counters.n;
             BFLK_CUDA(h, h->d_miso_counters.reserve(std::max<size_t>(n_targets, 256)));
@@ -1260,9 +1242,8 @@ static int miso_launch(bflk_handle *h, const double *theta, const double *phi, i
     a.epoch = ++h->miso_epoch;
     if (h->miso_epoch == 0x7fffffff) h->miso_epoch = 0;
     BFLK_CUDA(h, launch_das_miso(a, st));
-    BFLK_CUDA(h, cudaEventRecord(h->caller_event, st));
     h->launches++;
-    return BFLK_OK;
+    return note_use(h, st, false);
 }
 
 int bflk_miso_dev(bflk_handle *h, const double *theta, const double *phi, int32_t n_targets, const float *window_dev,
@@ -1309,10 +1290,8 @@ int bflk_miso_dev(bflk_handle *h, const double *theta, const double *phi, int32_
     a.norm = static_cast<float>(N);
     a.fir = h->d_fir.p; a.fir_phases = h->fir_phases; a.fir_taps = h->fir_taps;
     BFLK_CUDA(h, launch_das_generic(a, st));
-    if (!h->caller_event) BFLK_CUDA(h, cudaEventCreateWithFlags(&h->caller_event, cudaEventDisableTiming));
-    BFLK_CUDA(h, cudaEventRecord(h->caller_event, st));
     h->launches++;
-    return BFLK_OK;
+    return note_use(h, st, false);
 }
 
 int bflk_miso(bflk_handle *h, const double *theta, const double *phi, int32_t n_targets, const float *window,

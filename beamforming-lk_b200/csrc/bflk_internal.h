@@ -73,10 +73,8 @@ struct Tuning {
     int tile_mode = -1;      // BFLK_TILE_MODE: 0 one window per 2x2 tile, 1 / 2 one window per direction pair
     int lat_warps = 0;       // BFLK_LAT_WARPS / BFLK_LAT_SPLIT: force the CTA shape / cluster size of small calls (measurements)
     int lat_split = 0;
-    int sharded_overlap_compute = 0;   // BFLK_SHARDED_OVERLAP_COMPUTE=1: sharded device batches alternate their kernels between two streams too
     int no_ksplit = 0;       // BFLK_NO_KSPLIT=1: small calls never split the channels across a thread-block cluster
     int chunk_mib = 0;       // BFLK_CHUNK_MIB: host batches are uploaded in chunks of about this size
-    int chunk_one_stream = 0;  // BFLK_CHUNK_ONE_STREAM=1: the chunks' kernels on one stream (round-2 behaviour, for comparison)
 };
 
 // Shape of the packed rows the tiled kernel stages (das_tile.cu).
@@ -191,7 +189,6 @@ struct bflk_handle {
     bflk::DevBuf<char> d_tiles;             // tile_table_entries(n_tiles, usable) TileEntry / TileEntryFast, layout above
     bflk::DevBuf<int32_t> d_tile_dirs;      // [n_tiles][4] local direction index (or -1)
     bflk::TileGeometry tile_geom;
-    bflk::DevBuf<char> d_packed;            // pair-interleaved staging rows of the current batch
 
     // lane-broadcast kernel tables (built lazily for the current grid / mask / range)
     bool bcast_valid = false;
@@ -207,7 +204,6 @@ struct bflk_handle {
 
     // window kept on the device across calls (bflk_set_window): MISO / monopulse iterations on one frame do not re-upload it
     const float *resident_window = nullptr;   // d_resident.p, or a caller-owned device pointer (bflk_set_window_dev)
-    const int32_t *wire_src = nullptr;        // set for the duration of a wire-format call: power_map_dev packs from it
     bflk::DevBuf<int32_t> d_wire;
     bflk::DevBuf<uint8_t> d_bytes;            // heat-map / resize / peak-candidate scratch
     // bflk_power_map_batch_submit / _wait: two batches in flight, each with its own device buffers
@@ -226,7 +222,7 @@ struct bflk_handle {
     cudaStream_t last_stream = nullptr;       // stream of the last asynchronous call
 
     // scratch
-    bflk::DevBuf<float> d_window, d_power, d_audio, d_partial;
+    bflk::DevBuf<float> d_window, d_power, d_audio;
     bflk::DevBuf<bflk::DirTrig> d_trig;
     bflk::DevBuf<int32_t> d_soff;
     bflk::DevBuf<float> d_sfrac;
@@ -237,16 +233,16 @@ struct bflk_handle {
     // host-buffer batches are cut into chunks: copies on copy_stream overlap compute on stream
     cudaStream_t copy_stream = nullptr;
     std::vector<cudaEvent_t> chunk_events;
-    // ... and the chunks' kernels alternate between two compute streams, each with its own packed-row / partial-sum
-    // scratch: a launch on its own ends with half a CTA lifetime of idle SMs on average (the CTAs of a launch all take
-    // equally long and the SMs drift apart), which the next chunk's CTAs fill when they do not have to wait for it
-    cudaStream_t chunk_stream[2] = {nullptr, nullptr};
-    cudaEvent_t chunk_join[2] = {nullptr, nullptr};
-    bflk::DevBuf<char> d_packed_alt;
-    bflk::DevBuf<float> d_partial_alt;
-    int scratch_slot = 0;         // which scratch set power_map_dev uses (1 only inside a chunked host batch / overlapped device batches)
-    bool chunk_mode = false;      // power_map_dev is being called by the chunk loop, which orders the streams itself
-    // device batches in continuous operation (power_map_dev_overlapped): they alternate between the two compute streams too
+    // ... and the chunks' kernels alternate between two compute lanes (lanes_fork / lanes_join), each with its own scratch
+    // set: a launch on its own ends with half a CTA lifetime of idle SMs on average (the CTAs of a launch all take equally
+    // long and the SMs drift apart), which the next chunk's CTAs fill when they do not have to wait for it
+    cudaStream_t lane[2] = {nullptr, nullptr};
+    cudaEvent_t lane_done[2] = {nullptr, nullptr};
+    struct {
+        bflk::DevBuf<char> packed;     // pair-interleaved staging rows of the current batch
+        bflk::DevBuf<float> partial;   // partial sums of frames longer than one block
+    } scratch[2];                      // set 1 only for lane 1 (Launch::scratch)
+    // device batches in continuous operation (power_map_dev_overlapped): they alternate between the two lanes too
     cudaEvent_t dev_in[2] = {nullptr, nullptr};   // "the caller's stream has reached the submit" (inputs ready)
     uint64_t dev_seq = 0;
     bool caller_event_is_overlapped = false;      // the latest caller_event covers overlapped batches only (see power_map_dev_overlapped)
@@ -408,16 +404,34 @@ cudaError_t launch_map_targets(const float *d_power, int rows, int cols, int max
                                int32_t *d_index, float *d_pw, float *d_prob, int32_t *d_n, cudaStream_t st);
 
 // ---- bflk_api.cu internals used by multi.cu ---------------------------------------------------------------
+// How power_map_dev runs.  A plain call orders itself against the handle's earlier calls through caller_event; a pipelined
+// one runs on a lane between lanes_fork and lanes_join, which order the streams for it.
+struct Launch {
+    cudaStream_t st = nullptr;       // nullptr: the handle's stream
+    int scratch = 0;                 // which of the handle's two scratch sets
+    bool pipelined = false;          // on a lane: no caller_event wait or record; throughput CTA shape (tables built by lanes_fork)
+    const int32_t *wire = nullptr;   // wire-format input [n_samples][C] instead of stream_dev
+};
 // stream_dev: first sample of frame 0; rows are row_stride floats apart and hold n_samples valid samples
-// Continuous operation: the same as power_map_dev, but enqueued on one of the handle's two compute streams (alternating, each
-// with its own scratch) after `caller` has reached this point; *used = the stream the kernels are on.  Consecutive calls
-// overlap: the pack pre-pass of batch i + 1 runs under the kernel of batch i and its CTAs fill the SMs the last CTAs of
-// batch i leave idle.  caller_event afterwards covers everything enqueued so far.  Falls back to power_map_dev on `caller`
-// (*used = caller) when the register-tiled kernels do not serve the grid.
+int power_map_dev(bflk_handle *h, const float *stream_dev, int64_t row_stride, int64_t n_samples, int32_t n_frames,
+                  float *power_dev, const Launch &launch);
+// Continuous operation: the same as power_map_dev, but enqueued on one of the handle's two lanes (alternating, each with its
+// own scratch) after `caller` has reached this point; *used = the stream the kernels are on.  Consecutive calls overlap: the
+// pack pre-pass of batch i + 1 runs under the kernel of batch i and its CTAs fill the SMs the last CTAs of batch i leave
+// idle.  caller_event afterwards covers everything enqueued so far.  Falls back to power_map_dev on `caller` (*used = caller)
+// when the register-tiled kernels do not serve the grid.
 int power_map_dev_overlapped(bflk_handle *h, const float *stream_dev, int64_t row_stride, int64_t n_samples, int32_t n_frames,
                              float *power_dev, cudaStream_t caller, cudaStream_t *used);
-int power_map_dev(bflk_handle *h, const float *stream_dev, int64_t row_stride, int64_t n_samples, int32_t n_frames,
-                  float *power_dev, void *cuda_stream);
+// Stream ordering of the handle's scratch and tables.  note_use records caller_event on st (the only place it is recorded):
+// a later call on another stream waits for it.  overlapped: it covers overlapped device batches only.
+int note_use(bflk_handle *h, cudaStream_t st, bool overlapped);
+// lanes_fork: the two lanes wait for caller_event and for `after` (if given), once the tile tables are built; lanes_join:
+// the handle's stream waits for them and caller_event is recorded there.  only = 0 / 1: just that lane (one overlapped
+// device batch), which skips caller_event when it covers overlapped batches only (the lane's own are in its stream order).
+int lanes_fork(bflk_handle *h, cudaEvent_t after, int only = -1);
+int lanes_join(bflk_handle *h, int only = -1);
+// -1 when the register-tiled kernels cannot serve a call (FIR, or kernel 1 / 3), else the `fast` flag for ensure_tiles
+int tiled_form(const bflk_handle *h);
 int ensure_tiles(bflk_handle *h, int fast, int want_warps = 0);
 void latency_shape(long long n_tiles, long long pair_ctas, int sms, int n_stage, bool may_split, int *warps, int *split);
 int64_t min_stream_samples(const bflk_handle *h, int n_frames);

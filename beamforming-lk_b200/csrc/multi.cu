@@ -109,7 +109,7 @@ struct bflk_comm {
     cudaEvent_t ev_up[kRing] = {nullptr, nullptr, nullptr}, ev_done[kRing] = {nullptr, nullptr, nullptr};
     bool ev_done_recorded[kRing] = {false, false, false};
     cudaEvent_t ev_async = nullptr;   // end of the last submitted (not yet waited for) host batch
-    cudaEvent_t ev_fork = nullptr;    // start of a host batch on the handle's stream: its two chunk streams wait for it
+    cudaEvent_t ev_fork = nullptr;    // start of a host batch on the handle's stream: its two lanes wait for it
     int async_pending = 0;
     cudaStream_t copy_stream = nullptr;
     int agreed_for_frames = -1, agreed_chunk = 0;   // chunking the ranks of a frame group agreed on
@@ -198,23 +198,19 @@ int check_sharded(bflk_handle *h, const char *who) {
 }
 
 // local compute of one rank: its direction slice of frames [f0, f0 + nf) of a device-resident stream into c->d_send
-// used (optional): continuous operation -- the kernels go on one of the handle's two compute streams (power_map_dev_overlapped)
-// once st has reached this call; *used = that stream
 int compute_shard(bflk_handle *h, const Plan &p, const float *stream_dev, int64_t row_stride, int64_t n_samples, int f_rel0,
-                  int nf, int out_row0, cudaStream_t st, cudaStream_t *used = nullptr) {
+                  int nf, int out_row0, const Launch &launch) {
     bflk_comm *c = h->comm;
-    if (used) *used = st;
     if (nf <= 0 || p.dir_count <= 0) return BFLK_OK;
     const int N = h->cfg.frame_len;
     const bool tight = p.dir_count == p.dir_per;
     float *out = tight ? c->d_send().p + (size_t)out_row0 * p.dir_per : c->d_local().p + (size_t)out_row0 * p.dir_count;
-    int rc = used ? power_map_dev_overlapped(h, stream_dev + (size_t)f_rel0 * N, row_stride, n_samples - (int64_t)f_rel0 * N, nf, out, st, used)
-                  : power_map_dev(h, stream_dev + (size_t)f_rel0 * N, row_stride, n_samples - (int64_t)f_rel0 * N, nf, out, st);
+    int rc = power_map_dev(h, stream_dev + (size_t)f_rel0 * N, row_stride, n_samples - (int64_t)f_rel0 * N, nf, out, launch);
     if (rc) return rc;
     if (!tight)
         BFLK_CUDA(h, cudaMemcpy2DAsync(c->d_send().p + (size_t)out_row0 * p.dir_per, (size_t)p.dir_per * sizeof(float), out,
                                        (size_t)p.dir_count * sizeof(float), (size_t)p.dir_count * sizeof(float), nf,
-                                       cudaMemcpyDeviceToDevice, used ? *used : st));
+                                       cudaMemcpyDeviceToDevice, launch.st));
     return BFLK_OK;
 }
 
@@ -302,15 +298,14 @@ int sharded_dev(const std::vector<bflk_handle *> &hs, const std::vector<const fl
         plans[i] = make_plan(h->n_dir, n_frames, c->n_ranks, c->gd, c->gf, c->rank);
         if ((rc = apply_direction_range(h, plans[i]))) return rc;
         if ((rc = reserve_maps(h, plans[i], n_frames, false))) return rc;
-        // The kernels stay on the caller's stream.  Alternating them between the handle's two compute streams as well
-        // (power_map_dev_overlapped, BFLK_SHARDED_OVERLAP_COMPUTE=1) gains 1.6 % on two GPUs (149.4 k vs 147.0 k maps/s) but
-        // loses on eight (529.6 k vs 573.7 k): with two buffer sets, batch i + 2 waits for the all-gather of batch i, which
-        // waits for kernels that now share the SMs with batch i + 1 -- a bubble per batch once a launch is only four waves.
-        cudaStream_t used = st[i];
-        if ((rc = compute_shard(h, plans[i], stream_dev[i], n_samples, n_samples, plans[i].frame_first, plans[i].frame_count, 0, st[i],
-                                pipelined && h->tuning.sharded_overlap_compute ? &used : nullptr))) return rc;
+        // The kernels stay on the caller's stream.  Alternating them between the handle's two lanes as well
+        // (power_map_dev_overlapped) was measured and not kept: +1.6 % on two GPUs (149.4 k vs 147.0 k maps/s) but -7.7 % on
+        // eight (529.6 k vs 573.7 k): with two buffer sets, batch i + 2 waits for the all-gather of batch i, which waits for
+        // kernels that then share the SMs with batch i + 1 -- a bubble per batch once a launch is only four waves.
+        if ((rc = compute_shard(h, plans[i], stream_dev[i], n_samples, n_samples, plans[i].frame_first, plans[i].frame_count, 0,
+                                Launch{st[i]}))) return rc;
         if (pipelined) {
-            BFLK_CUDA(h, cudaEventRecord(c->ev_computed[c->slot], used));
+            BFLK_CUDA(h, cudaEventRecord(c->ev_computed[c->slot], st[i]));
             BFLK_CUDA(h, cudaStreamWaitEvent(c->gather_stream, c->ev_computed[c->slot], 0));
         }
     }
@@ -434,31 +429,19 @@ int sharded_host(const std::vector<bflk_handle *> &hs, const float *stream, int6
             if (split) BFLK_CUDA(hs[i], c->d_slice[k].reserve((size_t)(C / c->gd) * Tj));
         }
     }
-    // the chunks' kernels alternate between the handle's two chunk streams (own scratch each, bflk_api.cu host_batch_enqueue):
-    // the CTAs of chunk j + 1 fill the SMs that the last CTAs of chunk j leave idle one by one.  Both streams start after
-    // whatever the handle's stream has queued (the previous batch's all-gather reads the buffers this batch writes).
-    std::vector<char> two_streams(G, 0);
+    // the chunks' kernels alternate between the handle's two lanes (own scratch each, bflk_api.cu host_chunks): the CTAs of
+    // chunk j + 1 fill the SMs that the last CTAs of chunk j leave idle one by one.  Both lanes start after whatever the
+    // handle's stream has queued (the previous batch's all-gather reads the buffers this batch writes).
+    std::vector<char> lanes(G, 0);
     for (size_t i = 0; i < G; i++) {
         bflk_handle *h = hs[i];
-        two_streams[i] = n_chunks[i] > 1 && !h->tuning.chunk_one_stream;
-        if (!two_streams[i]) continue;
+        lanes[i] = n_chunks[i] > 1;
+        if (!lanes[i]) continue;
         BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
-        if (!h->fir_phases && (h->kernel_choice == 0 || h->kernel_choice == 2 || h->kernel_choice == 4)) {
-            if ((rc = ensure_tiles(h, h->kernel_choice != 2 ? 1 : 0, 0))) return rc;   // before anything is queued on the chunk streams
-        }
         if (!h->comm->ev_fork) BFLK_CUDA(h, cudaEventCreateWithFlags(&h->comm->ev_fork, cudaEventDisableTiming));
         BFLK_CUDA(h, cudaEventRecord(h->comm->ev_fork, h->stream));
-        for (int k = 0; k < 2; k++) {
-            if (!h->chunk_stream[k]) BFLK_CUDA(h, cudaStreamCreateWithFlags(&h->chunk_stream[k], cudaStreamNonBlocking));
-            if (!h->chunk_join[k]) BFLK_CUDA(h, cudaEventCreateWithFlags(&h->chunk_join[k], cudaEventDisableTiming));
-            BFLK_CUDA(h, cudaStreamWaitEvent(h->chunk_stream[k], h->comm->ev_fork, 0));
-            if (h->caller_event) BFLK_CUDA(h, cudaStreamWaitEvent(h->chunk_stream[k], h->caller_event, 0));
-        }
+        if ((rc = lanes_fork(h, h->comm->ev_fork))) return rc;
     }
-    struct ChunkMode {   // power_map_dev leaves the stream ordering to this loop while it runs
-        const std::vector<bflk_handle *> &hs;
-        ~ChunkMode() { for (bflk_handle *h : hs) { h->chunk_mode = false; h->scratch_slot = 0; } }
-    } mode{hs};
     for (int j = 0; j < max_chunks; j++) {
         const int buf = j % kRing;
         // upload this chunk's rows (copy stream), after the compute that last used the buffer
@@ -510,30 +493,19 @@ int sharded_host(const std::vector<bflk_handle *> &hs, const float *stream, int6
             bflk_comm *c = h->comm;
             BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
             const Chunk k = chunk_of(i, j);
-            cudaStream_t cs = two_streams[i] ? h->chunk_stream[j & 1] : h->stream;
-            h->chunk_mode = two_streams[i];
-            h->scratch_slot = two_streams[i] ? (j & 1) : 0;
+            cudaStream_t cs = lanes[i] ? h->lane[j & 1] : h->stream;
             BFLK_CUDA(h, cudaEventRecord(c->ev_up[buf], c->copy_stream));
             BFLK_CUDA(h, cudaStreamWaitEvent(cs, c->ev_up[buf], 0));
-            rc = compute_shard(h, plans[i], c->d_chunk[buf].p, k.pitch, k.Tj, 0, k.nfj, k.a, cs);
-            h->chunk_mode = false;
-            h->scratch_slot = 0;
+            rc = compute_shard(h, plans[i], c->d_chunk[buf].p, k.pitch, k.Tj, 0, k.nfj, k.a, Launch{cs, lanes[i] ? (j & 1) : 0, (bool)lanes[i]});
             if (rc) return rc;
             BFLK_CUDA(h, cudaEventRecord(c->ev_done[buf], cs));
             c->ev_done_recorded[buf] = true;
         }
     }
-    for (size_t i = 0; i < G; i++) {
-        bflk_handle *h = hs[i];
-        if (!two_streams[i]) continue;
-        BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
-        for (int k = 0; k < 2; k++) {   // the all-gather on the handle's stream follows every chunk
-            BFLK_CUDA(h, cudaEventRecord(h->chunk_join[k], h->chunk_stream[k]));
-            BFLK_CUDA(h, cudaStreamWaitEvent(h->stream, h->chunk_join[k], 0));
-        }
-        if (!h->caller_event) BFLK_CUDA(h, cudaEventCreateWithFlags(&h->caller_event, cudaEventDisableTiming));
-        BFLK_CUDA(h, cudaEventRecord(h->caller_event, h->stream));
-        h->last_stream = h->stream;
+    for (size_t i = 0; i < G; i++) {   // the all-gather on the handle's stream follows every chunk
+        if (!lanes[i]) continue;
+        BFLK_CUDA(hs[i], cudaSetDevice(hs[i]->cfg.device));
+        if ((rc = lanes_join(hs[i]))) return rc;
     }
     std::vector<float *> out_dev(G);
     std::vector<cudaStream_t> st(G);
