@@ -10,6 +10,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <functional>
+#include <memory>
 
 #include "bflk_internal.h"
 
@@ -20,6 +21,11 @@ static thread_local std::string g_create_error;
 static int create_fail(int code, const std::string &msg) {
     g_create_error = msg;
     return code;
+}
+
+bflk_handle::~bflk_handle() {
+    for (const Stream *s : {&stream, &copy_stream, &lane[0], &lane[1]}) s->sync();
+    comm_release(this);
 }
 
 extern "C" {
@@ -61,7 +67,10 @@ int bflk_create(const bflk_config *cfg, bflk_handle **out) {
         return create_fail(BFLK_ERR_NO_DEVICE, "bflk_create: device is not sm_100 (kernels are built for sm_100a only)");
     if ((e = cudaSetDevice(cfg->device)) != cudaSuccess)
         return create_fail(BFLK_ERR_CUDA, std::string("cudaSetDevice: ") + cudaGetErrorString(e));
-    bflk_handle *h = new bflk_handle();
+    cudaGetLastError();   // clear an earlier call's error: the check below is about the handle's streams and events
+    std::unique_ptr<bflk_handle> h(new bflk_handle());
+    if ((e = cudaGetLastError()) != cudaSuccess)
+        return create_fail(BFLK_ERR_CUDA, std::string("bflk_create: cannot create the streams and events: ") + cudaGetErrorString(e));
     h->cfg = *cfg;
     h->sm_count = prop.multiProcessorCount;
     // tuning knobs: read once here, never on a call path (a worker thread calls bflk_power_map every 5 ms)
@@ -75,42 +84,13 @@ int bflk_create(const bflk_config *cfg, bflk_handle **out) {
     h->tuning.lat_warps = env_int("BFLK_LAT_WARPS", 0);
     h->tuning.lat_split = env_int("BFLK_LAT_SPLIT", 0);
     h->tuning.chunk_mib = env_int("BFLK_CHUNK_MIB", 0);
-    if ((e = cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking)) != cudaSuccess) {
-        delete h;
-        return create_fail(BFLK_ERR_CUDA, std::string("cudaStreamCreate: ") + cudaGetErrorString(e));
-    }
-    *out = h;
+    *out = h.release();
     return BFLK_OK;
 }
 
 int bflk_destroy(bflk_handle *h) {
     if (!h) return BFLK_ERR_INVALID;
     cudaSetDevice(h->cfg.device);
-    comm_release(h);
-    if (h->stream) {
-        cudaStreamSynchronize(h->stream);
-        cudaStreamDestroy(h->stream);
-    }
-    if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
-    for (int k = 0; k < 2; k++) {
-        if (h->lane[k]) { cudaStreamSynchronize(h->lane[k]); cudaStreamDestroy(h->lane[k]); }
-        if (h->lane_done[k]) cudaEventDestroy(h->lane_done[k]);
-        if (h->dev_in[k]) cudaEventDestroy(h->dev_in[k]);
-        h->scratch[k].packed.release();
-        h->scratch[k].partial.release();
-    }
-    for (cudaEvent_t e : h->chunk_events) cudaEventDestroy(e);
-    h->d_fir.release(); h->d_xyz.release(); h->d_index.release(); h->d_off.release(); h->d_frac.release(); h->d_tiles.release();
-    h->d_tile_dirs.release(); h->d_bcast_table.release(); h->d_bcast_dirs.release(); h->d_bcast_globals.release(); h->d_window.release(); h->d_power.release(); h->d_audio.release();
-    h->d_trig.release(); h->d_soff.release(); h->d_sfrac.release(); h->d_misc.release();
-    h->p_in.release(); h->p_out.release(); h->p_trig.release(); h->p_misc.release(); h->p_stage.release();
-    for (int k = 0; k < 2; k++) {
-        h->d_async_in[k].release();
-        h->d_async_out[k].release();
-        if (h->async_done[k]) cudaEventDestroy(h->async_done[k]);
-    }
-    h->d_bytes.release(); h->d_wire.release(); h->d_resident.release(); h->d_miso_out.release(); h->d_miso_partial.release(); h->d_miso_counters.release();
-    if (h->caller_event) cudaEventDestroy(h->caller_event);
     delete h;
     return BFLK_OK;
 }
@@ -122,6 +102,7 @@ static void invalidate_tables(bflk_handle *h) {
     h->bcast_valid = false;
     h->n_dir = 0;
     h->dir_first = h->dir_count = 0;
+    h->last_map_on_device = false;
 }
 
 int bflk_set_geometry(bflk_handle *h, const float *xyz, int32_t n_channels) {
@@ -336,6 +317,7 @@ int bflk_set_direction_range(bflk_handle *h, int32_t first, int32_t count) {
     h->dir_count = count;
     h->tiles_valid = false;
     h->bcast_valid = false;
+    h->last_map_on_device = false;   // the map left on the device covers the old range
     return BFLK_OK;
 }
 
@@ -426,12 +408,9 @@ static void timing_hook(void *ctx, int kind, bool begin, cudaStream_t st) {
     bflk_handle *h = static_cast<bflk_handle *>(ctx);
     if (!h->timing) return;
     if (begin) {
-        bflk_handle::Timed t{};
-        t.kind = kind;
-        cudaEventCreate(&t.e0);
-        cudaEventCreate(&t.e1);
-        cudaEventRecord(t.e0, st);
-        h->timed.push_back(t);
+        h->timed.emplace_back();
+        h->timed.back().kind = kind;
+        cudaEventRecord(h->timed.back().e0, st);
     } else if (!h->timed.empty()) {
         cudaEventRecord(h->timed.back().e1, st);
     }
@@ -441,14 +420,14 @@ int bflk_fp32_peak_tflops(bflk_handle *h, float *tflops) {
     if (!h || !tflops) return BFLK_ERR_INVALID;
     BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
     const int blocks = h->sm_count, iters = 8192;
-    BFLK_CUDA(h, h->d_power.reserve((size_t)blocks * 512));
-    cudaEvent_t e0, e1;
-    BFLK_CUDA(h, cudaEventCreate(&e0));
-    BFLK_CUDA(h, cudaEventCreate(&e1));
+    DevBuf<float> d_out;
+    BFLK_CUDA(h, d_out.reserve((size_t)blocks * 512));
+    Event e0(cudaEventDefault), e1(cudaEventDefault);
+    if (!e0 || !e1) return h->fail(BFLK_ERR_CUDA, "bflk_fp32_peak_tflops: cannot create events: %s", cudaGetErrorString(cudaGetLastError()));
     float best = 0.f;
     for (int rep = 0; rep < 4; rep++) {   // first launch warms up; best of the rest
         BFLK_CUDA(h, cudaEventRecord(e0, h->stream));
-        BFLK_CUDA(h, launch_ffma2_peak(h->d_power.p, blocks, iters, h->stream));
+        BFLK_CUDA(h, launch_ffma2_peak(d_out.p, blocks, iters, h->stream));
         BFLK_CUDA(h, cudaEventRecord(e1, h->stream));
         BFLK_CUDA(h, cudaEventSynchronize(e1));
         float ms = 0.f;
@@ -457,8 +436,6 @@ int bflk_fp32_peak_tflops(bflk_handle *h, float *tflops) {
         const double flop = (double)blocks * 512 * iters * 16 * 4;   // a packed FMA = 2 lanes x 2 FLOP
         if (rep > 0) best = std::max(best, (float)(flop / (ms * 1e-3) / 1e12));
     }
-    cudaEventDestroy(e0);
-    cudaEventDestroy(e1);
     *tflops = best;
     return BFLK_OK;
 }
@@ -479,8 +456,6 @@ int bflk_kernel_time_ms(bflk_handle *h, float *das_ms, int32_t *das_launches, fl
         BFLK_CUDA(h, cudaEventElapsedTime(&v, t.e0, t.e1));
         ms[t.kind] += v;
         n[t.kind]++;
-        cudaEventDestroy(t.e0);
-        cudaEventDestroy(t.e1);
     }
     h->timed.clear();
     if (das_ms) *das_ms = ms[0];
@@ -502,7 +477,7 @@ int64_t min_stream_samples(const bflk_handle *h, int n_frames) {
 // the last step has succeeded, so a failed build is retried (and reported again) by the next call.
 int ensure_tiles(bflk_handle *h, int fast, int want_warps) {
     if (h->tiles_valid && h->tiles_fast == fast && h->tiles_want_warps == want_warps) return BFLK_OK;
-    if (h->caller_event) BFLK_CUDA(h, cudaEventSynchronize(h->caller_event));   // a queued kernel may still read the old tables
+    BFLK_CUDA(h, cudaEventSynchronize(h->caller_event));   // a queued kernel may still read the old tables
     h->tiles_valid = false;
     h->tiles_fast = fast;
     h->tiles_want_warps = want_warps;
@@ -576,7 +551,7 @@ extern "C" {
 // Builds (once per grid / mask / range) the direction tiles and per-lane tables of the lane-broadcast kernel.
 static int ensure_bcast(bflk_handle *h) {
     if (h->bcast_valid) return BFLK_OK;
-    if (h->caller_event) BFLK_CUDA(h, cudaEventSynchronize(h->caller_event));   // a queued kernel may still read the old tables
+    BFLK_CUDA(h, cudaEventSynchronize(h->caller_event));   // a queued kernel may still read the old tables
     const int first = h->dir_first, count = h->dir_count;
     std::vector<int32_t> globals;
     if (h->rows > 0 && h->cols > 0) {
@@ -664,7 +639,6 @@ int bflk::tiled_form(const bflk_handle *h) {
 }
 
 int bflk::note_use(bflk_handle *h, cudaStream_t st, bool overlapped) {
-    if (!h->caller_event) BFLK_CUDA(h, cudaEventCreateWithFlags(&h->caller_event, cudaEventDisableTiming));
     BFLK_CUDA(h, cudaEventRecord(h->caller_event, st));
     h->last_stream = st;
     h->caller_event_is_overlapped = overlapped;
@@ -672,17 +646,13 @@ int bflk::note_use(bflk_handle *h, cudaStream_t st, bool overlapped) {
 }
 
 int bflk::lanes_fork(bflk_handle *h, cudaEvent_t after, int only) {
-    for (int i = 0; i < 2; i++) {
-        if (!h->lane[i]) BFLK_CUDA(h, cudaStreamCreateWithFlags(&h->lane[i], cudaStreamNonBlocking));
-        if (!h->lane_done[i]) BFLK_CUDA(h, cudaEventCreateWithFlags(&h->lane_done[i], cudaEventDisableTiming));
-    }
     // tables first (ensure_tiles synchronises the handle's stream when it has to build them), before anything is queued
     const int form = tiled_form(h);
     if (form >= 0) {
         int rc = ensure_tiles(h, form, 0);
         if (rc) return rc;
     }
-    const bool wait_caller = h->caller_event && !(only >= 0 && h->caller_event_is_overlapped);
+    const bool wait_caller = !(only >= 0 && h->caller_event_is_overlapped);
     for (int i = 0; i < 2; i++) {
         if (only >= 0 && i != only) continue;
         if (after) BFLK_CUDA(h, cudaStreamWaitEvent(h->lane[i], after, 0));
@@ -712,7 +682,7 @@ int bflk::power_map_dev(bflk_handle *h, const float *stream_dev, int64_t row_str
     BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
     cudaStream_t st = launch.st ? launch.st : h->stream;
     // the packed rows, partial sums and tables are the handle's: a call on another stream than the previous one waits for it
-    if (!launch.pipelined && h->caller_event && h->last_stream != st) BFLK_CUDA(h, cudaStreamWaitEvent(st, h->caller_event, 0));
+    if (!launch.pipelined && h->last_stream != st) BFLK_CUDA(h, cudaStreamWaitEvent(st, h->caller_event, 0));
     struct Mark {   // every exit after this point leaves an event behind on the stream the call used
         bflk_handle *h;
         cudaStream_t st;
@@ -871,8 +841,6 @@ int bflk::power_map_dev_overlapped(bflk_handle *h, const float *stream_dev, int6
     if (form < 0 || !h->tiles_usable || (row_stride & 1) || ((uintptr_t)stream_dev & 7))
         return power_map_dev(h, stream_dev, row_stride, n_samples, n_frames, power_dev, Launch{caller});
     const int slot = (int)(h->dev_seq++ & 1);
-    for (int i = 0; i < 2; i++)
-        if (!h->dev_in[i]) BFLK_CUDA(h, cudaEventCreateWithFlags(&h->dev_in[i], cudaEventDisableTiming));
     // this batch's kernels wait for (a) the caller's stream having reached this call (its inputs), (b) whatever used the handle's
     // scratch on another stream before the overlapped batches began.  Earlier overlapped batches need no wait: the same
     // set's previous batch ran on this very lane, the other set's batch shares nothing with this one.
@@ -906,7 +874,7 @@ int bflk_power_map_batch_dev_join(bflk_handle *h, void *cuda_stream) {
     if (!h) return BFLK_ERR_INVALID;
     BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
     cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : h->stream;
-    if (h->caller_event && h->last_stream && h->last_stream != st) BFLK_CUDA(h, cudaStreamWaitEvent(st, h->caller_event, 0));
+    if (h->last_stream != st) BFLK_CUDA(h, cudaStreamWaitEvent(st, h->caller_event, 0));
     return BFLK_OK;
 }
 
@@ -973,11 +941,10 @@ static int host_chunks(bflk_handle *h, const HostSamples &in, int64_t n_samples,
     const int N = h->cfg.frame_len;
     const int n_chunks = (n_frames + chunk_frames - 1) / chunk_frames;
     const int64_t tail = frame_tail_samples(h);
-    if (!h->copy_stream) BFLK_CUDA(h, cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking));
     while ((int)h->chunk_events.size() < n_chunks) {
-        cudaEvent_t e;
-        BFLK_CUDA(h, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-        h->chunk_events.push_back(e);
+        Event e;
+        if (!e) return h->fail(BFLK_ERR_CUDA, "cannot create the chunk events: %s", cudaGetErrorString(cudaGetLastError()));
+        h->chunk_events.push_back(std::move(e));
     }
     if (reuse_after) BFLK_CUDA(h, cudaStreamWaitEvent(h->copy_stream, reuse_after, 0));
     const bool lanes = in.lanes && n_chunks > 1;
@@ -1080,9 +1047,8 @@ int bflk_power_map_batch_submit(bflk_handle *h, const float *stream, int64_t n_s
     while (h->async_pending >= 2)
         if ((rc = bflk_power_map_batch_wait(h))) return rc;
     const int slot = (int)(h->async_seq & 1);
-    if (!h->async_done[slot]) BFLK_CUDA(h, cudaEventCreateWithFlags(&h->async_done[slot], cudaEventDisableTiming));
     rc = host_batch_enqueue(h, stream, n_samples, n_frames, power_out, h->d_async_in[slot], h->d_async_out[slot],
-                            h->async_seq >= 2 ? h->async_done[slot] : nullptr);
+                            h->async_seq >= 2 ? (cudaEvent_t)h->async_done[slot] : nullptr);
     if (rc) return rc;
     BFLK_CUDA(h, cudaEventRecord(h->async_done[slot], h->stream));
     h->async_seq++;
@@ -1096,11 +1062,12 @@ int bflk_power_map_batch(bflk_handle *h, const float *stream, int64_t n_samples,
     int rc = host_batch_check(h, stream, n_samples, n_frames, power_out);
     if (rc) return rc;
     BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
-    rc = host_batch_enqueue(h, stream, n_samples, n_frames, power_out, h->d_window, h->d_power, nullptr);
+    h->last_map_on_device = false;
+    rc = host_batch_enqueue(h, stream, n_samples, n_frames, power_out, h->d_window, h->d_maps, nullptr);
     if (rc) return rc;
     BFLK_CUDA(h, cudaStreamSynchronize(h->stream));
     h->async_pending = 0;                    // everything queued on the stream before this call has completed too
-    h->last_map_on_device = n_frames == 1;   // d_power[0 .. count) is the map: bflk_targets(NULL) / bflk_heatmap(NULL) use it
+    h->last_map_on_device = n_frames == 1;   // d_maps[0 .. count) is the map: bflk_targets(NULL) / bflk_heatmap(NULL) use it
     return BFLK_OK;
 }
 
@@ -1134,7 +1101,8 @@ int bflk_power_map_batch_i32(bflk_handle *h, const int32_t *frames, int64_t n_sa
     BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
     const int C = h->cfg.n_channels, N = h->cfg.frame_len;
     BFLK_CUDA(h, h->d_wire.reserve((size_t)C * n_samples));
-    BFLK_CUDA(h, h->d_power.reserve((size_t)n_frames * h->dir_count));
+    h->last_map_on_device = false;
+    BFLK_CUDA(h, h->d_maps.reserve((size_t)n_frames * h->dir_count));
     int chunk_frames = n_frames;
     if ((rc = host_chunk_frames(h, n_frames, &chunk_frames))) return rc;
     HostSamples in;
@@ -1153,8 +1121,9 @@ int bflk_power_map_batch_i32(bflk_handle *h, const int32_t *frames, int64_t n_sa
         return cudaMemcpyAsync(dev + (size_t)t0 * C, frames + (size_t)t0 * C, (size_t)(t1 - t0) * C * sizeof(int32_t),
                                cudaMemcpyHostToDevice, st);
     };
-    if ((rc = host_chunks(h, in, n_samples, n_frames, chunk_frames, h->d_power.p, power_out, nullptr))) return rc;
+    if ((rc = host_chunks(h, in, n_samples, n_frames, chunk_frames, h->d_maps.p, power_out, nullptr))) return rc;
     BFLK_CUDA(h, cudaStreamSynchronize(h->stream));
+    h->last_map_on_device = n_frames == 1;
     return BFLK_OK;
 }
 
@@ -1180,7 +1149,7 @@ int bflk_set_window(bflk_handle *h, const float *window) {
     BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
     const size_t n_in = (size_t)h->cfg.n_channels * h->cfg.window_len;
     BFLK_CUDA(h, h->d_resident.reserve(n_in));
-    if (h->caller_event) BFLK_CUDA(h, cudaEventSynchronize(h->caller_event));   // a caller's stream may still read the old one
+    BFLK_CUDA(h, cudaEventSynchronize(h->caller_event));   // a caller's stream may still read the old one
     BFLK_CUDA(h, cudaMemcpyAsync(h->d_resident.p, window, n_in * sizeof(float), cudaMemcpyHostToDevice, h->stream));
     BFLK_CUDA(h, cudaStreamSynchronize(h->stream));
     h->resident_window = h->d_resident.p;
@@ -1206,7 +1175,7 @@ static int miso_launch(bflk_handle *h, const double *theta, const double *phi, i
     } else {
         BFLK_CUDA(h, h->p_trig.reserve(n_targets));
         BFLK_CUDA(h, h->d_trig.reserve(n_targets));
-        if (h->caller_event) BFLK_CUDA(h, cudaEventSynchronize(h->caller_event));   // the previous call's copy is done with the staging
+        BFLK_CUDA(h, cudaEventSynchronize(h->caller_event));   // the previous call's copy is done with the staging
         for (int i = 0; i < n_targets; i++) h->p_trig.p[i] = make_trig(theta[i], phi[i]);
         BFLK_CUDA(h, cudaMemcpyAsync(h->d_trig.p, h->p_trig.p, n_targets * sizeof(DirTrig), cudaMemcpyHostToDevice, st));
         a.trig = h->d_trig.p;
@@ -1214,7 +1183,7 @@ static int miso_launch(bflk_handle *h, const double *theta, const double *phi, i
     if (power_dev) {
         const size_t slots = (size_t)n_targets * das_miso_slices(N);
         if (slots > h->d_miso_partial.n || (size_t)n_targets > h->d_miso_counters.n) {
-            if (h->caller_event) BFLK_CUDA(h, cudaEventSynchronize(h->caller_event));
+            BFLK_CUDA(h, cudaEventSynchronize(h->caller_event));
             BFLK_CUDA(h, h->d_miso_partial.reserve(slots));
             const size_t had = h->d_miso_counters.n;
             BFLK_CUDA(h, h->d_miso_counters.reserve(std::max<size_t>(n_targets, 256)));
@@ -1266,7 +1235,7 @@ int bflk_miso_dev(bflk_handle *h, const double *theta, const double *phi, int32_
     const size_t TC = (size_t)n_targets * C;
     BFLK_CUDA(h, h->d_soff.reserve(TC));
     BFLK_CUDA(h, h->d_sfrac.reserve(TC));
-    if (h->caller_event) BFLK_CUDA(h, cudaEventSynchronize(h->caller_event));
+    BFLK_CUDA(h, cudaEventSynchronize(h->caller_event));
     int32_t max_delay = 0;
     int rc = run_steer_tables(h, theta, phi, n_targets, h->d_soff.p, h->d_sfrac.p, &max_delay);  // Particle::steer
     if (rc) return rc;
@@ -1306,14 +1275,14 @@ int bflk_miso(bflk_handle *h, const double *theta, const double *phi, int32_t n_
     const float *wdev = h->resident_window;
     if (window) {
         BFLK_CUDA(h, h->d_window.reserve(n_in));
-        if (h->caller_event) BFLK_CUDA(h, cudaEventSynchronize(h->caller_event));
+        BFLK_CUDA(h, cudaEventSynchronize(h->caller_event));
         BFLK_CUDA(h, cudaMemcpyAsync(h->d_window.p, window, n_in * sizeof(float), cudaMemcpyHostToDevice, h->stream));
         wdev = h->d_window.p;
     }
     // device output block [flag | audio | power] -> ONE copy into pinned staging -> the caller's buffers
     const size_t n_audio = audio_out ? (size_t)n_targets * N : 0, n_power = power_out ? n_targets : 0, n_all = 1 + n_audio + n_power;
     if (n_all > h->d_miso_out.n) {
-        if (h->caller_event) BFLK_CUDA(h, cudaEventSynchronize(h->caller_event));
+        BFLK_CUDA(h, cudaEventSynchronize(h->caller_event));
         BFLK_CUDA(h, h->d_miso_out.reserve(n_all));
         BFLK_CUDA(h, cudaMemsetAsync(h->d_miso_out.p, 0, sizeof(float), h->stream));   // the range flag starts clear
     }
@@ -1437,12 +1406,12 @@ int bflk_heatmap(bflk_handle *h, const float *power, int32_t n, uint8_t *heat, i
     if (n <= 0 || (!power && !(h->last_map_on_device && n == h->dir_count)))
         return h->fail(BFLK_ERR_INVALID, "bflk_heatmap: null / empty map (and no map of that size left on the device)");
     BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
-    BFLK_CUDA(h, h->d_power.reserve(n));
+    if (power) BFLK_CUDA(h, h->d_post.reserve(n));
     BFLK_CUDA(h, h->d_misc.reserve(4 + (n + 3) / 4));
     BFLK_CUDA(h, h->p_misc.reserve(4));
     uint8_t *d_heat = reinterpret_cast<uint8_t *>(h->d_misc.p + 4);
-    if (power) BFLK_CUDA(h, cudaMemcpyAsync(h->d_power.p, power, n * sizeof(float), cudaMemcpyHostToDevice, h->stream));
-    BFLK_CUDA(h, launch_heatmap(h->d_power.p, n, d_heat, h->d_misc.p, reinterpret_cast<float *>(h->d_misc.p + 1), h->stream));
+    if (power) BFLK_CUDA(h, cudaMemcpyAsync(h->d_post.p, power, n * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+    BFLK_CUDA(h, launch_heatmap(power ? h->d_post.p : h->d_maps.p, n, d_heat, h->d_misc.p, reinterpret_cast<float *>(h->d_misc.p + 1), h->stream));
     h->launches++;
     BFLK_CUDA(h, cudaMemcpyAsync(h->p_misc.p, h->d_misc.p, 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
     if (heat) BFLK_CUDA(h, cudaMemcpyAsync(heat, d_heat, n, cudaMemcpyDeviceToHost, h->stream));
@@ -1498,14 +1467,14 @@ int bflk_targets(bflk_handle *h, const float *power, int32_t max_targets, float 
     if (!power && !h->last_map_on_device) return h->fail(BFLK_ERR_STATE, "bflk_targets: no map given and none left on the device by bflk_power_map");
     BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
     const int D = h->n_dir;
-    BFLK_CUDA(h, h->d_power.reserve(D));
+    if (power) BFLK_CUDA(h, h->d_post.reserve(D));
     BFLK_CUDA(h, h->d_bytes.reserve(D));
     BFLK_CUDA(h, h->d_misc.reserve(3 * (size_t)max_targets + 1));
     BFLK_CUDA(h, h->p_misc.reserve(3 * (size_t)max_targets + 1));
-    if (power) BFLK_CUDA(h, cudaMemcpyAsync(h->d_power.p, power, D * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+    if (power) BFLK_CUDA(h, cudaMemcpyAsync(h->d_post.p, power, D * sizeof(float), cudaMemcpyHostToDevice, h->stream));
     int32_t *d_index = h->d_misc.p, *d_n = h->d_misc.p + 3 * max_targets;
     float *d_pw = reinterpret_cast<float *>(h->d_misc.p + max_targets), *d_prob = reinterpret_cast<float *>(h->d_misc.p + 2 * max_targets);
-    BFLK_CUDA(h, launch_map_targets(h->d_power.p, h->rows, h->cols, max_targets, min_rel_power, h->d_bytes.p, d_index, d_pw, d_prob, d_n, h->stream));
+    BFLK_CUDA(h, launch_map_targets(power ? h->d_post.p : h->d_maps.p, h->rows, h->cols, max_targets, min_rel_power, h->d_bytes.p, d_index, d_pw, d_prob, d_n, h->stream));
     h->launches++;
     BFLK_CUDA(h, cudaMemcpyAsync(h->p_misc.p, h->d_misc.p, (3 * (size_t)max_targets + 1) * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
     BFLK_CUDA(h, cudaStreamSynchronize(h->stream));
@@ -1531,13 +1500,14 @@ int bflk_calibrate(bflk_handle *h, const float *signals, int32_t window_len, flo
     if (!signals || window_len <= 0 || !index || !usable) return h->fail(BFLK_ERR_INVALID, "bflk_calibrate: null arguments");
     BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
     const int E = 64;  // ELEMENTS, antenna.h:20
+    BFLK_CUDA(h, cudaEventSynchronize(h->caller_event));   // a caller's stream may still use d_window
     BFLK_CUDA(h, h->d_window.reserve((size_t)E * window_len));
-    BFLK_CUDA(h, h->d_power.reserve(E));
+    BFLK_CUDA(h, h->d_post.reserve(E));
     BFLK_CUDA(h, h->p_out.reserve(E));
     BFLK_CUDA(h, cudaMemcpyAsync(h->d_window.p, signals, (size_t)E * window_len * sizeof(float), cudaMemcpyHostToDevice, h->stream));
-    BFLK_CUDA(h, launch_channel_power(h->d_window.p, E, window_len, h->d_power.p, h->stream));
+    BFLK_CUDA(h, launch_channel_power(h->d_window.p, E, window_len, h->d_post.p, h->stream));
     h->launches++;
-    BFLK_CUDA(h, cudaMemcpyAsync(h->p_out.p, h->d_power.p, E * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+    BFLK_CUDA(h, cudaMemcpyAsync(h->p_out.p, h->d_post.p, E * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
     BFLK_CUDA(h, cudaStreamSynchronize(h->stream));
     const float *power = h->p_out.p;
     // median gate, aw_processing_unit.cpp:144-185 (the "median" is (m[32] + m[33]) / 2 as written there)
@@ -1572,6 +1542,7 @@ int bflk_ingest_i32(bflk_handle *h, const int32_t *frames, int32_t n, int32_t n_
         return h->fail(BFLK_ERR_INVALID, "bflk_ingest_i32: null buffers or n_sensors not a multiple of 8");
     BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
     const size_t cnt = (size_t)n * n_sensors;
+    BFLK_CUDA(h, cudaEventSynchronize(h->caller_event));   // a caller's stream may still use d_window
     BFLK_CUDA(h, h->d_misc.reserve(cnt));
     BFLK_CUDA(h, h->d_window.reserve(cnt));
     BFLK_CUDA(h, cudaMemcpyAsync(h->d_misc.p, frames, cnt * sizeof(int32_t), cudaMemcpyHostToDevice, h->stream));

@@ -106,55 +106,76 @@ struct BcastGeometry {
     int row_bytes = 0;
 };
 
-template <typename T>
-struct DevBuf {
+// n elements of T in device memory (cudaMalloc) or page-locked host memory (cudaMallocHost), freed by the destructor.
+// Move-only.  reserve only grows: it frees the old block before it allocates the new one, and leaves n = 0 on failure.
+enum class Mem { device, pinned };
+template <typename T, Mem kind>
+struct Buf {
     T *p = nullptr;
     size_t n = 0;
+    Buf() = default;
+    Buf(Buf &&o) noexcept : p(o.p), n(o.n) { o.p = nullptr; o.n = 0; }
+    Buf &operator=(Buf &&o) noexcept { std::swap(p, o.p); std::swap(n, o.n); return *this; }
+    ~Buf() { reset(); }
     cudaError_t reserve(size_t count) {
         if (count <= n) return cudaSuccess;
-        if (p) cudaFree(p);
-        p = nullptr;
-        n = 0;
-        cudaError_t e = cudaMalloc((void **)&p, count * sizeof(T));
+        reset();
+        cudaError_t e = kind == Mem::device ? cudaMalloc((void **)&p, count * sizeof(T)) : cudaMallocHost((void **)&p, count * sizeof(T));
         if (e == cudaSuccess) n = count;
+        else p = nullptr;
         return e;
     }
-    void release() {
-        if (p) cudaFree(p);
+  private:
+    void reset() {
+        if (p) kind == Mem::device ? cudaFree(p) : cudaFreeHost(p);
         p = nullptr;
         n = 0;
     }
 };
+template <typename T> using DevBuf = Buf<T, Mem::device>;
+template <typename T> using PinBuf = Buf<T, Mem::pinned>;
 
-template <typename T>
-struct PinBuf {
-    T *p = nullptr;
-    size_t n = 0;
-    cudaError_t reserve(size_t count) {
-        if (count <= n) return cudaSuccess;
-        if (p) cudaFreeHost(p);
-        p = nullptr;
-        n = 0;
-        cudaError_t e = cudaMallocHost((void **)&p, count * sizeof(T));
-        if (e == cudaSuccess) n = count;
-        return e;
+// A non-blocking stream and an event, created by the constructor of the object that owns them and destroyed with it.
+// A failed creation leaves a null handle and the error in cudaGetLastError(), which the owner's creator checks.  A stream
+// is synchronised before it is destroyed.  An event that was never recorded is an empty set of work: waiting for it
+// returns at once.
+class Stream {
+  public:
+    Stream() { if (cudaStreamCreateWithFlags(&s_, cudaStreamNonBlocking) != cudaSuccess) s_ = nullptr; }
+    Stream(const Stream &) = delete;
+    Stream &operator=(const Stream &) = delete;
+    ~Stream() {
+        sync();
+        if (s_) cudaStreamDestroy(s_);
     }
-    void release() {
-        if (p) cudaFreeHost(p);
-        p = nullptr;
-        n = 0;
-    }
+    void sync() const { if (s_) cudaStreamSynchronize(s_); }
+    operator cudaStream_t() const { return s_; }
+  private:
+    cudaStream_t s_ = nullptr;
+};
+
+class Event {   // move-only
+  public:
+    Event() : Event(cudaEventDisableTiming) {}
+    explicit Event(unsigned flags) { if (cudaEventCreateWithFlags(&e_, flags) != cudaSuccess) e_ = nullptr; }
+    Event(Event &&o) noexcept : e_(o.e_) { o.e_ = nullptr; }
+    Event &operator=(Event &&o) noexcept { std::swap(e_, o.e_); return *this; }
+    ~Event() { if (e_) cudaEventDestroy(e_); }
+    operator cudaEvent_t() const { return e_; }
+  private:
+    cudaEvent_t e_ = nullptr;
 };
 
 }  // namespace bflk
 
 struct bflk_comm;   // multi.cu: NCCL communicator state of a handle that is one rank of a multi-GPU job
 
+// Created on its device by bflk_create, with all of its streams and events; bflk_destroy deletes it on that device.
 struct bflk_handle {
     bflk_config cfg{};
     bflk::Tuning tuning;
     bflk_comm *comm = nullptr;
-    cudaStream_t stream = nullptr;
+    bflk::Stream stream;
     int sm_count = 0;
     std::string error;
     int64_t launches = 0;
@@ -208,49 +229,57 @@ struct bflk_handle {
     bflk::DevBuf<uint8_t> d_bytes;            // heat-map / resize / peak-candidate scratch
     // bflk_power_map_batch_submit / _wait: two batches in flight, each with its own device buffers
     bflk::DevBuf<float> d_async_in[2], d_async_out[2];
-    cudaEvent_t async_done[2] = {nullptr, nullptr};
+    bflk::Event async_done[2];
     uint64_t async_seq = 0;
     int async_pending = 0;
-    bool last_map_on_device = false;          // d_power holds the [count] map of the last single-frame call
+    // maps of the synchronous host batches (bflk_power_map_batch, bflk_power_map_batch_i32); nothing else writes them
+    bflk::DevBuf<float> d_maps;
+    bool last_map_on_device = false;          // d_maps holds the [count] map of the last batch, which had one frame
+    bflk::DevBuf<float> d_post;               // host map of bflk_heatmap / bflk_targets, channel powers of bflk_calibrate
     bflk::DevBuf<float> d_resident;
     bflk::DevBuf<float> d_miso_out;           // [flag | audio | power]: one D2H copy per call
     bflk::DevBuf<float> d_miso_partial;
     bflk::DevBuf<unsigned> d_miso_counters;
     int32_t miso_epoch = 0;
     bflk::PinBuf<float> p_stage;              // pinned staging of single-frame inputs / small outputs
-    cudaEvent_t caller_event = nullptr;       // orders work the library puts on a caller's stream against the handle's scratch
+    bflk::Event caller_event;                 // orders work the library puts on a caller's stream against the handle's scratch
     cudaStream_t last_stream = nullptr;       // stream of the last asynchronous call
 
     // scratch
-    bflk::DevBuf<float> d_window, d_power, d_audio;
+    bflk::DevBuf<float> d_window;
     bflk::DevBuf<bflk::DirTrig> d_trig;
     bflk::DevBuf<int32_t> d_soff;
     bflk::DevBuf<float> d_sfrac;
     bflk::DevBuf<int32_t> d_misc;
-    bflk::PinBuf<float> p_in, p_out;
+    bflk::PinBuf<float> p_out;
     bflk::PinBuf<bflk::DirTrig> p_trig;
     bflk::PinBuf<int32_t> p_misc;
     // host-buffer batches are cut into chunks: copies on copy_stream overlap compute on stream
-    cudaStream_t copy_stream = nullptr;
-    std::vector<cudaEvent_t> chunk_events;
+    bflk::Stream copy_stream;
+    std::vector<bflk::Event> chunk_events;    // grows with the chunk count of a batch
     // ... and the chunks' kernels alternate between two compute lanes (lanes_fork / lanes_join), each with its own scratch
     // set: a launch on its own ends with half a CTA lifetime of idle SMs on average (the CTAs of a launch all take equally
     // long and the SMs drift apart), which the next chunk's CTAs fill when they do not have to wait for it
-    cudaStream_t lane[2] = {nullptr, nullptr};
-    cudaEvent_t lane_done[2] = {nullptr, nullptr};
+    bflk::Stream lane[2];
+    bflk::Event lane_done[2];
     struct {
         bflk::DevBuf<char> packed;     // pair-interleaved staging rows of the current batch
         bflk::DevBuf<float> partial;   // partial sums of frames longer than one block
     } scratch[2];                      // set 1 only for lane 1 (Launch::scratch)
     // device batches in continuous operation (power_map_dev_overlapped): they alternate between the two lanes too
-    cudaEvent_t dev_in[2] = {nullptr, nullptr};   // "the caller's stream has reached the submit" (inputs ready)
+    bflk::Event dev_in[2];                        // "the caller's stream has reached the submit" (inputs ready)
     uint64_t dev_seq = 0;
     bool caller_event_is_overlapped = false;      // the latest caller_event covers overlapped batches only (see power_map_dev_overlapped)
 
     // optional kernel timing (bflk_enable_timing): event pairs recorded on the launching stream
     bool timing = false;
-    struct Timed { cudaEvent_t e0, e1; int kind; };  // kind 0: delay-and-sum kernel, 1: pack pre-pass
+    struct Timed {
+        bflk::Event e0{cudaEventDefault}, e1{cudaEventDefault};
+        int kind = 0;   // 0: delay-and-sum kernel, 1: pack pre-pass
+    };
     std::vector<Timed> timed;
+
+    ~bflk_handle();   // waits for the handle's and its communicator's streams before anything is freed
 
     int fail(int code, const char *fmt, ...) {
         char buf[512];
@@ -439,6 +468,6 @@ int64_t min_stream_samples(const bflk_handle *h, int n_frames);
 // frame needs beyond its own N
 int host_chunk_frames(bflk_handle *h, int n_frames, int *chunk_frames);
 int64_t frame_tail_samples(const bflk_handle *h);
-void comm_release(bflk_handle *h);   // multi.cu
+void comm_release(bflk_handle *h);   // multi.cu: deletes h->comm (bflk_comm is a complete type only there)
 
 }  // namespace bflk

@@ -21,6 +21,7 @@
 
 #include <algorithm>
 #include <cstring>
+#include <memory>
 #include <mutex>
 
 #include "bflk_internal.h"
@@ -83,42 +84,56 @@ constexpr int kRing = 3;   // chunk buffers of the host path: upload / replicate
 
 }  // namespace
 
+// One set of a rank's map buffers.  A handle has two: the synchronous calls use set 0;
+// bflk_power_map_batch_sharded_dev_submit alternates, so the kernels of batch i + 1 fill one set while the all-gather of
+// batch i still reads the other.
+struct MapSet {
+    DevBuf<float> local;    // [nf][count] tight output of this rank's kernel when the shard is ragged
+    DevBuf<float> send;     // [nf_max][per] what the all-gather sends
+    DevBuf<float> gather;   // [G][nf_max][per]
+    Event computed;         // the set's kernels are done (the all-gather may start)
+    Event gathered;         // the set's all-gather + assembly are done (set reusable, maps complete)
+};
+
+// Created on the handle's device by init_comms, with all of its streams and events.
 struct bflk_comm {
     nccl_comm_t all = nullptr;   // every rank
     nccl_comm_t sub = nullptr;   // the G_d ranks that share this rank's frame slice (== all when G_f == 1; null when G_d == 1)
     int n_ranks = 1, rank = 0, gd = 1, gf = 1, dgrp = 0, fgrp = 0;
     int planned_dirs = -1;       // grid size the direction range was set for
-    // two sets: the synchronous calls use set 0; bflk_power_map_batch_sharded_dev_submit alternates, so the kernels of
-    // batch i + 1 fill one set while the all-gather of batch i still reads the other
-    DevBuf<float> d_local_[2];   // [nf][count] tight output of this rank's kernel when the shard is ragged
-    DevBuf<float> d_send_[2];    // [nf_max][per] what the all-gather sends
-    DevBuf<float> d_gather_[2];  // [G][nf_max][per]
-    int slot = 0;                // set in use by the call being enqueued
-    DevBuf<float> &d_local() { return d_local_[slot]; }
-    DevBuf<float> &d_send() { return d_send_[slot]; }
-    DevBuf<float> &d_gather() { return d_gather_[slot]; }
-    cudaStream_t gather_stream = nullptr;                    // collectives of submitted device batches
-    cudaEvent_t ev_computed[2] = {nullptr, nullptr};         // a set's kernels are done (gather may start)
-    cudaEvent_t ev_gathered[2] = {nullptr, nullptr};         // a set's all-gather + assembly are done (set reusable, maps complete)
-    bool gathered_recorded[2] = {false, false};
+    MapSet sets[2];
+    Stream gather_stream;        // collectives of submitted device batches
     uint64_t dev_seq = 0;
     DevBuf<float> d_all;         // [B][D] assembled maps (host variant)
     DevBuf<float> d_slice[kRing];   // [C / G_d][Tj] rows this rank uploads
     DevBuf<float> d_chunk[kRing];   // [C][Tj] replicated chunk
     DevBuf<int32_t> d_agree;
-    cudaEvent_t ev_up[kRing] = {nullptr, nullptr, nullptr}, ev_done[kRing] = {nullptr, nullptr, nullptr};
-    bool ev_done_recorded[kRing] = {false, false, false};
-    cudaEvent_t ev_async = nullptr;   // end of the last submitted (not yet waited for) host batch
-    cudaEvent_t ev_fork = nullptr;    // start of a host batch on the handle's stream: its two lanes wait for it
+    Event ev_up[kRing], ev_done[kRing];
+    Event ev_async;              // end of the last submitted (not yet waited for) host batch
+    Event ev_fork;               // start of a host batch on the handle's stream: its two lanes wait for it
     int async_pending = 0;
-    cudaStream_t copy_stream = nullptr;
+    Stream copy_stream;
     int agreed_for_frames = -1, agreed_chunk = 0;   // chunking the ranks of a frame group agreed on
     int64_t collectives = 0;
+
+    // ~bflk_handle and init_comms wait for the handle's streams first: once these two are done too, no work of this rank
+    // still uses the communicators or the buffers
+    ~bflk_comm() {
+        gather_stream.sync();
+        copy_stream.sync();
+        if (nccl().ok()) {
+            if (sub && sub != all) nccl().CommDestroy(sub);
+            if (all) nccl().CommDestroy(all);
+        }
+    }
 };
 
 struct bflk_group {
     std::vector<bflk_handle *> hs;
     std::string error;
+    ~bflk_group() {
+        for (bflk_handle *h : hs) bflk_destroy(h);
+    }
 };
 
 #define BFLK_NCCL(h, expr)                                                                                          \
@@ -197,43 +212,39 @@ int check_sharded(bflk_handle *h, const char *who) {
     return BFLK_OK;
 }
 
-// local compute of one rank: its direction slice of frames [f0, f0 + nf) of a device-resident stream into c->d_send
-int compute_shard(bflk_handle *h, const Plan &p, const float *stream_dev, int64_t row_stride, int64_t n_samples, int f_rel0,
-                  int nf, int out_row0, const Launch &launch) {
-    bflk_comm *c = h->comm;
+// local compute of one rank: its direction slice of frames [f0, f0 + nf) of a device-resident stream into set.send
+int compute_shard(bflk_handle *h, const Plan &p, MapSet &set, const float *stream_dev, int64_t row_stride, int64_t n_samples,
+                  int f_rel0, int nf, int out_row0, const Launch &launch) {
     if (nf <= 0 || p.dir_count <= 0) return BFLK_OK;
     const int N = h->cfg.frame_len;
     const bool tight = p.dir_count == p.dir_per;
-    float *out = tight ? c->d_send().p + (size_t)out_row0 * p.dir_per : c->d_local().p + (size_t)out_row0 * p.dir_count;
+    float *out = tight ? set.send.p + (size_t)out_row0 * p.dir_per : set.local.p + (size_t)out_row0 * p.dir_count;
     int rc = power_map_dev(h, stream_dev + (size_t)f_rel0 * N, row_stride, n_samples - (int64_t)f_rel0 * N, nf, out, launch);
     if (rc) return rc;
     if (!tight)
-        BFLK_CUDA(h, cudaMemcpy2DAsync(c->d_send().p + (size_t)out_row0 * p.dir_per, (size_t)p.dir_per * sizeof(float), out,
+        BFLK_CUDA(h, cudaMemcpy2DAsync(set.send.p + (size_t)out_row0 * p.dir_per, (size_t)p.dir_per * sizeof(float), out,
                                        (size_t)p.dir_count * sizeof(float), (size_t)p.dir_count * sizeof(float), nf,
                                        cudaMemcpyDeviceToDevice, launch.st));
     return BFLK_OK;
 }
 
-int reserve_maps(bflk_handle *h, const Plan &p, int B, bool need_all) {
+int reserve_maps(bflk_handle *h, const Plan &p, MapSet &set, int B, bool need_all) {
     bflk_comm *c = h->comm;
     const size_t slice = (size_t)p.frame_per * p.dir_per;
-    const bool grows = slice > c->d_send().n || slice * c->n_ranks > c->d_gather().n ||
-                       (p.dir_count != p.dir_per && (size_t)p.frame_per * p.dir_count > c->d_local().n);
-    if (grows && c->gathered_recorded[c->slot]) {   // a submitted batch may still use the set that is about to be reallocated
-        BFLK_CUDA(h, cudaEventSynchronize(c->ev_gathered[c->slot]));
-        c->gathered_recorded[c->slot] = false;
-    }
-    BFLK_CUDA(h, c->d_send().reserve(slice));
-    BFLK_CUDA(h, c->d_gather().reserve(slice * c->n_ranks));
-    if (p.dir_count != p.dir_per) BFLK_CUDA(h, c->d_local().reserve((size_t)p.frame_per * p.dir_count));
+    const bool grows = slice > set.send.n || slice * c->n_ranks > set.gather.n ||
+                       (p.dir_count != p.dir_per && (size_t)p.frame_per * p.dir_count > set.local.n);
+    if (grows) BFLK_CUDA(h, cudaEventSynchronize(set.gathered));   // a submitted batch may still use the set
+    BFLK_CUDA(h, set.send.reserve(slice));
+    BFLK_CUDA(h, set.gather.reserve(slice * c->n_ranks));
+    if (p.dir_count != p.dir_per) BFLK_CUDA(h, set.local.reserve((size_t)p.frame_per * p.dir_count));
     if (need_all) BFLK_CUDA(h, c->d_all.reserve((size_t)B * h->n_dir));
     return BFLK_OK;
 }
 
 // one all-gather of the ranks' slices + assembly into out_dev[B][D]; hs = the local handles of the job (1 per process,
-// or all of them in a single-process group)
-int gather_and_assemble(const std::vector<bflk_handle *> &hs, const std::vector<Plan> &plans, int B,
-                        const std::vector<float *> &out_dev, const std::vector<cudaStream_t> &st) {
+// or all of them in a single-process group), sets[i] = the map set handle i uses
+int gather_and_assemble(const std::vector<bflk_handle *> &hs, const std::vector<Plan> &plans, const std::vector<MapSet *> &sets,
+                        int B, const std::vector<float *> &out_dev, const std::vector<cudaStream_t> &st) {
     Nccl &n = nccl();
     n.GroupStart();
     for (size_t i = 0; i < hs.size(); i++) {
@@ -241,7 +252,7 @@ int gather_and_assemble(const std::vector<bflk_handle *> &hs, const std::vector<
         bflk_comm *c = h->comm;
         cudaSetDevice(h->cfg.device);
         const size_t slice = (size_t)plans[i].frame_per * plans[i].dir_per;
-        int r = n.AllGather(c->d_send().p, c->d_gather().p, slice, kNcclFloat, c->all, st[i]);
+        int r = n.AllGather(sets[i]->send.p, sets[i]->gather.p, slice, kNcclFloat, c->all, st[i]);
         if (r != 0) {
             n.GroupEnd();
             return h->fail(BFLK_ERR_CUDA, "ncclAllGather failed: %s", n.GetErrorString(r));
@@ -256,7 +267,7 @@ int gather_and_assemble(const std::vector<bflk_handle *> &hs, const std::vector<
         BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
         const Plan &p = plans[i];
         dim3 grid((h->n_dir + 255) / 256, B);
-        assemble_kernel<<<grid, 256, 0, st[i]>>>(h->comm->d_gather().p, B, h->n_dir, p.gd, p.frame_per, p.dir_per, out_dev[i]);
+        assemble_kernel<<<grid, 256, 0, st[i]>>>(sets[i]->gather.p, B, h->n_dir, p.gd, p.frame_per, p.dir_per, out_dev[i]);
         BFLK_CUDA(h, cudaGetLastError());
         h->launches++;
     }
@@ -269,6 +280,7 @@ int gather_and_assemble(const std::vector<bflk_handle *> &hs, const std::vector<
 int sharded_dev(const std::vector<bflk_handle *> &hs, const std::vector<const float *> &stream_dev, int64_t n_samples,
                 int32_t n_frames, const std::vector<float *> &power_all_dev, const std::vector<cudaStream_t> &st, bool pipelined = false) {
     std::vector<Plan> plans(hs.size());
+    std::vector<MapSet *> sets(hs.size());
     std::vector<cudaStream_t> gst = st;
     for (size_t i = 0; i < hs.size(); i++) {
         bflk_handle *h = hs[i];
@@ -279,53 +291,43 @@ int sharded_dev(const std::vector<bflk_handle *> &hs, const std::vector<const fl
             return h->fail(BFLK_ERR_INVALID, "bflk_power_map_batch_sharded_dev: %lld samples per channel cannot hold %d frames", (long long)n_samples, n_frames);
         BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
         bflk_comm *c = h->comm;
-        c->slot = 0;
         if (pipelined) {
-            if (!c->gather_stream) BFLK_CUDA(h, cudaStreamCreateWithFlags(&c->gather_stream, cudaStreamNonBlocking));
-            for (int k = 0; k < 2; k++) {
-                if (!c->ev_computed[k]) BFLK_CUDA(h, cudaEventCreateWithFlags(&c->ev_computed[k], cudaEventDisableTiming));
-                if (!c->ev_gathered[k]) BFLK_CUDA(h, cudaEventCreateWithFlags(&c->ev_gathered[k], cudaEventDisableTiming));
-            }
-            c->slot = (int)(c->dev_seq++ & 1);
+            sets[i] = &c->sets[c->dev_seq++ & 1];
             gst[i] = c->gather_stream;
             // the batch that used this set two submits ago: its collective must be done before the kernels overwrite the set
-            if (c->gathered_recorded[c->slot]) BFLK_CUDA(h, cudaStreamWaitEvent(st[i], c->ev_gathered[c->slot], 0));
+            BFLK_CUDA(h, cudaStreamWaitEvent(st[i], sets[i]->gathered, 0));
         } else {
             // a synchronous call after submitted batches: set 0 may still be in flight on the communicator's stream
-            for (int k = 0; k < 2; k++)
-                if (c->gathered_recorded[k]) BFLK_CUDA(h, cudaStreamWaitEvent(st[i], c->ev_gathered[k], 0));
+            sets[i] = &c->sets[0];
+            for (MapSet &s : c->sets) BFLK_CUDA(h, cudaStreamWaitEvent(st[i], s.gathered, 0));
         }
         plans[i] = make_plan(h->n_dir, n_frames, c->n_ranks, c->gd, c->gf, c->rank);
         if ((rc = apply_direction_range(h, plans[i]))) return rc;
-        if ((rc = reserve_maps(h, plans[i], n_frames, false))) return rc;
+        if ((rc = reserve_maps(h, plans[i], *sets[i], n_frames, false))) return rc;
         // The kernels stay on the caller's stream.  Alternating them between the handle's two lanes as well
         // (power_map_dev_overlapped) was measured and not kept: +1.6 % on two GPUs (149.4 k vs 147.0 k maps/s) but -7.7 % on
         // eight (529.6 k vs 573.7 k): with two buffer sets, batch i + 2 waits for the all-gather of batch i, which waits for
         // kernels that then share the SMs with batch i + 1 -- a bubble per batch once a launch is only four waves.
-        if ((rc = compute_shard(h, plans[i], stream_dev[i], n_samples, n_samples, plans[i].frame_first, plans[i].frame_count, 0,
-                                Launch{st[i]}))) return rc;
+        if ((rc = compute_shard(h, plans[i], *sets[i], stream_dev[i], n_samples, n_samples, plans[i].frame_first,
+                                plans[i].frame_count, 0, Launch{st[i]}))) return rc;
         if (pipelined) {
-            BFLK_CUDA(h, cudaEventRecord(c->ev_computed[c->slot], st[i]));
-            BFLK_CUDA(h, cudaStreamWaitEvent(c->gather_stream, c->ev_computed[c->slot], 0));
+            BFLK_CUDA(h, cudaEventRecord(sets[i]->computed, st[i]));
+            BFLK_CUDA(h, cudaStreamWaitEvent(c->gather_stream, sets[i]->computed, 0));
         }
     }
-    int rc = gather_and_assemble(hs, plans, n_frames, power_all_dev, gst);
-    for (size_t i = 0; i < hs.size(); i++) {
-        bflk_comm *c = hs[i]->comm;
-        if (pipelined && rc == BFLK_OK) {
-            cudaSetDevice(hs[i]->cfg.device);
-            if (cudaEventRecord(c->ev_gathered[c->slot], c->gather_stream) == cudaSuccess) c->gathered_recorded[c->slot] = true;
+    int rc = gather_and_assemble(hs, plans, sets, n_frames, power_all_dev, gst);
+    if (pipelined && rc == BFLK_OK) {
+        for (size_t i = 0; i < hs.size(); i++) {
+            BFLK_CUDA(hs[i], cudaSetDevice(hs[i]->cfg.device));
+            BFLK_CUDA(hs[i], cudaEventRecord(sets[i]->gathered, hs[i]->comm->gather_stream));
         }
-        c->slot = 0;
     }
     return rc;
 }
 
 int sharded_dev_join(bflk_handle *h, cudaStream_t st) {
-    bflk_comm *c = h->comm;
     BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
-    for (int k = 0; k < 2; k++)
-        if (c->gathered_recorded[k]) BFLK_CUDA(h, cudaStreamWaitEvent(st, c->ev_gathered[k], 0));
+    for (MapSet &s : h->comm->sets) BFLK_CUDA(h, cudaStreamWaitEvent(st, s.gathered, 0));
     return BFLK_OK;
 }
 
@@ -374,6 +376,7 @@ int sharded_host(const std::vector<bflk_handle *> &hs, const float *stream, int6
     Nccl &n = nccl();
     const size_t G = hs.size();
     std::vector<Plan> plans(G);
+    std::vector<MapSet *> sets(G);
     for (size_t i = 0; i < G; i++) {
         bflk_handle *h = hs[i];
         int rc = check_sharded(h, "bflk_power_map_batch_sharded");
@@ -383,17 +386,12 @@ int sharded_host(const std::vector<bflk_handle *> &hs, const float *stream, int6
             return h->fail(BFLK_ERR_INVALID, "bflk_power_map_batch_sharded: %lld samples per channel cannot hold %d frames", (long long)n_samples, n_frames);
         BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
         bflk_comm *c = h->comm;
-        c->slot = 0;
-        for (int k = 0; k < 2; k++)   // device batches submitted earlier may still use buffer set 0 on the communicator's stream
-            if (c->gathered_recorded[k]) BFLK_CUDA(h, cudaStreamWaitEvent(h->stream, c->ev_gathered[k], 0));
+        sets[i] = &c->sets[0];
+        for (MapSet &s : c->sets)   // device batches submitted earlier may still use buffer set 0 on the communicator's stream
+            BFLK_CUDA(h, cudaStreamWaitEvent(h->stream, s.gathered, 0));
         plans[i] = make_plan(h->n_dir, n_frames, c->n_ranks, c->gd, c->gf, c->rank);
         if ((rc = apply_direction_range(h, plans[i]))) return rc;
-        if ((rc = reserve_maps(h, plans[i], n_frames, true))) return rc;
-        if (!c->copy_stream) BFLK_CUDA(h, cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
-        for (int k = 0; k < kRing; k++) {
-            if (!c->ev_up[k]) BFLK_CUDA(h, cudaEventCreateWithFlags(&c->ev_up[k], cudaEventDisableTiming));
-            if (!c->ev_done[k]) BFLK_CUDA(h, cudaEventCreateWithFlags(&c->ev_done[k], cudaEventDisableTiming));
-        }
+        if ((rc = reserve_maps(h, plans[i], *sets[i], n_frames, true))) return rc;
     }
     int rc = agree_on_chunk(hs, plans);
     if (rc) return rc;
@@ -438,7 +436,6 @@ int sharded_host(const std::vector<bflk_handle *> &hs, const float *stream, int6
         lanes[i] = n_chunks[i] > 1;
         if (!lanes[i]) continue;
         BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
-        if (!h->comm->ev_fork) BFLK_CUDA(h, cudaEventCreateWithFlags(&h->comm->ev_fork, cudaEventDisableTiming));
         BFLK_CUDA(h, cudaEventRecord(h->comm->ev_fork, h->stream));
         if ((rc = lanes_fork(h, h->comm->ev_fork))) return rc;
     }
@@ -453,7 +450,7 @@ int sharded_host(const std::vector<bflk_handle *> &hs, const float *stream, int6
             const Chunk k = chunk_of(i, j);
             // the compute that last used this ring buffer (an earlier chunk of this batch, or of the previous batch when
             // batches are submitted back to back) must be done before the copy overwrites it
-            if (c->ev_done_recorded[buf]) BFLK_CUDA(h, cudaStreamWaitEvent(c->copy_stream, c->ev_done[buf], 0));
+            BFLK_CUDA(h, cudaStreamWaitEvent(c->copy_stream, c->ev_done[buf], 0));
             const bool split = c->gd > 1 && C % c->gd == 0;
             if (split) {
                 const int rows = C / c->gd;
@@ -496,10 +493,10 @@ int sharded_host(const std::vector<bflk_handle *> &hs, const float *stream, int6
             cudaStream_t cs = lanes[i] ? h->lane[j & 1] : h->stream;
             BFLK_CUDA(h, cudaEventRecord(c->ev_up[buf], c->copy_stream));
             BFLK_CUDA(h, cudaStreamWaitEvent(cs, c->ev_up[buf], 0));
-            rc = compute_shard(h, plans[i], c->d_chunk[buf].p, k.pitch, k.Tj, 0, k.nfj, k.a, Launch{cs, lanes[i] ? (j & 1) : 0, (bool)lanes[i]});
+            rc = compute_shard(h, plans[i], *sets[i], c->d_chunk[buf].p, k.pitch, k.Tj, 0, k.nfj, k.a,
+                               Launch{cs, lanes[i] ? (j & 1) : 0, (bool)lanes[i]});
             if (rc) return rc;
             BFLK_CUDA(h, cudaEventRecord(c->ev_done[buf], cs));
-            c->ev_done_recorded[buf] = true;
         }
     }
     for (size_t i = 0; i < G; i++) {   // the all-gather on the handle's stream follows every chunk
@@ -513,7 +510,7 @@ int sharded_host(const std::vector<bflk_handle *> &hs, const float *stream, int6
         out_dev[i] = power_out[i] ? hs[i]->comm->d_all.p : nullptr;
         st[i] = hs[i]->stream;
     }
-    if ((rc = gather_and_assemble(hs, plans, n_frames, out_dev, st))) return rc;
+    if ((rc = gather_and_assemble(hs, plans, sets, n_frames, out_dev, st))) return rc;
     for (size_t i = 0; i < G; i++) {
         bflk_handle *h = hs[i];
         BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
@@ -527,7 +524,6 @@ int sharded_host(const std::vector<bflk_handle *> &hs, const float *stream, int6
             BFLK_CUDA(h, cudaStreamSynchronize(h->stream));
             h->comm->async_pending = 0;
         } else {
-            if (!h->comm->ev_async) BFLK_CUDA(h, cudaEventCreateWithFlags(&h->comm->ev_async, cudaEventDisableTiming));
             BFLK_CUDA(h, cudaEventRecord(h->comm->ev_async, h->stream));   // everything of this batch precedes it on the stream
             h->comm->async_pending++;
         }
@@ -541,8 +537,12 @@ int init_comms(const std::vector<bflk_handle *> &hs, const std::vector<int> &ran
     if (!resolve_groups(n_ranks, dir_groups, &gd, &gf))
         return hs[0]->fail(BFLK_ERR_INVALID, "bflk_comm_init: %d direction groups do not divide %d ranks", dir_groups, n_ranks);
     for (bflk_handle *h : hs) {
-        if (h->comm) comm_release(h);
+        BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
+        BFLK_CUDA(h, cudaStreamSynchronize(h->stream));   // the collectives of the old communicator are done
+        comm_release(h);
+        cudaGetLastError();   // clear an earlier call's error: the check below is about the new streams and events
         h->comm = new bflk_comm();
+        BFLK_CUDA(h, cudaGetLastError());
     }
     n.GroupStart();
     for (size_t i = 0; i < hs.size(); i++) {
@@ -584,34 +584,7 @@ int init_comms(const std::vector<bflk_handle *> &hs, const std::vector<int> &ran
 }  // namespace
 
 void bflk::comm_release(bflk_handle *h) {
-    bflk_comm *c = h->comm;
-    if (!c) return;
-    cudaSetDevice(h->cfg.device);
-    if (h->stream) cudaStreamSynchronize(h->stream);
-    if (c->copy_stream) {
-        cudaStreamSynchronize(c->copy_stream);
-        cudaStreamDestroy(c->copy_stream);
-    }
-    if (c->ev_async) cudaEventDestroy(c->ev_async);
-    if (c->ev_fork) cudaEventDestroy(c->ev_fork);
-    for (int k = 0; k < kRing; k++) {
-        if (c->ev_up[k]) cudaEventDestroy(c->ev_up[k]);
-        if (c->ev_done[k]) cudaEventDestroy(c->ev_done[k]);
-        c->d_slice[k].release();
-        c->d_chunk[k].release();
-    }
-    for (int k = 0; k < 2; k++) {
-        c->d_local_[k].release(); c->d_send_[k].release(); c->d_gather_[k].release();
-        if (c->ev_computed[k]) cudaEventDestroy(c->ev_computed[k]);
-        if (c->ev_gathered[k]) cudaEventDestroy(c->ev_gathered[k]);
-    }
-    if (c->gather_stream) { cudaStreamSynchronize(c->gather_stream); cudaStreamDestroy(c->gather_stream); }
-    c->d_all.release(); c->d_agree.release();
-    if (nccl().ok()) {
-        if (c->sub && c->sub != c->all) nccl().CommDestroy(c->sub);
-        if (c->all) nccl().CommDestroy(c->all);
-    }
-    delete c;
+    delete h->comm;
     h->comm = nullptr;
 }
 
@@ -706,42 +679,29 @@ int bflk_power_map_batch_sharded_wait(bflk_handle *h) {
 int bflk_group_create(const bflk_config *cfg, const int32_t *device_ids, int32_t n_devices, int32_t dir_groups, bflk_group **out) {
     if (!cfg || !device_ids || n_devices < 1 || !out) return BFLK_ERR_INVALID;
     *out = nullptr;
-    bflk_group *g = new bflk_group();
+    std::unique_ptr<bflk_group> g(new bflk_group());
     for (int i = 0; i < n_devices; i++) {
         bflk_config c = *cfg;
         c.device = device_ids[i];
         bflk_handle *h = nullptr;
         int rc = bflk_create(&c, &h);
-        if (rc) {
-            for (bflk_handle *p : g->hs) bflk_destroy(p);
-            delete g;
-            return rc;
-        }
+        if (rc) return rc;
         g->hs.push_back(h);
     }
     if (n_devices > 1) {
-        if (!nccl().ok()) {
-            for (bflk_handle *p : g->hs) bflk_destroy(p);
-            delete g;
-            return BFLK_ERR_STATE;
-        }
+        if (!nccl().ok()) return BFLK_ERR_STATE;
         nccl_uid id;
         std::vector<int> ranks(n_devices);
         for (int i = 0; i < n_devices; i++) ranks[i] = i;
         int rc = nccl().GetUniqueId(&id) == 0 ? init_comms(g->hs, ranks, id, n_devices, dir_groups) : BFLK_ERR_CUDA;
-        if (rc) {
-            for (bflk_handle *p : g->hs) bflk_destroy(p);
-            delete g;
-            return rc;
-        }
+        if (rc) return rc;
     }
-    *out = g;
+    *out = g.release();
     return BFLK_OK;
 }
 
 int bflk_group_destroy(bflk_group *g) {
     if (!g) return BFLK_ERR_INVALID;
-    for (bflk_handle *h : g->hs) bflk_destroy(h);
     delete g;
     return BFLK_OK;
 }
