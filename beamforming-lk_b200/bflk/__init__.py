@@ -33,6 +33,8 @@ SYMBOLS = [
     "bflk_power_map_batch_dev", "bflk_power_map_batch_dev_submit", "bflk_power_map_batch_dev_join", "bflk_set_kernel", "bflk_set_channel_split", "bflk_launch_shape", "bflk_get_kernel", "bflk_launch_count", "bflk_enable_timing",
     "bflk_kernel_time_ms", "bflk_fp32_peak_tflops", "bflk_set_window", "bflk_set_window_dev", "bflk_miso", "bflk_miso_dev", "bflk_monopulse", "bflk_set_fir",
     "bflk_pin_host", "bflk_unpin_host", "bflk_heatmap", "bflk_resize_u8", "bflk_targets", "bflk_calibrate", "bflk_ingest_i32",
+    "bflk_stream_open", "bflk_stream_close", "bflk_stream_push", "bflk_stream_push_i32", "bflk_stream_power_maps",
+    "bflk_stream_discard", "bflk_stream_status", "bflk_stream_window",
     "bflk_comm_unique_id", "bflk_comm_init_rank", "bflk_comm_info", "bflk_shard_plan",
     "bflk_power_map_batch_sharded_dev", "bflk_power_map_batch_sharded_dev_submit", "bflk_power_map_batch_sharded_dev_join", "bflk_power_map_batch_sharded", "bflk_power_map_batch_sharded_submit", "bflk_power_map_batch_sharded_wait",
     "bflk_group_create", "bflk_group_destroy", "bflk_group_size", "bflk_group_handle", "bflk_group_last_error",
@@ -123,6 +125,14 @@ def load_library():
     L.bflk_targets.argtypes = [vp, vp, i32, f32, vp, C.POINTER(i32)]
     L.bflk_calibrate.argtypes = [vp, vp, i32, f32, vp, vp, C.POINTER(i32), C.POINTER(f32), C.POINTER(f32)]
     L.bflk_ingest_i32.argtypes = [vp, vp, i32, i32, vp]
+    L.bflk_stream_open.argtypes = [vp, i32]
+    L.bflk_stream_close.argtypes = [vp]
+    L.bflk_stream_push.argtypes = [vp, vp, i32]
+    L.bflk_stream_push_i32.argtypes = [vp, vp, i32]
+    L.bflk_stream_power_maps.argtypes = [vp, i32, vp, C.POINTER(i64), C.POINTER(i32)]
+    L.bflk_stream_discard.argtypes = [vp, i32]
+    L.bflk_stream_status.argtypes = [vp, C.POINTER(i64), C.POINTER(i64), C.POINTER(i32), C.POINTER(i64)]
+    L.bflk_stream_window.argtypes = [vp, i64]
     L.bflk_comm_unique_id.argtypes = [vp]
     L.bflk_comm_init_rank.argtypes = [vp, vp, i32, i32, i32]
     L.bflk_comm_info.argtypes = [vp, C.POINTER(i32), C.POINTER(i32), C.POINTER(i32), C.POINTER(i32), C.POINTER(i64)]
@@ -466,6 +476,47 @@ class Beamformer:
         self._check(self._L.bflk_monopulse(self._h, _ptr(theta), _ptr(phi), P, C.c_double(spread), C.c_double(theta_limit),
                                            C.c_double(reference), _ptr(window) if window is not None else None, _ptr(nth), _ptr(nph), _ptr(q), _ptr(grad), _ptr(err)))
         return theta, nth, nph, q, grad, err
+
+    # -- streaming session (bflk.h: bflk_stream_*) ----------------------------------------------------------------
+    def stream_open(self, max_frames):
+        """(Re)start a session at sample 0 with device history for max_frames ready frames."""
+        self._check(self._L.bflk_stream_open(self._h, max_frames))
+
+    def stream_close(self):
+        self._check(self._L.bflk_stream_close(self._h))
+
+    def stream_push(self, samples):
+        """samples [C][n] float32, the next n samples of every channel."""
+        samples = _np(samples, np.float32)
+        assert samples.ndim == 2 and samples.shape[0] == self.n_channels, samples.shape
+        self._check(self._L.bflk_stream_push(self._h, _ptr(samples), samples.shape[1]))
+
+    def stream_push_i32(self, rows):
+        """rows [n][C] int32 wire samples, one row per time sample."""
+        rows = _np(rows, np.int32)
+        assert rows.ndim == 2 and rows.shape[1] == self.n_channels, rows.shape
+        self._check(self._L.bflk_stream_push_i32(self._h, _ptr(rows), rows.shape[0]))
+
+    def stream_power_maps(self, max_frames=1):
+        """Maps the oldest ready frames (at most max_frames) in one call: (first_frame, power [n][count]), n may be 0."""
+        out = np.zeros((max_frames, self.n_directions()[2]), np.float32)
+        first, n = C.c_int64(), C.c_int32()
+        self._check(self._L.bflk_stream_power_maps(self._h, max_frames, _ptr(out), C.byref(first), C.byref(n)))
+        return first.value, out[:n.value].copy()
+
+    def stream_discard(self, keep=0):
+        """Skip every ready frame but the newest `keep`."""
+        self._check(self._L.bflk_stream_discard(self._h, keep))
+
+    def stream_status(self):
+        """(samples pushed per channel, next frame to map, frames ready, frames skipped)."""
+        a, b, c, d = C.c_int64(), C.c_int64(), C.c_int32(), C.c_int64()
+        self._check(self._L.bflk_stream_status(self._h, C.byref(a), C.byref(b), C.byref(c), C.byref(d)))
+        return a.value, b.value, c.value, d.value
+
+    def stream_window(self, frame):
+        """Session frame `frame` becomes the resident window of miso() / monopulse() with window=None."""
+        self._check(self._L.bflk_stream_window(self._h, frame))
 
     # -- neighbours ---------------------------------------------------------------------------------------------
     def heatmap(self, power):

@@ -7,6 +7,7 @@
 #include <algorithm>
 #include <cstdint>
 #include <cstdio>
+#include <memory>
 #include <string>
 #include <vector>
 
@@ -166,6 +167,24 @@ class Event {   // move-only
     cudaEvent_t e_ = nullptr;
 };
 
+// Streaming session (bflk_stream_*): the last `cap` samples of every channel on the device, in a mirrored ring (the twin of
+// the reference's double-mapped Streams, src/fpga/streams.hpp:152-182).  Sample t is stored at columns t % cap and
+// t % cap + cap of its channel's row of 2 * cap floats, so any window of at most cap samples is contiguous: it starts at
+// column start % cap, rows 2 * cap apart.  Nothing is ever moved, and cap is a multiple of N, so frame starts keep the
+// alignment of the ring.  Created by bflk_stream_open with its buffers and events; bflk_stream_close deletes it.
+struct Session {
+    DevBuf<float> ring;          // [C][2 * cap]
+    DevBuf<float> stage;         // one push: [C][n] float or [n][C] int32 (cap * C elements)
+    Event copied;                // the push's upload has read the caller's buffer
+    Event written;               // the push's samples are in the ring
+    int64_t cap = 0;
+    int64_t tail = 0;            // samples a frame needs beyond its own N, as the ring was sized for (frame_tail_samples)
+    int64_t pushed = 0;          // samples per channel since bflk_stream_open
+    int64_t next_frame = 0;      // oldest frame not yet mapped, discarded or skipped
+    int64_t skipped = 0;         // frames passed over: overwritten before they were mapped, or discarded
+    int64_t window_frame = -1;   // the frame that is the handle's resident window (bflk_stream_window), -1: none
+};
+
 }  // namespace bflk
 
 struct bflk_comm;   // multi.cu: NCCL communicator state of a handle that is one rank of a multi-GPU job
@@ -224,7 +243,9 @@ struct bflk_handle {
     int32_t fir_phases = 0, fir_taps = 0;
 
     // window kept on the device across calls (bflk_set_window): MISO / monopulse iterations on one frame do not re-upload it
-    const float *resident_window = nullptr;   // d_resident.p, or a caller-owned device pointer (bflk_set_window_dev)
+    const float *resident_window = nullptr;   // d_resident.p, a caller-owned device pointer (bflk_set_window_dev) or a session frame
+    int64_t resident_stride = 0;              // its row stride: window_len, or 2 * cap of the session's ring
+    std::unique_ptr<bflk::Session> session;   // bflk_stream_open .. bflk_stream_close
     bflk::DevBuf<int32_t> d_wire;
     bflk::DevBuf<uint8_t> d_bytes;            // heat-map / resize / peak-candidate scratch
     // bflk_power_map_batch_submit / _wait: two batches in flight, each with its own device buffers
@@ -427,6 +448,9 @@ cudaError_t launch_das_bcast(const BcastArgs &a, cudaStream_t st, int *launches,
 cudaError_t launch_heatmap(const float *d_power, int n, uint8_t *d_heat, int32_t *d_argmax, float *d_max, cudaStream_t st);
 cudaError_t launch_channel_power(const float *d_signals, int n_ch, int W, float *d_power, cudaStream_t st);
 cudaError_t launch_ingest(const int32_t *d_frames, int n, int n_sensors, float *d_exposure, cudaStream_t st);
+// samples t0 .. t0 + n of every channel into a Session's ring: d_block [C][n] float, or d_wire [n][C] int32 when it is set
+cudaError_t launch_history_push(const float *d_block, const int32_t *d_wire, int n, int C, int64_t t0, int cap, float *d_ring,
+                                cudaStream_t st);
 cudaError_t launch_ffma2_peak(float *d_out, int n_blocks, int iters, cudaStream_t st);
 cudaError_t launch_resize_u8(const uint8_t *d_src, int ih, int iw, uint8_t *d_dst, int oh, int ow, const int32_t *d_tab, cudaStream_t st);
 cudaError_t launch_map_targets(const float *d_power, int rows, int cols, int max_targets, float min_rel, uint8_t *d_cand,

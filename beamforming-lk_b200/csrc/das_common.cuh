@@ -1,5 +1,5 @@
 // das_common.cuh -- PTX helpers shared by the delay-and-sum kernels: packed FP32 (FFMA2 / FADD2),
-// mbarrier and TMA bulk-copy wrappers for sm_100a.
+// mbarrier and TMA bulk-copy wrappers for sm_100a; the wire-format un-flip and scale of the ingest kernels.
 #pragma once
 #include <cuda/std/cstdint>
 
@@ -60,6 +60,15 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void *src, uint32_t
                  : "memory");
 }
 
+
+// Wire format (one int32 row per time sample, src/fpga/receiver.h:24-30): the row column that holds a sensor -- every
+// second group of 8 is mirrored (daisy-chained arrays, pipeline.cpp:273-287) -- and the sample as a float (/ 2^23, exact
+// for 24-bit samples).  Every kernel that reads wire rows goes through these two, so they all hold the same floats.
+__device__ __forceinline__ int wire_column(int sensor) {
+    const int grp = sensor >> 3;
+    return (grp & 1) ? sensor : 8 * (1 + grp) - 1 - (sensor & 7);
+}
+__device__ __forceinline__ float wire_to_float(int32_t v) { return __fdiv_rn((float)v, 8388608.0f); }
 
 // output block q of a frame: first sample s_q = min(254 q, N - 256); it owns the high-pass outputs
 // MA_i for i in [254 q + 1, min(254 q + 254, N - 2)]  (N = 256: one block, i in [1, 254], mimo.cpp:132)

@@ -29,6 +29,8 @@
  *   bflk_targets                    Worker::tracking / getTargets (src/dsp/worker.h:32-61,136-142) for the MIMO map
  *   bflk_calibrate                  AWProcessingUnit::calibrate mask (aw_processing_unit.cpp:126-200)
  *   bflk_ingest_i32, bflk_power_map_i32   Pipeline::receive_exposure conversion (src/fpga/pipeline.cpp:260-297)
+ *   bflk_stream_*                   Streams (src/fpga/streams.hpp:152-182) + the worker loop (src/dsp/worker.h:212-224),
+ *                                   kept on the device: push samples as they arrive, map every frame
  *   bflk_comm_*, bflk_shard_plan, bflk_power_map_batch_sharded*, bflk_group_*   (no reference counterpart: the reference
  *                                   is single-threaded per worker, src/dsp/worker.h:90; AWProcessingUnit::start,
  *                                   src/aw_processing_unit/aw_processing_unit.cpp:67-95, is where a group is created)
@@ -174,6 +176,42 @@ int bflk_enable_timing(bflk_handle *h, int32_t on);
  * denominator reported next to the nominal FP32 roofline. */
 int bflk_fp32_peak_tflops(bflk_handle *h, float *tflops);
 int bflk_kernel_time_ms(bflk_handle *h, float *das_ms, int32_t *das_launches, float *pack_ms, int32_t *pack_launches);
+
+/* ---- streaming session: samples in as they arrive, a power map for every frame ------------------------- */
+/* The session keeps the history of every channel on the device (a mirrored ring, the twin of the reference's double-mapped
+ * Streams, src/fpga/streams.hpp:152-182), so a live caller pushes only new samples and maps every frame -- where the
+ * reference's worker loop drops the frames that arrive while it computes (src/dsp/worker.h:212-224).
+ * Frame b is frame b of bflk_power_map_batch over everything pushed since bflk_stream_open: samples
+ * [b*N, b*N + H + N + 1), plus n_taps - 2 with bflk_set_fir.  It is READY once that many samples have been pushed.
+ *
+ * bflk_stream_open (re)starts a session at sample 0, frame 0 with room for max_frames ready frames.  The session keeps raw
+ * samples only: kernel, grid, mask, direction range and channel split are read by each maps call.  A bflk_set_fir that
+ * lengthens a frame beyond what open sized the history for makes the maps calls fail with BFLK_ERR_STATE until the next
+ * open.  bflk_stream_close (or bflk_destroy) frees the session.
+ *
+ * A push of n samples per channel (1 <= n <= the ring's capacity) returns once the caller's buffer may be reused; the
+ * wire form needs n_channels % 8 == 0.  A push never blocks on or fails for a slow consumer: it overwrites the oldest
+ * sample, and every frame whose first sample is gone is SKIPPED (next_frame moves past it, skipped counts it).
+ *
+ * bflk_stream_power_maps maps the oldest min(max_frames, ready) frames in ONE call -- a backlog as one batch, a single frame
+ * in the latency shape -- into power_out[n][count] for the current direction range, reports the first frame and n, and
+ * consumes them.  Nothing ready: *n_frames = 0, BFLK_OK, and nothing else changes.  Synchronous on the handle's stream;
+ * after a call that returned one frame, bflk_targets / bflk_heatmap with a NULL map use it (as after bflk_power_map).
+ * bflk_stream_discard skips every ready frame but the newest `keep`.  bflk_stream_status: samples pushed per channel, the
+ * next frame a maps call returns, frames ready, frames skipped so far.
+ *
+ * bflk_stream_window makes a pushed frame still held by the ring the resident window: bflk_miso, bflk_miso_dev and
+ * bflk_monopulse with window == NULL then read it in place.  It is forgotten when the ring overwrites the frame, on close
+ * and on a new open (MISO with NULL then fails with BFLK_ERR_INVALID).  A frame that is no longer held or not fully pushed:
+ * BFLK_ERR_STATE.  Any session call without an open session: BFLK_ERR_STATE. */
+int bflk_stream_open(bflk_handle *h, int32_t max_frames);
+int bflk_stream_close(bflk_handle *h);
+int bflk_stream_push(bflk_handle *h, const float *samples, int32_t n);      /* [C][n], channel-major */
+int bflk_stream_push_i32(bflk_handle *h, const int32_t *rows, int32_t n);   /* [n][C], wire order */
+int bflk_stream_power_maps(bflk_handle *h, int32_t max_frames, float *power_out, int64_t *first_frame, int32_t *n_frames);
+int bflk_stream_discard(bflk_handle *h, int32_t keep);
+int bflk_stream_status(const bflk_handle *h, int64_t *pushed, int64_t *next_frame, int32_t *ready, int64_t *skipped);
+int bflk_stream_window(bflk_handle *h, int64_t frame);
 
 /* ---- multi-GPU: the grid (x the frames of a batch) sharded across the GPUs of one box ---------------- */
 /* Every direction's power is independent (src/dsp/mimo.cpp:121-151), so G ranks are arranged as G_d direction groups x
