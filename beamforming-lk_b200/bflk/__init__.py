@@ -399,6 +399,11 @@ class Beamformer:
         self._check(self._L.bflk_power_map_batch_i32(self._h, _ptr(frames), frames.shape[0], n_frames, _ptr(out)))
         return out
 
+    def power_map_batch_i32_dev(self, frames_dev_ptr, n_samples, n_frames, power_dev_ptr, cuda_stream=0):
+        """Device wire rows [T][C] int32 (e.g. a torch tensor's data_ptr()) -> power [B][count] on the device, asynchronous."""
+        self._check(self._L.bflk_power_map_batch_i32_dev(self._h, C.c_void_p(frames_dev_ptr), n_samples, n_frames,
+                                                         C.c_void_p(power_dev_ptr), C.c_void_p(cuda_stream)))
+
     def power_map_batch(self, stream, n_frames):
         """stream [C][T] float32 (host), frame b at sample b*N -> power [B][count]."""
         stream = _np(stream, np.float32)

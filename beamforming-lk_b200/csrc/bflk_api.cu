@@ -731,7 +731,7 @@ int bflk::power_map_dev(bflk_handle *h, const float *stream_dev, int64_t row_str
     if (wire && !tiled) {
         // the other kernels read channel-major float rows: convert the wire samples first (ingest_kernel), then carry on
         BFLK_CUDA(h, h->d_window.reserve((size_t)C * (n_samples + 1)));
-        BFLK_CUDA(h, launch_ingest(wire, (int)n_samples, C, h->d_window.p, st));
+        BFLK_CUDA(h, launch_ingest(wire, n_samples, C, h->d_window.p, st));
         h->launches++;
         stream_dev = h->d_window.p;
         row_stride = n_samples;

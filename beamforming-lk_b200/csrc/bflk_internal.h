@@ -447,7 +447,7 @@ cudaError_t launch_das_bcast(const BcastArgs &a, cudaStream_t st, int *launches,
 // ---- post.cu ----------------------------------------------------------------------------------------
 cudaError_t launch_heatmap(const float *d_power, int n, uint8_t *d_heat, int32_t *d_argmax, float *d_max, cudaStream_t st);
 cudaError_t launch_channel_power(const float *d_signals, int n_ch, int W, float *d_power, cudaStream_t st);
-cudaError_t launch_ingest(const int32_t *d_frames, int n, int n_sensors, float *d_exposure, cudaStream_t st);
+cudaError_t launch_ingest(const int32_t *d_frames, int64_t n, int n_sensors, float *d_exposure, cudaStream_t st);
 // samples t0 .. t0 + n of every channel into a Session's ring: d_block [C][n] float, or d_wire [n][C] int32 when it is set
 cudaError_t launch_history_push(const float *d_block, const int32_t *d_wire, int n, int C, int64_t t0, int cap, float *d_ring,
                                 cudaStream_t st);

@@ -202,13 +202,16 @@ __global__ void bcast_table_kernel(const int32_t *__restrict__ off, const float 
     }
 }
 
-__global__ void bcast_finalize_kernel(const float *__restrict__ partial, int nblk, int n_dir, float norm,
+// grid.y strides over the frames (it is limited to 65535)
+__global__ void bcast_finalize_kernel(const float *__restrict__ partial, int n_frames, int nblk, int n_dir, float norm,
                                       float *__restrict__ power) {
-    const int d = blockIdx.x * blockDim.x + threadIdx.x, b = blockIdx.y;
+    const int d = blockIdx.x * blockDim.x + threadIdx.x;
     if (d >= n_dir) return;
-    float p = 0.f;
-    for (int q = 0; q < nblk; q++) p += partial[((size_t)b * nblk + q) * n_dir + d];
-    power[(size_t)b * n_dir + d] = __fdiv_rn(p, norm);
+    for (int b = blockIdx.y; b < n_frames; b += gridDim.y) {
+        float p = 0.f;
+        for (int q = 0; q < nblk; q++) p += partial[((size_t)b * nblk + q) * n_dir + d];
+        power[(size_t)b * n_dir + d] = __fdiv_rn(p, norm);
+    }
 }
 
 }  // namespace
@@ -302,8 +305,8 @@ cudaError_t launch_das_bcast(const BcastArgs &a, cudaStream_t st, int *launches,
         *launches += 2;
     }
     if (nblk > 1) {
-        dim3 fg((a.n_dir + 255) / 256, a.n_frames);
-        bcast_finalize_kernel<<<fg, 256, 0, st>>>(a.partial, nblk, a.n_dir, a.norm, a.power);
+        dim3 fg((a.n_dir + 255) / 256, min(a.n_frames, 65535));
+        bcast_finalize_kernel<<<fg, 256, 0, st>>>(a.partial, a.n_frames, nblk, a.n_dir, a.norm, a.power);
         if ((e = cudaGetLastError()) != cudaSuccess) return e;
         *launches += 1;
     }

@@ -371,14 +371,17 @@ __global__ void __launch_bounds__(kWarps * 32, 1) das_tile_kernel(KernelArgs a) 
     }  // block pairs of this CTA
 }
 
-// frames longer than one block: power[b][d] = (sum_q partial[b*nblk + q][d]) / norm, blocks in order
+// frames longer than one block: power[b][d] = (sum_q partial[b*nblk + q][d]) / norm, blocks in order; grid.y strides over
+// the frames (it is limited to 65535)
 __global__ void finalize_kernel(const float *__restrict__ partial, int n_frames, int nblk, int n_dir, float norm,
                                 float *__restrict__ power) {
-    const int d = blockIdx.x * blockDim.x + threadIdx.x, b = blockIdx.y;
+    const int d = blockIdx.x * blockDim.x + threadIdx.x;
     if (d >= n_dir) return;
-    float p = 0.f;
-    for (int q = 0; q < nblk; q++) p += partial[((size_t)b * nblk + q) * n_dir + d];
-    power[(size_t)b * n_dir + d] = __fdiv_rn(p, norm);
+    for (int b = blockIdx.y; b < n_frames; b += gridDim.y) {
+        float p = 0.f;
+        for (int q = 0; q < nblk; q++) p += partial[((size_t)b * nblk + q) * n_dir + d];
+        power[(size_t)b * n_dir + d] = __fdiv_rn(p, norm);
+    }
 }
 
 // ---- host side ---------------------------------------------------------------------------------------------------
@@ -676,7 +679,7 @@ cudaError_t launch_das_tile(const TileArgs &a, int sm_count, cudaStream_t st, in
         *launches += 2;
     }
     if (nblk > 1) {
-        dim3 fg((a.n_dir + 255) / 256, a.n_frames);
+        dim3 fg((a.n_dir + 255) / 256, std::min(a.n_frames, 65535));
         finalize_kernel<<<fg, 256, 0, st>>>(a.partial, a.n_frames, nblk, a.n_dir, a.norm, a.power);
         cudaError_t e = cudaGetLastError();
         if (e != cudaSuccess) return e;

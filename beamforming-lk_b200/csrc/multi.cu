@@ -191,14 +191,16 @@ Plan make_plan(int D, int B, int n_ranks, int gd, int gf, int rank) {
 // gathered[G][frame_per][dir_per] (rank r = frame group r / gd, direction group r % gd) -> out[B][D]
 __global__ void assemble_kernel(const float *__restrict__ gathered, int B, int D, int gd, int frame_per, int dir_per,
                                 float *__restrict__ out) {
-    const int d = blockIdx.x * blockDim.x + threadIdx.x, b = blockIdx.y;
-    if (d >= D || b >= B) return;
+    const int d = blockIdx.x * blockDim.x + threadIdx.x;
+    if (d >= D) return;
     const int base = D / gd, extra = D % gd;
     int dg, dl;
     if (d < extra * (base + 1)) { dg = d / (base + 1); dl = d - dg * (base + 1); }
     else { dg = extra + (d - extra * (base + 1)) / base; dl = d - (dg * base + extra); }
-    const int fg = b / frame_per, bl = b - fg * frame_per;
-    out[(size_t)b * D + d] = gathered[((size_t)(fg * gd + dg) * frame_per + bl) * dir_per + dl];
+    for (int b = blockIdx.y; b < B; b += gridDim.y) {   // grid.y is limited to 65535
+        const int fg = b / frame_per, bl = b - fg * frame_per;
+        out[(size_t)b * D + d] = gathered[((size_t)(fg * gd + dg) * frame_per + bl) * dir_per + dl];
+    }
 }
 
 int apply_direction_range(bflk_handle *h, const Plan &p) {
@@ -266,7 +268,7 @@ int gather_and_assemble(const std::vector<bflk_handle *> &hs, const std::vector<
         if (!out_dev[i]) continue;
         BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
         const Plan &p = plans[i];
-        dim3 grid((h->n_dir + 255) / 256, B);
+        dim3 grid((h->n_dir + 255) / 256, std::min(B, 65535));
         assemble_kernel<<<grid, 256, 0, st[i]>>>(sets[i]->gather.p, B, h->n_dir, p.gd, p.frame_per, p.dir_per, out_dev[i]);
         BFLK_CUDA(h, cudaGetLastError());
         h->launches++;

@@ -75,25 +75,29 @@ cudaError_t launch_channel_power(const float *d_signals, int n_ch, int W, float 
 
 // ---- ingest -------------------------------------------------------------------------------------------
 // frames[n][n_sensors] (one UDP message per time sample, src/fpga/receiver.h:24-30) ->
-// exposure[n_sensors][n]: serpentine column un-flip + int32 / 2^23 (exact), 32x32 transpose tiles.
-__global__ void __launch_bounds__(256) ingest_kernel(const int32_t *__restrict__ frames, int n, int n_sensors,
+// exposure[n_sensors][n]: serpentine column un-flip + int32 / 2^23 (exact), 32x32 transpose tiles.  Sample tiles on grid.x
+// (grid.y is limited to 65535 tiles, 2 M samples), sensor tiles on grid.y.
+__global__ void __launch_bounds__(256) ingest_kernel(const int32_t *__restrict__ frames, int64_t n, int n_sensors,
                                                     float *__restrict__ exposure) {
     __shared__ float tile[32][33];
-    const int s0 = blockIdx.x * 32, i0 = blockIdx.y * 32;
+    const int64_t i0 = (int64_t)blockIdx.x * 32;
+    const int s0 = blockIdx.y * 32;
     const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
     for (int r = ty; r < 32; r += 8) {
-        int i = i0 + r, sensor = s0 + tx;
+        const int64_t i = i0 + r;
+        const int sensor = s0 + tx;
         if (i < n && sensor < n_sensors) tile[r][tx] = wire_to_float(frames[(size_t)i * n_sensors + wire_column(sensor)]);
     }
     __syncthreads();
     for (int r = ty; r < 32; r += 8) {
-        int sensor = s0 + r, i = i0 + tx;
+        const int64_t i = i0 + tx;
+        const int sensor = s0 + r;
         if (i < n && sensor < n_sensors) exposure[(size_t)sensor * n + i] = tile[tx][r];
     }
 }
 
-cudaError_t launch_ingest(const int32_t *d_frames, int n, int n_sensors, float *d_exposure, cudaStream_t st) {
-    dim3 grid((n_sensors + 31) / 32, (n + 31) / 32);
+cudaError_t launch_ingest(const int32_t *d_frames, int64_t n, int n_sensors, float *d_exposure, cudaStream_t st) {
+    dim3 grid((unsigned)((n + 31) / 32), (n_sensors + 31) / 32);
     ingest_kernel<<<grid, 256, 0, st>>>(d_frames, n, n_sensors, d_exposure);
     return cudaGetLastError();
 }

@@ -111,7 +111,8 @@ int bflk_steer_tables(bflk_handle *h, const double *theta, const double *phi, in
 int bflk_power_map(bflk_handle *h, const float *window, float *power_out);
 /* Batched: stream[C][T] channel-major continuous samples; frame b uses window stream[c][b*N .. b*N+W'),
  * i.e. consecutive frames advance by N samples like Streams::forward().  T >= (B-1)*N + H + N + 1.
- * power_out[B][count]. */
+ * power_out[B][count].  Every batch call takes any B >= 1: batches beyond the 65 535 blocks of a CUDA grid dimension
+ * run in slabs or grid-stride loops. */
 int bflk_power_map_batch(bflk_handle *h, const float *stream, int64_t n_samples, int32_t n_frames, float *power_out);
 /* Continuous operation: _submit returns as soon as the batch is enqueued (at most two batches in flight; a third submit
  * waits for the oldest), _wait blocks until the oldest batch in flight has delivered its maps into the power_out it was
@@ -126,7 +127,8 @@ int bflk_power_map_i32(bflk_handle *h, const int32_t *frames, float *power_out);
 /* A batch from the wire format: frames[T][C] int32 (T time samples, every sensor of the message in wire order), frame b
  * uses rows [b*N, b*N + H + N + 1).  One fused pass turns the wire samples into the kernel's staged layout (un-flip
  * folded into the column index, / 2^23, transpose, pair-interleave): no float copy of the stream exists, and the maps
- * are bit-identical to bflk_power_map_batch on the converted stream.  power_out[B][count]. */
+ * are bit-identical to bflk_power_map_batch on the converted stream.  power_out[B][count].  At most 2^31 - 1 rows per
+ * call (BFLK_ERR_INVALID beyond). */
 int bflk_power_map_batch_i32(bflk_handle *h, const int32_t *frames, int64_t n_samples, int32_t n_frames, float *power_out);
 int bflk_power_map_batch_i32_dev(bflk_handle *h, const int32_t *frames_dev, int64_t n_samples, int32_t n_frames,
                                  float *power_dev, void *cuda_stream);
@@ -145,7 +147,10 @@ int bflk_power_map_batch_dev_join(bflk_handle *h, void *cuda_stream);
 /* Selects the kernel: 0 = automatic, 1 = generic per-direction kernel, 2 = register-tiled kernel with the reference's
  * exact operation triple (delayed sums bit-identical to delay(), src/dsp/delay.cpp:16-26), 3 = lane-broadcast kernel,
  * 4 = register-tiled kernel in two-FMA form (f*s[i] + (1-f)*s[i+1]: as accurate as the reference against exact
- * arithmetic, power maps within the 1e-4 bar, ~13 % faster than 2).  Automatic = 4 when the grid tiles, else 3, else 1. */
+ * arithmetic, power maps within the 1e-4 bar, ~13 % faster than 2).  Automatic = 4 when the grid tiles, else 3, else 1.
+ * 2 and 4 need an even frame_len >= 256 and float rows of even length (the row stride: T of a batch, W of a single frame;
+ * wire rows have no such condition); 3 needs frame_len >= 256.  A call the chosen kernel cannot serve returns
+ * BFLK_ERR_STATE; the automatic choice falls back instead. */
 int bflk_set_kernel(bflk_handle *h, int32_t which);
 /* Latency option for calls too small to fill the GPU (a live worker's single frame, MIMOWorker::update once per 5.24 ms,
  * src/dsp/mimo.cpp:97-151): on != 0 lets the two-FMA form (kernel 0 / 4) split the CHANNELS of a frame across a thread-block
