@@ -285,7 +285,9 @@ class Beamformer:
                                                          C.c_void_p(power_ptr) if power_ptr else None))
 
     def kernel_info(self):
-        """(last kernel used: 1 generic / 2 tiled, tile span, window chunks of the tiled variant)."""
+        """(last kernel used: 1 generic / 2 tiled exact / 3 lane-broadcast / 4 tiled two-FMA / 0 none yet, largest offset
+        spread of a direction tile in the mode the grid tiles with (-1 before the tiles are built), window chunks of the
+        tiled variant (0 when the grid does not tile))."""
         a, b, c = C.c_int32(), C.c_int32(), C.c_int32()
         self._check(self._L.bflk_get_kernel(self._h, C.byref(a), C.byref(b), C.byref(c)))
         return a.value, b.value, c.value

@@ -81,7 +81,7 @@ struct Tuning {
 // Shape of the packed rows the tiled kernel stages (das_tile.cu).
 struct TileGeometry {
     int stage_off = 0;   // first packed sample, relative to a block's first output sample (even)
-    int nch = 0;         // 16-byte chunks per lane window the kernel variant loads (6, 8 or 10)
+    int nch = 0;         // 16-byte chunks per lane window the kernel variant loads (5 - 10; the exact form has no 9)
     int warps = 0;       // compute warps (= direction tiles) per CTA of the launch
     int tmpl_warps = 0;  // compiled variant (register budget / launch bound) the launch runs on; >= warps
     int fast = 0;        // 1: two-FMA form (TileEntryFast / TileEntryFastDual tables)
@@ -91,7 +91,7 @@ struct TileGeometry {
     int row_bytes = 0;   // bytes per packed row: the even-aligned copy followed by the copy shifted by one sample pair
     int stages = 0;      // stage buffers that fit shared memory (4 or 3; 0 = the variant does not fit at all)
     int pairs_per_cta = 0;  // 0 = automatic
-    int ksplit = 1;      // 2 / 4 / 8: a thread-block cluster of that size splits the channels of a block pair (small calls, two-FMA form)
+    int ksplit = 1;      // 2 / 4: a thread-block cluster of that size splits the channels of a block pair (small calls, two-FMA form)
 };
 
 // ---- lane-broadcast kernel (das_bcast.cu) -----------------------------------------------------------------

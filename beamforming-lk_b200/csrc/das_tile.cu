@@ -168,7 +168,7 @@ struct KernelArgs {
 // DUAL: two NCH-chunk windows per channel, one per direction pair (tile tables built with mode 1 / 2), NCH 6 or 7
 // FAST: two-FMA form acc += g s[i+1]; acc += f s[i] (TileEntryFast tables; power within 1e-4 of the reference instead of
 //       bit-identical delayed sums) -- 16 FFMA2 per (direction, channel) and no other FP instruction.
-// KSPLIT: the CTAs of a thread-block cluster (grid.z = cluster size 2 / 4 / 8) split the CHANNELS of a block pair between
+// KSPLIT: the CTAs of a thread-block cluster (grid.z = cluster size 2 or 4) split the CHANNELS of a block pair between
 //       them and add their partial delayed sums through distributed shared memory, in rank order, before the epilogue.
 //       For calls too small to fill the SMs (a live worker's single frame: cfg3 is 16 CTAs): the serial channel loop gets
 //       shorter by the cluster size.  The channel sum is re-associated (rank sums added at the end), so FAST only.

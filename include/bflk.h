@@ -154,7 +154,7 @@ int bflk_power_map_batch_dev_join(bflk_handle *h, void *cuda_stream);
 int bflk_set_kernel(bflk_handle *h, int32_t which);
 /* Latency option for calls too small to fill the GPU (a live worker's single frame, MIMOWorker::update once per 5.24 ms,
  * src/dsp/mimo.cpp:97-151): on != 0 lets the two-FMA form (kernel 0 / 4) split the CHANNELS of a frame across a thread-block
- * cluster of 2 / 4 / 8 CTAs, whose partial delayed sums are added through distributed shared memory in a fixed order before
+ * cluster of 2 or 4 CTAs, whose partial delayed sums are added through distributed shared memory in a fixed order before
  * the power epilogue (cfg3 single frame: 16 CTAs become 128).  The result is deterministic and within the same 1e-4 bar, but
  * the channel sum is associated differently than in a large batch, so "a batch gives the same bits as its frames one by
  * one" holds only with the option off (the default).  Kernel 2 never splits (its sums stay bit-identical to delay()). */
