@@ -383,12 +383,9 @@ int bflk_set_channel_split(bflk_handle *h, int32_t on) {
 int bflk_launch_shape(int32_t rows, int32_t cols, int32_t n_channels, int32_t frame_len, int32_t n_frames, int32_t n_sms,
                       int32_t channel_split, int32_t *warps, int32_t *split) {
     if (rows <= 0 || cols <= 0 || n_channels <= 0 || frame_len < 256 || n_frames <= 0 || n_sms <= 0 || !warps || !split) return BFLK_ERR_INVALID;
-    const int nblk = frame_len <= 256 ? 1 : (frame_len - 2 + 253) / 254;
-    const long long pairs = ((long long)n_frames * nblk + 1) / 2;
-    const int ppc = std::max(1, std::min(8, 512 / n_channels));
     int w = 0, sp = 1;
-    bflk::latency_shape((long long)((rows + 1) / 2) * ((cols + 1) / 2), (pairs + ppc - 1) / ppc, n_sms, (n_channels + kTileCC - 1) / kTileCC,
-                        channel_split != 0, &w, &sp);
+    bflk::latency_shape((long long)((rows + 1) / 2) * ((cols + 1) / 2), n_frames, frame_len, n_channels,
+                        block_pairs_per_cta(0, n_channels), n_sms, channel_split != 0, &w, &sp);
     *warps = w;
     *split = sp;
     return BFLK_OK;
@@ -473,6 +470,13 @@ int64_t min_stream_samples(const bflk_handle *h, int n_frames) {
     return (int64_t)(n_frames - 1) * h->cfg.frame_len + h->cfg.history + h->cfg.frame_len + 1;
 }
 
+// 2x2 direction tiles of the handle's direction range (whole rows of the grid; the first is even)
+static int tile_count(const bflk_handle *h) {
+    const int row0 = (h->dir_first / h->cols) & ~1;
+    const int row1 = (h->dir_first + h->dir_count - 1) / h->cols;  // inclusive
+    return ((row1 - row0) / 2 + 1) * ((h->cols + 1) / 2);
+}
+
 // Builds (once per grid / mask / range) the packed tables of the register-tiled kernel.  tiles_valid is set only after
 // the last step has succeeded, so a failed build is retried (and reported again) by the next call.
 int ensure_tiles(bflk_handle *h, int fast, int want_warps) {
@@ -487,10 +491,7 @@ int ensure_tiles(bflk_handle *h, int fast, int want_warps) {
         return BFLK_OK;
     }
     const int cols = h->cols;
-    const int row0 = (h->dir_first / cols) & ~1;
-    const int row1 = (h->dir_first + h->dir_count - 1) / cols;  // inclusive
-    const int tile_rows = (row1 - row0) / 2 + 1, tile_cols = (cols + 1) / 2;
-    const int n_tiles = tile_rows * tile_cols;
+    const int n_tiles = tile_count(h);
     const int usable = (int)h->index.size();
     BFLK_CUDA(h, h->d_tile_dirs.reserve((size_t)n_tiles * 4));
     BFLK_CUDA(h, h->d_misc.reserve(4));
@@ -614,9 +615,13 @@ static int ensure_bcast(bflk_handle *h) {
 // do not all fit at once next to 200 KB of shared memory per CTA).
 // Returns warps = 0 (throughput shape) for larger calls; otherwise the shape with the smallest estimate -- the larger CTA
 // (fewer copies of the rows staged) on ties, no split unless it wins by 10 %.
-void bflk::latency_shape(long long n_tiles, long long pair_ctas, int sms, int n_stage, bool may_split, int *warps, int *split) {
+void bflk::latency_shape(long long n_tiles, int n_frames, int frame_len, int usable, int pairs_per_cta, int sms, bool may_split,
+                         int *warps, int *split) {
     *warps = 0;
     *split = 1;
+    const long long pairs = ((long long)n_frames * blocks_per_frame(frame_len) + 1) / 2;
+    const long long pair_ctas = (pairs + pairs_per_cta - 1) / pairs_per_cta;
+    const int n_stage = (usable + kTileCC - 1) / kTileCC;
     if (((n_tiles + 15) / 16) * pair_ctas >= 2LL * sms) return;
     static const double step[6] = {0, 455, 538, 658, 880, 1100};
     const double fixed = 19650, exchange = 6000;
@@ -707,16 +712,9 @@ int bflk::power_map_dev(bflk_handle *h, const float *stream_dev, int64_t row_str
         // channels with four warps per scheduler): smaller CTAs trade per-SM efficiency for latency.  The shape is part of
         // the table layout, so a handle that alternates between single frames and large batches rebuilds its tables.
         int want_warps = 0, want_split = 1;
-        if (h->rows > 0 && h->cols > 0 && h->tuning.tile_warps == 0) {
-            const int nblk = N <= 256 ? 1 : (N - 2 + 253) / 254;
-            const long long pairs = ((long long)n_frames * nblk + 1) / 2;
-            const int ppc = h->tuning.tile_pairs > 0 ? h->tuning.tile_pairs : std::max(1, std::min(8, 512 / std::max(1, usable)));
-            const int row0 = (h->dir_first / h->cols) & ~1, row1 = (h->dir_first + h->dir_count - 1) / h->cols;
-            const long long n_tiles = (long long)((row1 - row0) / 2 + 1) * ((h->cols + 1) / 2);
-            latency_shape(n_tiles, (pairs + ppc - 1) / ppc, h->sm_count, (usable + kTileCC - 1) / kTileCC,
-                          h->kernel_choice != 2 && h->allow_ksplit && !h->tuning.no_ksplit,
-                          &want_warps, &want_split);
-        }
+        if (h->rows > 0 && h->cols > 0 && h->tuning.tile_warps == 0)
+            latency_shape(tile_count(h), n_frames, N, usable, block_pairs_per_cta(h->tuning.tile_pairs, usable), h->sm_count,
+                          h->kernel_choice != 2 && h->allow_ksplit && !h->tuning.no_ksplit, &want_warps, &want_split);
         if (want_warps > 0 && h->tuning.lat_warps >= 2 && h->tuning.lat_warps <= 16) want_warps = h->tuning.lat_warps;   // experiments
         if (want_warps > 0 && h->tuning.lat_split >= 1 && h->allow_ksplit) want_split = h->tuning.lat_split;
         if (launch.pipelined) { want_warps = 0; want_split = 1; }   // lanes_fork built the throughput-shape tables
@@ -740,69 +738,8 @@ int bflk::power_map_dev(bflk_handle *h, const float *stream_dev, int64_t row_str
     const bool bcast_ok = N >= 256 && das_bcast_fits(das_bcast_geometry(h->cfg.history, h->max_delay));
     if (h->kernel_choice == 3 && !bcast_ok)
         return h->fail(BFLK_ERR_STATE, "bflk_power_map: the lane-broadcast kernel needs frame_len >= 256 and a stage ring that fits shared memory");
-    if (!fir && !tiled && (h->kernel_choice == 0 || h->kernel_choice == 3) && bcast_ok) {
-        int rc = ensure_bcast(h);
-        if (rc) return rc;
-        BcastArgs a{};
-        a.stream = stream_dev;
-        a.row_stride = row_stride;
-        a.row_len = n_samples;
-        a.n_frames = n_frames;
-        a.frame_len = N;
-        a.frame_stride = N;
-        a.table = h->d_bcast_table.p;
-        a.tile_dirs = h->d_bcast_dirs.p;
-        a.n_tiles = h->bcast_tiles;
-        a.usable = usable;
-        a.n_dir = h->dir_count;
-        a.index = h->d_index.p;
-        a.geom = h->bcast_geom;
-        a.power = power_dev;
-        a.norm = norm;
-        BFLK_CUDA(h, d_packed.reserve(das_bcast_packed_bytes(a)));
-        a.packed = d_packed.p;
-        const int nblk = N <= 256 ? 1 : (N - 2 + 253) / 254;
-        if (nblk > 1) {
-            BFLK_CUDA(h, d_partial.reserve((size_t)n_frames * nblk * h->dir_count));
-            a.partial = d_partial.p;
-        }
-        int launches = 0;
-        BFLK_CUDA(h, launch_das_bcast(a, st, &launches, timing_hook, h));
-        h->launches += launches;
-        h->kernel_last = 3;
-        return BFLK_OK;
-    }
-    if (tiled) {
-        TileArgs a{};
-        a.wire = wire;
-        a.wire_cols = C;
-        a.stream = stream_dev;
-        a.row_stride = row_stride;
-        a.row_len = n_samples;
-        a.n_frames = n_frames;
-        a.frame_len = N;
-        a.frame_stride = N;
-        a.tiles = h->d_tiles.p;
-        a.tile_dirs = h->d_tile_dirs.p;
-        a.n_tiles = h->n_tiles;
-        a.usable = usable;
-        a.n_dir = h->dir_count;
-        a.index = h->d_index.p;
-        a.geom = h->tile_geom;
-        a.power = power_dev;
-        a.norm = norm;
-        BFLK_CUDA(h, d_packed.reserve(das_tile_packed_bytes(a)));
-        a.packed = d_packed.p;
-        const int blocks_per_frame = N <= 256 ? 1 : (N - 2 + 253) / 254;
-        if (blocks_per_frame > 1) {
-            BFLK_CUDA(h, d_partial.reserve((size_t)n_frames * blocks_per_frame * h->dir_count));
-            a.partial = d_partial.p;
-        }
-        int launches = 0;
-        BFLK_CUDA(h, launch_das_tile(a, h->sm_count, st, &launches, timing_hook, h));
-        h->launches += launches;
-        h->kernel_last = h->tile_geom.fast ? 4 : 2;
-    } else {
+    const bool bcast = !fir && !tiled && (h->kernel_choice == 0 || h->kernel_choice == 3) && bcast_ok;
+    if (!tiled && !bcast) {
         GenericArgs a{};
         a.stream = stream_dev;
         a.row_stride = row_stride;
@@ -824,7 +761,54 @@ int bflk::power_map_dev(bflk_handle *h, const float *stream_dev, int64_t row_str
         timing_hook(h, 0, false, st);
         h->launches++;
         h->kernel_last = 1;
+        return BFLK_OK;
     }
+    // the staged kernels: pack pre-pass, delay-and-sum, and for frames longer than one block finalize_kernel
+    if (bcast) {
+        int rc = ensure_bcast(h);
+        if (rc) return rc;
+    }
+    FrameArgs f;
+    f.stream = stream_dev;
+    f.row_stride = row_stride;
+    f.row_len = n_samples;
+    f.n_frames = n_frames;
+    f.frame_len = N;
+    f.frame_stride = N;
+    f.usable = usable;
+    f.n_dir = h->dir_count;
+    f.index = h->d_index.p;
+    f.power = power_dev;
+    f.norm = norm;
+    BFLK_CUDA(h, d_packed.reserve(packed_bytes(f, tiled ? h->tile_geom.row_bytes : h->bcast_geom.row_bytes)));
+    f.packed = d_packed.p;
+    if (blocks_per_frame(N) > 1) {
+        BFLK_CUDA(h, d_partial.reserve((size_t)n_frames * blocks_per_frame(N) * h->dir_count));
+        f.partial = d_partial.p;
+    }
+    int launches = 0;
+    if (tiled) {
+        TileArgs a;
+        a.f = f;
+        a.wire = wire;
+        a.wire_cols = C;
+        a.tiles = h->d_tiles.p;
+        a.tile_dirs = h->d_tile_dirs.p;
+        a.n_tiles = h->n_tiles;
+        a.geom = h->tile_geom;
+        BFLK_CUDA(h, launch_das_tile(a, h->sm_count, st, &launches, timing_hook, h));
+        h->kernel_last = h->tile_geom.fast ? 4 : 2;
+    } else {
+        BcastArgs a;
+        a.f = f;
+        a.table = h->d_bcast_table.p;
+        a.tile_dirs = h->d_bcast_dirs.p;
+        a.n_tiles = h->bcast_tiles;
+        a.geom = h->bcast_geom;
+        BFLK_CUDA(h, launch_das_bcast(a, st, &launches, timing_hook, h));
+        h->kernel_last = 3;
+    }
+    h->launches += launches;
     return BFLK_OK;
 }
 
@@ -897,9 +881,10 @@ int host_chunk_frames(bflk_handle *h, int n_frames, int *chunk_frames_out) {
     const int64_t frame_bytes = (int64_t)C * N * sizeof(float);
     int n_chunks = (int)std::max<int64_t>(1, ((int64_t)n_frames * frame_bytes + chunk_bytes / 2) / chunk_bytes);
     int chunk_frames = (n_frames + n_chunks - 1) / n_chunks;  // even split
-    if (n_chunks > 1 && N == 256 && h->kernel_choice != 1 && h->kernel_choice != 3 && h->sm_count > 0) {
+    const int form = tiled_form(h);
+    if (n_chunks > 1 && N == 256 && form >= 0 && h->sm_count > 0) {
         // the tiled kernel runs one CTA per (tile group, block pair): round the chunk to a whole number of CTA waves
-        int rc = ensure_tiles(h, h->kernel_choice != 2 ? 1 : 0);
+        int rc = ensure_tiles(h, form);
         if (rc) return rc;
         if (h->tiles_usable) {
             const int ctas_per_pair = (h->n_tiles + h->tile_geom.warps - 1) / h->tile_geom.warps;

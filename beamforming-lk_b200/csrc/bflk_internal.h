@@ -78,6 +78,15 @@ struct Tuning {
     int chunk_mib = 0;       // BFLK_CHUNK_MIB: host batches are uploaded in chunks of about this size
 };
 
+// Output blocks of a frame of frame_len samples: 256 samples each, 254 apart (das_common.cuh: the samples a block owns).
+__host__ __device__ inline int blocks_per_frame(int frame_len) { return frame_len <= 256 ? 1 : (frame_len - 2 + 253) / 254; }
+
+// Block pairs one CTA of the tiled kernel works on, one after the other: BFLK_TILE_PAIRS when set (tile_pairs > 0), else
+// enough to hide a CTA's ramp-up and epilogue behind short channel lists (a CTA lives ~0.6 us per channel).
+inline int block_pairs_per_cta(int tile_pairs, int usable) {
+    return tile_pairs > 0 ? tile_pairs : std::max(1, std::min(8, 512 / std::max(1, usable)));
+}
+
 // Shape of the packed rows the tiled kernel stages (das_tile.cu).
 struct TileGeometry {
     int stage_off = 0;   // first packed sample, relative to a block's first output sample (even)
@@ -384,30 +393,41 @@ struct MisoArgs {
 cudaError_t launch_das_miso(const MisoArgs &a, cudaStream_t st);
 int das_miso_slices(int frame_len);
 
-// ---- das_tile.cu ------------------------------------------------------------------------------------
-struct TileArgs {
-    const int32_t *wire = nullptr;   // when set: sample-major wire frames [row_len][wire_cols] instead of `stream` (pack_wire_kernel)
-    int wire_cols = 0;
-    const float *stream;
-    int64_t row_stride;
-    int64_t row_len;             // valid samples per row from `stream` (chunked host batches pass row_len < row_stride)
-    int n_frames;
-    int frame_len;
-    int frame_stride;
-    const void *tiles;           // tile_table_entries() entries (TileEntry, or TileEntryFast when geom.fast), grouped per (tile group, stage)
-    const int32_t *tile_dirs;    // [n_tiles][4]
-    int n_tiles;
-    int usable;
-    int n_dir;                   // directions in this handle's range (power row length)
-    const int32_t *index;        // [usable] channel mask (pack gathers rows in this order)
-    TileGeometry geom;
-    void *packed;                // das_tile_packed_bytes() of scratch
-    float *power;                // [B][n_dir]
-    float *partial;              // [B * blocks][n_dir] when frame_len > 256
-    float norm;
+// ---- staged kernels (das_tile.cu, das_bcast.cu): a pack pre-pass, the delay-and-sum kernel, finalize_kernel ------------
+// The frames of a call and where their maps go, as both staged kernels take them.
+struct FrameArgs {
+    const float *stream = nullptr;   // [C][row_stride] channel-major rows; frame b starts at column b * frame_stride
+    int64_t row_stride = 0;
+    int64_t row_len = 0;             // valid samples per row from `stream` (chunked host batches pass row_len < row_stride)
+    int n_frames = 0, frame_len = 0, frame_stride = 0;
+    int usable = 0;
+    int n_dir = 0;                   // directions in this handle's range (power row length)
+    const int32_t *index = nullptr;  // [usable] channel mask (pack gathers rows in this order)
+    void *packed = nullptr;          // packed_bytes() of scratch
+    float *power = nullptr;          // [B][n_dir]
+    float *partial = nullptr;        // [B * blocks_per_frame][n_dir] when frame_len > 256
+    float norm = 0.f;
 };
+// bytes of the packed rows of a call: one row of row_bytes per (block pair, usable channel)
+inline size_t packed_bytes(const FrameArgs &f, int row_bytes) {
+    const int n_items = f.n_frames * blocks_per_frame(f.frame_len);
+    return (size_t)((n_items + 1) / 2) * f.usable * row_bytes;
+}
+// frames longer than one block: power = the partial sums of each frame's blocks, added in block order, / norm (one launch)
+cudaError_t launch_finalize(const FrameArgs &f, cudaStream_t st);
 // hook(kind, begin): called right before (begin = true) and after each pack (kind 1) / main (kind 0) launch
 typedef void (*TileLaunchHook)(void *ctx, int kind, bool begin, cudaStream_t st);
+
+// ---- das_tile.cu ------------------------------------------------------------------------------------
+struct TileArgs {
+    FrameArgs f;
+    const int32_t *wire = nullptr;   // when set: sample-major wire frames [row_len][wire_cols] instead of f.stream (pack_wire_kernel)
+    int wire_cols = 0;
+    const void *tiles = nullptr;     // tile_table_entries() entries (TileEntry, or TileEntryFast when geom.fast), grouped per (tile group, stage)
+    const int32_t *tile_dirs = nullptr;   // [n_tiles][4]
+    int n_tiles = 0;
+    TileGeometry geom;
+};
 cudaError_t launch_das_tile(const TileArgs &a, int sm_count, cudaStream_t st, int *launches, TileLaunchHook hook = nullptr,
                             void *hook_ctx = nullptr);
 int das_tile_max_span();
@@ -415,29 +435,21 @@ TileGeometry das_tile_geometry(int history, int max_delay, int max_span, int n_t
                                const Tuning *tuning = nullptr, int want_warps = 0);
 // shared memory the variant needs with `stages` stage buffers
 size_t das_tile_smem_bytes(const TileGeometry &g, int stages);
-size_t das_tile_packed_bytes(const TileArgs &a);
-// can this geometry split the channels of a block pair across a cluster of `split` CTAs (two-FMA 16-warp variants only)?
+// can this geometry split the channels of a block pair across a cluster of `split` CTAs (compiled for some variants only)?
 bool das_tile_ksplit_ok(const TileGeometry &g, int split);
 size_t das_tile_entry_bytes(const TileGeometry &g);
 
 // ---- das_bcast.cu -----------------------------------------------------------------------------------
 struct BcastArgs {
-    const float *stream;
-    int64_t row_stride, row_len;
-    int n_frames, frame_len, frame_stride;
-    const BcastEntry *table;
-    const int32_t *tile_dirs;   // [n_tiles][32] local direction index or -1
-    int n_tiles, usable, n_dir;
-    const int32_t *index;
+    FrameArgs f;
+    const BcastEntry *table = nullptr;
+    const int32_t *tile_dirs = nullptr;   // [n_tiles][32] local direction index or -1
+    int n_tiles = 0;
     BcastGeometry geom;
-    void *packed;               // das_bcast_packed_bytes() of scratch
-    float *power, *partial;
-    float norm;
 };
 BcastGeometry das_bcast_geometry(int history, int max_delay);
 bool das_bcast_fits(const BcastGeometry &g);
 size_t das_bcast_table_entries(int n_tiles, int usable);
-size_t das_bcast_packed_bytes(const BcastArgs &a);
 cudaError_t launch_bcast_table(const int32_t *d_off, const float *d_frac, int C, const int32_t *d_index, int usable,
                                const int32_t *d_tile_globals, int n_tiles, const BcastGeometry &g, BcastEntry *d_table,
                                cudaStream_t st);
@@ -486,7 +498,9 @@ int lanes_join(bflk_handle *h, int only = -1);
 // -1 when the register-tiled kernels cannot serve a call (FIR, or kernel 1 / 3), else the `fast` flag for ensure_tiles
 int tiled_form(const bflk_handle *h);
 int ensure_tiles(bflk_handle *h, int fast, int want_warps = 0);
-void latency_shape(long long n_tiles, long long pair_ctas, int sms, int n_stage, bool may_split, int *warps, int *split);
+// CTA shape of a tiled call over n_tiles direction tiles and n_frames frames: warps = 0 (throughput shape) or 2..16
+void latency_shape(long long n_tiles, int n_frames, int frame_len, int usable, int pairs_per_cta, int sms, bool may_split,
+                   int *warps, int *split);
 int64_t min_stream_samples(const bflk_handle *h, int n_frames);
 // frames per chunk of a host batch of n_frames (whole CTA waves of the tiled kernel where it applies) and the samples a
 // frame needs beyond its own N

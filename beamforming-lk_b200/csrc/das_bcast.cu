@@ -202,18 +202,6 @@ __global__ void bcast_table_kernel(const int32_t *__restrict__ off, const float 
     }
 }
 
-// grid.y strides over the frames (it is limited to 65535)
-__global__ void bcast_finalize_kernel(const float *__restrict__ partial, int n_frames, int nblk, int n_dir, float norm,
-                                      float *__restrict__ power) {
-    const int d = blockIdx.x * blockDim.x + threadIdx.x;
-    if (d >= n_dir) return;
-    for (int b = blockIdx.y; b < n_frames; b += gridDim.y) {
-        float p = 0.f;
-        for (int q = 0; q < nblk; q++) p += partial[((size_t)b * nblk + q) * n_dir + d];
-        power[(size_t)b * n_dir + d] = __fdiv_rn(p, norm);
-    }
-}
-
 }  // namespace
 
 BcastGeometry das_bcast_geometry(int history, int max_delay) {
@@ -227,11 +215,6 @@ BcastGeometry das_bcast_geometry(int history, int max_delay) {
 
 size_t das_bcast_table_entries(int n_tiles, int usable) {
     return (size_t)n_tiles * ((usable + kCC - 1) / kCC) * kCC * 32;
-}
-
-size_t das_bcast_packed_bytes(const BcastArgs &a) {
-    const int n_items = a.n_frames * blocks_per_frame(a.frame_len);
-    return (size_t)((n_items + 1) / 2) * a.usable * a.geom.row_bytes;
 }
 
 cudaError_t launch_bcast_table(const int32_t *d_off, const float *d_frac, int C, const int32_t *d_index, int usable,
@@ -252,47 +235,48 @@ bool das_bcast_fits(const BcastGeometry &g) {
 }
 
 cudaError_t launch_das_bcast(const BcastArgs &a, cudaStream_t st, int *launches, TileLaunchHook hook, void *hook_ctx) {
-    const int nblk = blocks_per_frame(a.frame_len);
-    const int n_items = a.n_frames * nblk;
+    const FrameArgs &f = a.f;
+    const int nblk = blocks_per_frame(f.frame_len);
+    const int n_items = f.n_frames * nblk;
     const int n_pairs = (n_items + 1) / 2;
-    if (a.frame_len < kBlock) return cudaErrorInvalidValue;
+    if (f.frame_len < kBlock) return cudaErrorInvalidValue;
     const size_t smem = bcast_smem_bytes(a.geom);
     if (!das_bcast_fits(a.geom)) return cudaErrorInvalidConfiguration;
     cudaError_t e = cudaFuncSetAttribute(bcast_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
 
     PackArgs p{};
-    p.stream = a.stream;
-    p.row_stride = a.row_stride;
-    p.row_len = a.row_len;
-    p.frame_len = a.frame_len;
-    p.frame_stride = a.frame_stride;
+    p.stream = f.stream;
+    p.row_stride = f.row_stride;
+    p.row_len = f.row_len;
+    p.frame_len = f.frame_len;
+    p.frame_stride = f.frame_stride;
     p.nblk = nblk;
     p.n_items = n_items;
-    p.index = a.index;
-    p.usable = a.usable;
+    p.index = f.index;
+    p.usable = f.usable;
     p.first_sample = a.geom.first_sample;
     p.row_elems = a.geom.row_elems;
-    p.packed = reinterpret_cast<float4 *>(a.packed);
+    p.packed = reinterpret_cast<float4 *>(f.packed);
 
     KernelArgs k{};
     k.packed = p.packed;
     k.table = a.table;
     k.tile_dirs = a.tile_dirs;
-    k.usable = a.usable;
-    k.n_dir = a.n_dir;
+    k.usable = f.usable;
+    k.n_dir = f.n_dir;
     k.row_bytes = a.geom.row_bytes;
     k.n_items = n_items;
     k.nblk = nblk;
-    k.frame_len = a.frame_len;
-    k.out = nblk == 1 ? a.power : a.partial;
-    k.norm = a.norm;
+    k.frame_len = f.frame_len;
+    k.out = nblk == 1 ? f.power : f.partial;
+    k.norm = f.norm;
 
     const int max_slab = 32768;  // grid.y / grid.z limits
     for (int p0 = 0; p0 < n_pairs; p0 += max_slab) {
         const int np = min(max_slab, n_pairs - p0);
         p.pair0 = k.pair0 = p0;
-        dim3 pg((a.geom.row_elems + 255) / 256, a.usable, np);
+        dim3 pg((a.geom.row_elems + 255) / 256, f.usable, np);
         if (hook) hook(hook_ctx, 1, true, st);
         bcast_pack_kernel<<<pg, 256, 0, st>>>(p);
         if (hook) hook(hook_ctx, 1, false, st);
@@ -305,9 +289,7 @@ cudaError_t launch_das_bcast(const BcastArgs &a, cudaStream_t st, int *launches,
         *launches += 2;
     }
     if (nblk > 1) {
-        dim3 fg((a.n_dir + 255) / 256, min(a.n_frames, 65535));
-        bcast_finalize_kernel<<<fg, 256, 0, st>>>(a.partial, a.n_frames, nblk, a.n_dir, a.norm, a.power);
-        if ((e = cudaGetLastError()) != cudaSuccess) return e;
+        if ((e = launch_finalize(f, st)) != cudaSuccess) return e;
         *launches += 1;
     }
     return cudaSuccess;

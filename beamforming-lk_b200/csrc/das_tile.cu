@@ -24,7 +24,9 @@
 //  * epilogue: 3-tap high-pass + squares (mimo.cpp:131-135) with neighbour samples from lane +-1,
 //    warp-shuffle reduction, one store per (block, direction).
 #include <algorithm>
+#include <array>
 #include <cstdlib>
+#include <utility>
 
 #include "bflk_internal.h"
 #include "das_common.cuh"
@@ -37,7 +39,6 @@ constexpr int kCC = kTileCC;         // channels per pipeline stage
 constexpr int kMaxStages = 4;        // stage buffers (KernelArgs::stages: 4 when shared memory allows, else 3)
 constexpr int kBlock = 256;          // output samples per block
 constexpr int kK = 8;                // sample pairs per lane
-constexpr int kFastMaxNch16 = 10;    // largest window of the two-FMA variant that still runs 16 warps per CTA
 
 // chunk (16 B = 2 sample pairs) c of a row lives at padded chunk c + (c >> 2)
 __host__ __device__ __forceinline__ int padded_chunk(int c) { return c + (c >> 2); }
@@ -69,19 +70,13 @@ struct PackArgs {
     float4 *packed;
 };
 
-__device__ __forceinline__ int64_t item_start(int item, int blocks_per_frame, int frame_len, int frame_stride) {
-    const int b = item / blocks_per_frame, q = item - b * blocks_per_frame;
-    const int s = min(254 * q, frame_len - kBlock);
-    return (int64_t)b * frame_stride + s;
-}
-
 __global__ void __launch_bounds__(256) pack_kernel(PackArgs a) {
     const int pair = a.pair0 + blockIdx.z, s = blockIdx.y;
     const int ch = blockIdx.x * blockDim.x + threadIdx.x;
     if (ch >= a.row_chunks) return;
     const int itemA = 2 * pair, itemB = min(2 * pair + 1, a.n_items - 1);
-    const int64_t tA = item_start(itemA, a.blocks_per_frame, a.frame_len, a.frame_stride) + a.stage_off + 2 * ch;
-    const int64_t tB = item_start(itemB, a.blocks_per_frame, a.frame_len, a.frame_stride) + a.stage_off + 2 * ch;
+    const int64_t tA = item_first_sample(itemA, a.blocks_per_frame, a.frame_len, a.frame_stride) + a.stage_off + 2 * ch;
+    const int64_t tB = item_first_sample(itemB, a.blocks_per_frame, a.frame_len, a.frame_stride) + a.stage_off + 2 * ch;
     const float *row = a.stream + (size_t)a.index[s] * a.row_stride;
     // samples 2ch, 2ch+1, 2ch+2 of both blocks (8-byte loads, zero beyond the end of the stream)
     auto load2 = [&](int64_t t) {
@@ -117,8 +112,8 @@ __global__ void __launch_bounds__(256) pack_wire_kernel(PackArgs a) {
     __shared__ float sm[2][kWireCh][kWirePitch];
     const int pair = a.pair0 + blockIdx.z, s0 = blockIdx.y * kWireCh, ch0 = blockIdx.x * kWireChunks;
     const int itemA = 2 * pair, itemB = min(2 * pair + 1, a.n_items - 1);
-    const int64_t t0[2] = {item_start(itemA, a.blocks_per_frame, a.frame_len, a.frame_stride) + a.stage_off + 2 * ch0,
-                           item_start(itemB, a.blocks_per_frame, a.frame_len, a.frame_stride) + a.stage_off + 2 * ch0};
+    const int64_t t0[2] = {item_first_sample(itemA, a.blocks_per_frame, a.frame_len, a.frame_stride) + a.stage_off + 2 * ch0,
+                           item_first_sample(itemB, a.blocks_per_frame, a.frame_len, a.frame_stride) + a.stage_off + 2 * ch0};
     const int cl = threadIdx.x & 31, r = threadIdx.x >> 5;
     const int s = s0 + cl;
     int col = -1;
@@ -328,13 +323,7 @@ __global__ void __launch_bounds__(kWarps * 32, 1) das_tile_kernel(KernelArgs a) 
     const int itemA = 2 * pair, itemB = 2 * pair + 1;
     int jlo[2], jhi[2];
 #pragma unroll
-    for (int h = 0; h < 2; h++) {
-        const int item = min(h ? itemB : itemA, a.n_items - 1);
-        const int q = item % a.blocks_per_frame;
-        const int s = min(254 * q, a.frame_len - kBlock);
-        jlo[h] = 254 * q + 1 - s;
-        jhi[h] = min(254 * q + 254, a.frame_len - 2) - s;
-    }
+    for (int h = 0; h < 2; h++) item_ma_range(min(h ? itemB : itemA, a.n_items - 1), a.blocks_per_frame, a.frame_len, jlo[h], jhi[h]);
 #pragma unroll
     for (int r = 0; r < 4; r++) {
         u64 prev = __shfl_up_sync(0xffffffffu, acc[r][kK - 1], 1);
@@ -371,8 +360,8 @@ __global__ void __launch_bounds__(kWarps * 32, 1) das_tile_kernel(KernelArgs a) 
     }  // block pairs of this CTA
 }
 
-// frames longer than one block: power[b][d] = (sum_q partial[b*nblk + q][d]) / norm, blocks in order; grid.y strides over
-// the frames (it is limited to 65535)
+// frames longer than one block (this kernel and das_bcast's): power[b][d] = (sum_q partial[b*nblk + q][d]) / norm, blocks
+// in order; grid.y strides over the frames (it is limited to 65535)
 __global__ void finalize_kernel(const float *__restrict__ partial, int n_frames, int nblk, int n_dir, float norm,
                                 float *__restrict__ power) {
     const int d = blockIdx.x * blockDim.x + threadIdx.x;
@@ -384,8 +373,55 @@ __global__ void finalize_kernel(const float *__restrict__ partial, int n_frames,
     }
 }
 
+cudaError_t launch_finalize(const FrameArgs &f, cudaStream_t st) {
+    dim3 fg((f.n_dir + 255) / 256, std::min(f.n_frames, 65535));
+    finalize_kernel<<<fg, 256, 0, st>>>(f.partial, f.n_frames, blocks_per_frame(f.frame_len), f.n_dir, f.norm, f.power);
+    return cudaGetLastError();
+}
+
 // ---- host side ---------------------------------------------------------------------------------------------------
 int das_tile_max_span() { return 11; }
+
+// Every compiled instantiation das_tile_kernel<nch, warps, dual, fast, ksplit>: the kernel is instantiated from this list
+// (kTileLaunchers), and it alone answers which variants exist.  warps is the register budget (launch bound); a launch may
+// run fewer warps per CTA on it.  The exact form has no 9-chunk window, and the channel split is two-FMA and 16 warps only.
+struct TileVariant {
+    int nch, warps;
+    bool dual, fast, ksplit;
+};
+constexpr TileVariant kTileVariants[] = {
+    // two-FMA form, channels split across a cluster
+    {5, 16, false, true, true}, {6, 16, false, true, true}, {7, 16, false, true, true},
+    {8, 16, false, true, true}, {9, 16, false, true, true}, {10, 16, false, true, true},
+    {6, 16, true, true, true}, {7, 16, true, true, true},
+    // two-FMA form
+    {5, 10, false, true, false}, {5, 11, false, true, false}, {5, 12, false, true, false}, {5, 16, false, true, false},
+    {6, 10, false, true, false}, {6, 11, false, true, false}, {6, 12, false, true, false}, {6, 16, false, true, false},
+    {7, 10, false, true, false}, {7, 11, false, true, false}, {7, 12, false, true, false}, {7, 16, false, true, false},
+    {8, 10, false, true, false}, {8, 11, false, true, false}, {8, 12, false, true, false}, {8, 16, false, true, false},
+    {9, 10, false, true, false}, {9, 11, false, true, false}, {9, 12, false, true, false}, {9, 16, false, true, false},
+    {10, 10, false, true, false}, {10, 11, false, true, false}, {10, 12, false, true, false}, {10, 16, false, true, false},
+    {6, 10, true, true, false}, {6, 11, true, true, false}, {6, 12, true, true, false}, {6, 16, true, true, false},
+    {7, 10, true, true, false}, {7, 11, true, true, false}, {7, 12, true, true, false}, {7, 16, true, true, false},
+    // exact form
+    {5, 10, false, false, false}, {5, 11, false, false, false}, {5, 12, false, false, false}, {5, 16, false, false, false},
+    {6, 10, false, false, false}, {6, 11, false, false, false}, {6, 12, false, false, false}, {6, 16, false, false, false},
+    {7, 10, false, false, false}, {7, 11, false, false, false}, {7, 12, false, false, false}, {7, 16, false, false, false},
+    {8, 10, false, false, false}, {8, 11, false, false, false}, {8, 12, false, false, false}, {8, 16, false, false, false},
+    {10, 10, false, false, false}, {10, 11, false, false, false}, {10, 12, false, false, false}, {10, 16, false, false, false},
+    {6, 10, true, false, false}, {6, 11, true, false, false}, {6, 12, true, false, false}, {6, 16, true, false, false},
+    {7, 10, true, false, false}, {7, 11, true, false, false}, {7, 12, true, false, false},
+};
+constexpr int kNumTileVariants = (int)(sizeof(kTileVariants) / sizeof(kTileVariants[0]));
+
+// index of the variant in kTileVariants, -1 when it is not compiled
+static int tile_variant(int nch, int warps, bool dual, bool fast, bool ksplit) {
+    for (int i = 0; i < kNumTileVariants; i++) {
+        const TileVariant &v = kTileVariants[i];
+        if (v.nch == nch && v.warps == warps && v.dual == dual && v.fast == fast && v.ksplit == ksplit) return i;
+    }
+    return -1;
+}
 
 // experiment switch (read once): BFLK_NO_PACK_CARVEOUT=1 leaves the pack kernels' L1 / shared split to the driver
 static bool getenv_once_no_carveout() {
@@ -412,18 +448,17 @@ TileGeometry das_tile_geometry(int history, int max_delay, int max_span, int n_t
         g.nch = std::max(mode ? 6 : 5, (9 + max_span + 1) / 2);
         if (tuning && tuning->tile_nch > 0) g.nch = std::min(mode ? 7 : 10, std::max(g.nch, tuning->tile_nch));
     }
-    // Warps (= direction tiles) per CTA.  The kernel is issue-bound (an FFMA2 / FADD2 holds a scheduler's issue
-    // port for two cycles), so more resident warps help only while registers allow: the 6-chunk variant fits
-    // 128 registers (16 warps, +5 % over 12); the 8- and 10-chunk variants need ~150-165 (12 warps; 16 would
-    // spill).  Smaller CTAs only when a small direction shard (multi-GPU) would leave the last CTA mostly idle.
-    const bool can16 = g.nch <= 6 || (fast && g.nch <= kFastMaxNch16 && !(mode != 0 && g.nch > 7));
-    const bool exact_dual7 = !fast && mode != 0 && g.nch == 7;   // compiled for 10 - 12 warps only
+    // Warps (= direction tiles) per CTA, among the compiled variants of this window.  The kernel is issue-bound (an FFMA2 /
+    // FADD2 holds a scheduler's issue port for two cycles), so more resident warps help only while registers allow: the
+    // 6-chunk and the two-FMA variants fit 128 registers (16 warps, +5 % over 12); the exact 7- to 10-chunk variants need
+    // ~150-165 (12 warps; at 16 they spill, so only BFLK_TILE_WARPS=16 runs them).  Smaller CTAs only when a small direction
+    // shard (multi-GPU) would leave the last CTA mostly idle.
+    const bool dual = mode != 0;
+    const bool policy16 = fast || g.nch <= 6;
     const int n_cand = 4;
     const int cand[n_cand] = {16, 12, 11, 10};
-    const double tlp[n_cand] = {can16 && !exact_dual7 ? 1.05 : 0.0, 1.0, 0.95, 0.88};
-    int forced = 0;
-    if (tuning && ((tuning->tile_warps >= 10 && tuning->tile_warps <= 12) || (tuning->tile_warps == 16 && !exact_dual7)))
-        forced = tuning->tile_warps;
+    const double tlp[n_cand] = {policy16 ? 1.05 : 0.0, 1.0, 0.95, 0.88};
+    const int forced = tuning && tile_variant(g.nch, tuning->tile_warps, dual, fast, false) >= 0 ? tuning->tile_warps : 0;
     // the largest logical chunk a lane can touch: (H - stage_off)/2 + 4*31 + nch - 1
     g.row_chunks = (history - g.stage_off) / 2 + 4 * 31 + g.nch;
     g.copy_bytes = 16 * (padded_chunk(g.row_chunks - 1) + 1);
@@ -434,8 +469,8 @@ TileGeometry das_tile_geometry(int history, int max_delay, int max_span, int n_t
     g.warps = 0;
     g.stages = 0;
     for (int i = 0; i < n_cand; i++) {
-        if (forced && cand[i] != forced) continue;
-        if (tlp[i] <= 0.0 && !forced) continue;
+        if (forced ? cand[i] != forced : tlp[i] <= 0.0) continue;
+        if (tile_variant(g.nch, cand[i], dual, fast, false) < 0) continue;
         TileGeometry t = g;
         t.warps = cand[i];
         int stages = tuning && tuning->tile_stages == 3 ? 3 : kMaxStages;
@@ -449,8 +484,9 @@ TileGeometry das_tile_geometry(int history, int max_delay, int max_span, int n_t
     g.tmpl_warps = g.warps;
     if (want_warps > 0 && want_warps <= 16 && g.stages >= 3) {
         // latency shape (single-frame calls): fewer warps per CTA than the throughput shape, run on the largest compiled
-        // variant (its register budget is an upper bound); the stage ring of a smaller CTA always fits if the large one does
-        const int tmpl = can16 && !exact_dual7 ? 16 : 12;
+        // variant the policy allows (its register budget is an upper bound); the stage ring of a smaller CTA always fits if
+        // the large one does
+        const int tmpl = policy16 && tile_variant(g.nch, 16, dual, fast, false) >= 0 ? 16 : 12;
         TileGeometry t = g;
         t.warps = std::min(want_warps, tmpl);
         int stages = tuning && tuning->tile_stages == 3 ? 3 : kMaxStages;
@@ -468,7 +504,7 @@ TileGeometry das_tile_geometry(int history, int max_delay, int max_span, int n_t
 
 bool das_tile_ksplit_ok(const TileGeometry &g, int split) {
     // the exchange area (8 KB per (source rank, tile finished here)) reuses the stage buffers' rows
-    return (split == 2 || split == 4) && g.fast && g.tmpl_warps == 16 && g.stages >= 3 &&
+    return (split == 2 || split == 4) && tile_variant(g.nch, g.tmpl_warps, g.mode != 0, g.fast, true) >= 0 && g.stages >= 3 &&
            (size_t)split * ((g.warps + split - 1) / split) * 8192 <= (size_t)g.stages * kCC * g.row_bytes;
 }
 
@@ -508,56 +544,63 @@ static cudaError_t launch_main(const KernelArgs &k, dim3 grid, size_t smem, cuda
     return cudaGetLastError();
 }
 
-size_t das_tile_packed_bytes(const TileArgs &a) {
-    const int nblk = a.frame_len <= kBlock ? 1 : (a.frame_len - 2 + 253) / 254;
-    const int n_items = a.n_frames * nblk;
-    return (size_t)((n_items + 1) / 2) * a.usable * a.geom.row_bytes;
+using TileLauncher = cudaError_t (*)(const KernelArgs &, dim3, size_t, cudaStream_t);
+template <size_t... I>
+static constexpr std::array<TileLauncher, sizeof...(I)> tile_launchers(std::index_sequence<I...>) {
+    return {launch_main<kTileVariants[I].nch, kTileVariants[I].warps, kTileVariants[I].dual, kTileVariants[I].fast,
+                        kTileVariants[I].ksplit>...};
 }
+// kTileLaunchers[i] launches kTileVariants[i]
+static constexpr auto kTileLaunchers = tile_launchers(std::make_index_sequence<kNumTileVariants>());
 
 cudaError_t launch_das_tile(const TileArgs &a, int sm_count, cudaStream_t st, int *launches, TileLaunchHook hook, void *hook_ctx) {
     (void)sm_count;
-    const int nblk = a.frame_len <= kBlock ? 1 : (a.frame_len - 2 + 253) / 254;
-    const int n_items = a.n_frames * nblk;
+    const FrameArgs &f = a.f;
+    const int nblk = blocks_per_frame(f.frame_len);
+    const int n_items = f.n_frames * nblk;
     const int n_pairs = (n_items + 1) / 2;
-    if (a.frame_len < kBlock || (!a.wire && (a.row_stride & 1)) || (a.frame_stride & 1) || (a.frame_len & 1)) return cudaErrorInvalidValue;
+    if (f.frame_len < kBlock || (!a.wire && (f.row_stride & 1)) || (f.frame_stride & 1) || (f.frame_len & 1)) return cudaErrorInvalidValue;
+    // channel split across a cluster (latency shape of small calls): das_tile_ksplit_ok allows it where it is compiled
+    const int ksplit = std::max(1, a.geom.ksplit);
+    const int variant = tile_variant(a.geom.nch, a.geom.tmpl_warps, a.geom.mode != 0, a.geom.fast, ksplit > 1);
+    const int stages = a.geom.stages;
+    if (stages < 3 || variant < 0) return cudaErrorInvalidConfiguration;   // ensure_tiles never selects such a geometry
+    const size_t smem = das_tile_smem_bytes(a.geom, stages);
 
     PackArgs p{};
     p.wire = a.wire;
     p.wire_cols = a.wire_cols;
-    p.stream = a.stream;
-    p.row_stride = a.row_stride;
-    p.row_len = a.row_len;
-    p.n_frames = a.n_frames;
-    p.frame_len = a.frame_len;
-    p.frame_stride = a.frame_stride;
+    p.stream = f.stream;
+    p.row_stride = f.row_stride;
+    p.row_len = f.row_len;
+    p.n_frames = f.n_frames;
+    p.frame_len = f.frame_len;
+    p.frame_stride = f.frame_stride;
     p.blocks_per_frame = nblk;
     p.n_items = n_items;
-    p.index = a.index;
-    p.usable = a.usable;
+    p.index = f.index;
+    p.usable = f.usable;
     p.stage_off = a.geom.stage_off;
     p.row_chunks = a.geom.row_chunks;
     p.row_bytes = a.geom.row_bytes;
     p.copy_bytes = a.geom.copy_bytes;
-    p.packed = reinterpret_cast<float4 *>(a.packed);
+    p.packed = reinterpret_cast<float4 *>(f.packed);
     const int kWarps = a.geom.warps;
-    const int tw = a.geom.tmpl_warps;   // compiled variant (register budget) the launch uses
-    const int stages = a.geom.stages;
-    if (stages < 3) return cudaErrorInvalidConfiguration;   // ensure_tiles never selects such a geometry
-    const size_t smem = das_tile_smem_bytes(a.geom, stages);
 
     KernelArgs k{};
-    k.packed = reinterpret_cast<const char *>(a.packed);
+    k.packed = reinterpret_cast<const char *>(f.packed);
     k.tiles = static_cast<const char *>(a.tiles);
     k.tile_dirs = a.tile_dirs;
     k.n_tiles = a.n_tiles;
-    k.usable = a.usable;
-    k.n_dir = a.n_dir;
+    k.usable = f.usable;
+    k.n_dir = f.n_dir;
     k.row_bytes = a.geom.row_bytes;
     k.n_items = n_items;
     k.blocks_per_frame = nblk;
-    k.frame_len = a.frame_len;
-    k.out = nblk == 1 ? a.power : a.partial;
-    k.norm = a.norm;
+    k.frame_len = f.frame_len;
+    k.pairs_per_cta = ksplit > 1 ? 1 : block_pairs_per_cta(a.geom.pairs_per_cta, f.usable);
+    k.out = nblk == 1 ? f.power : f.partial;
+    k.norm = f.norm;
     k.stages = stages;
     k.launch_warps = kWarps;
 
@@ -582,8 +625,8 @@ cudaError_t launch_das_tile(const TileArgs &a, int sm_count, cudaStream_t st, in
         KernelArgs ks = k;
         ps.pair0 = p0;
         ks.pair0 = p0;
-        dim3 pg((a.geom.row_chunks + 255) / 256, a.usable, np);
-        dim3 wg((a.geom.row_chunks + kWireChunks - 1) / kWireChunks, (a.usable + kWireCh - 1) / kWireCh, np);
+        dim3 pg((a.geom.row_chunks + 255) / 256, f.usable, np);
+        dim3 wg((a.geom.row_chunks + kWireChunks - 1) / kWireChunks, (f.usable + kWireCh - 1) / kWireCh, np);
         if (hook) hook(hook_ctx, 1, true, st);
         if (a.wire) pack_wire_kernel<<<wg, 256, 0, st>>>(ps);
         else pack_kernel<<<pg, 256, 0, st>>>(ps);
@@ -591,97 +634,15 @@ cudaError_t launch_das_tile(const TileArgs &a, int sm_count, cudaStream_t st, in
         cudaError_t e = cudaGetLastError();
         if (e != cudaSuccess) return e;
         ks.n_pairs = np;
-        // a CTA lives ~0.6 us per channel: with few channels several block pairs per CTA hide its ramp-up and epilogue
-        ks.pairs_per_cta = a.geom.pairs_per_cta > 0 ? a.geom.pairs_per_cta : std::max(1, std::min(8, 512 / std::max(1, a.usable)));
-        // channel split across a cluster (latency shape of small calls): compiled for the 16-warp two-FMA variants
-        const int ksplit = a.geom.fast && tw == 16 && a.geom.ksplit > 1 ? a.geom.ksplit : 1;
-        if (ksplit > 1) ks.pairs_per_cta = 1;
         dim3 grid((a.n_tiles + kWarps - 1) / kWarps, (np + ks.pairs_per_cta - 1) / ks.pairs_per_cta, ksplit);
         if (hook) hook(hook_ctx, 0, true, st);
-        if (ksplit > 1 && a.geom.mode != 0) {
-            if (a.geom.nch == 6) e = launch_main<6, 16, true, true, true>(ks, grid, smem, st);
-            else e = launch_main<7, 16, true, true, true>(ks, grid, smem, st);
-        } else if (ksplit > 1) {
-            switch (a.geom.nch) {
-                case 5: e = launch_main<5, 16, false, true, true>(ks, grid, smem, st); break;
-                case 6: e = launch_main<6, 16, false, true, true>(ks, grid, smem, st); break;
-                case 7: e = launch_main<7, 16, false, true, true>(ks, grid, smem, st); break;
-                case 8: e = launch_main<8, 16, false, true, true>(ks, grid, smem, st); break;
-                case 9: e = launch_main<9, 16, false, true, true>(ks, grid, smem, st); break;
-                default: e = launch_main<10, 16, false, true, true>(ks, grid, smem, st); break;
-            }
-        } else if (a.geom.fast && a.geom.mode != 0) {
-            if (a.geom.nch == 6) {
-                switch (tw) {
-                    case 10: e = launch_main<6, 10, true, true>(ks, grid, smem, st); break;
-                    case 11: e = launch_main<6, 11, true, true>(ks, grid, smem, st); break;
-                    case 12: e = launch_main<6, 12, true, true>(ks, grid, smem, st); break;
-                    default: e = launch_main<6, 16, true, true>(ks, grid, smem, st); break;
-                }
-            } else {
-                switch (tw) {
-                    case 10: e = launch_main<7, 10, true, true>(ks, grid, smem, st); break;
-                    case 11: e = launch_main<7, 11, true, true>(ks, grid, smem, st); break;
-                    case 12: e = launch_main<7, 12, true, true>(ks, grid, smem, st); break;
-                    default: e = launch_main<7, 16, true, true>(ks, grid, smem, st); break;
-                }
-            }
-        } else if (a.geom.fast) {
-            switch (a.geom.nch) {
-#define BFLK_LAUNCH_FAST(NCH)                                                          \
-    switch (tw) {                                                            \
-        case 10: e = launch_main<NCH, 10, false, true>(ks, grid, smem, st); break;     \
-        case 11: e = launch_main<NCH, 11, false, true>(ks, grid, smem, st); break;     \
-        case 16: e = launch_main<NCH, 16, false, true>(ks, grid, smem, st); break;     \
-        default: e = launch_main<NCH, 12, false, true>(ks, grid, smem, st); break;     \
-    }
-                case 5: BFLK_LAUNCH_FAST(5) break;
-                case 6: BFLK_LAUNCH_FAST(6) break;
-                case 7: BFLK_LAUNCH_FAST(7) break;
-                case 8: BFLK_LAUNCH_FAST(8) break;
-                case 9: BFLK_LAUNCH_FAST(9) break;
-                default: BFLK_LAUNCH_FAST(10) break;
-#undef BFLK_LAUNCH_FAST
-            }
-        } else if (a.geom.mode != 0) {
-            if (a.geom.nch == 6) {
-                switch (tw) {
-                    case 10: e = launch_main<6, 10, true>(ks, grid, smem, st); break;
-                    case 11: e = launch_main<6, 11, true>(ks, grid, smem, st); break;
-                    case 12: e = launch_main<6, 12, true>(ks, grid, smem, st); break;
-                    default: e = launch_main<6, 16, true>(ks, grid, smem, st); break;
-                }
-            } else {
-                switch (tw) {
-                    case 10: e = launch_main<7, 10, true>(ks, grid, smem, st); break;
-                    case 11: e = launch_main<7, 11, true>(ks, grid, smem, st); break;
-                    default: e = launch_main<7, 12, true>(ks, grid, smem, st); break;
-                }
-            }
-        } else
-        switch (a.geom.nch) {
-#define BFLK_LAUNCH(NCH)                                                              \
-    switch (tw) {                                                            \
-        case 10: e = launch_main<NCH, 10>(ks, grid, smem, st); break;                  \
-        case 11: e = launch_main<NCH, 11>(ks, grid, smem, st); break;                  \
-        case 16: e = launch_main<NCH, 16>(ks, grid, smem, st); break;                  \
-        default: e = launch_main<NCH, 12>(ks, grid, smem, st); break;                  \
-    }
-            case 5: BFLK_LAUNCH(5) break;
-            case 6: BFLK_LAUNCH(6) break;
-            case 7: BFLK_LAUNCH(7) break;
-            case 8: BFLK_LAUNCH(8) break;
-            default: BFLK_LAUNCH(10) break;
-#undef BFLK_LAUNCH
-        }
+        e = kTileLaunchers[variant](ks, grid, smem, st);
         if (hook) hook(hook_ctx, 0, false, st);
         if (e != cudaSuccess) return e;
         *launches += 2;
     }
     if (nblk > 1) {
-        dim3 fg((a.n_dir + 255) / 256, std::min(a.n_frames, 65535));
-        finalize_kernel<<<fg, 256, 0, st>>>(a.partial, a.n_frames, nblk, a.n_dir, a.norm, a.power);
-        cudaError_t e = cudaGetLastError();
+        cudaError_t e = launch_finalize(f, st);
         if (e != cudaSuccess) return e;
         *launches += 1;
     }
