@@ -30,11 +30,11 @@ SYMBOLS = [
     "bflk_set_grid_fov", "bflk_set_grid_tables", "bflk_set_grid_shape", "bflk_set_direction_range", "bflk_get_n_directions",
     "bflk_get_grid", "bflk_get_tables", "bflk_steer_tables", "bflk_power_map", "bflk_power_map_i32",
     "bflk_power_map_batch", "bflk_power_map_batch_submit", "bflk_power_map_batch_wait", "bflk_power_map_batch_i32", "bflk_power_map_batch_i32_dev",
-    "bflk_power_map_batch_dev", "bflk_power_map_batch_dev_submit", "bflk_power_map_batch_dev_join", "bflk_set_kernel", "bflk_set_channel_split", "bflk_launch_shape", "bflk_get_kernel", "bflk_launch_count", "bflk_enable_timing",
+    "bflk_power_map_batch_dev", "bflk_beams_batch_dev", "bflk_power_map_batch_dev_submit", "bflk_power_map_batch_dev_join", "bflk_set_kernel", "bflk_set_channel_split", "bflk_launch_shape", "bflk_get_kernel", "bflk_launch_count", "bflk_enable_timing",
     "bflk_kernel_time_ms", "bflk_fp32_peak_tflops", "bflk_set_window", "bflk_set_window_dev", "bflk_miso", "bflk_miso_dev", "bflk_monopulse", "bflk_set_fir",
     "bflk_pin_host", "bflk_unpin_host", "bflk_heatmap", "bflk_resize_u8", "bflk_targets", "bflk_calibrate", "bflk_ingest_i32",
     "bflk_stream_open", "bflk_stream_close", "bflk_stream_push", "bflk_stream_push_i32", "bflk_stream_power_maps",
-    "bflk_stream_discard", "bflk_stream_status", "bflk_stream_window",
+    "bflk_stream_discard", "bflk_stream_status", "bflk_stream_window", "bflk_session_beams",
     "bflk_comm_unique_id", "bflk_comm_init_rank", "bflk_comm_info", "bflk_shard_plan",
     "bflk_power_map_batch_sharded_dev", "bflk_power_map_batch_sharded_dev_submit", "bflk_power_map_batch_sharded_dev_join", "bflk_power_map_batch_sharded", "bflk_power_map_batch_sharded_submit", "bflk_power_map_batch_sharded_wait",
     "bflk_group_create", "bflk_group_destroy", "bflk_group_size", "bflk_group_handle", "bflk_group_last_error",
@@ -101,6 +101,7 @@ def load_library():
     L.bflk_power_map_batch_i32.argtypes = [vp, vp, i64, i32, vp]
     L.bflk_power_map_batch_i32_dev.argtypes = [vp, vp, i64, i32, vp, vp]
     L.bflk_power_map_batch_dev.argtypes = [vp, vp, i64, i32, vp, vp]
+    L.bflk_beams_batch_dev.argtypes = [vp, vp, i64, i32, vp, vp, vp]
     L.bflk_power_map_batch_dev_submit.argtypes = [vp, vp, i64, i32, vp, vp]
     L.bflk_power_map_batch_dev_join.argtypes = [vp, vp]
     L.bflk_set_kernel.argtypes = [vp, i32]
@@ -130,6 +131,7 @@ def load_library():
     L.bflk_stream_push.argtypes = [vp, vp, i32]
     L.bflk_stream_push_i32.argtypes = [vp, vp, i32]
     L.bflk_stream_power_maps.argtypes = [vp, i32, vp, C.POINTER(i64), C.POINTER(i32)]
+    L.bflk_session_beams.argtypes = [vp, i32, vp, vp, C.POINTER(i64), C.POINTER(i32)]
     L.bflk_stream_discard.argtypes = [vp, i32]
     L.bflk_stream_status.argtypes = [vp, C.POINTER(i64), C.POINTER(i64), C.POINTER(i32), C.POINTER(i64)]
     L.bflk_stream_window.argtypes = [vp, i64]
@@ -431,6 +433,11 @@ class Beamformer:
         self._check(self._L.bflk_power_map_batch_dev(self._h, C.c_void_p(stream_dev_ptr), n_samples, n_frames,
                                                      C.c_void_p(power_dev_ptr), C.c_void_p(cuda_stream)))
 
+    def beams_batch_dev(self, stream_dev_ptr, n_samples, n_frames, beams_dev_ptr, power_dev_ptr, cuda_stream=0):
+        """power_map_batch_dev that also writes the delayed sums its maps square: beams [B][count][N] (device, 8-byte aligned)."""
+        self._check(self._L.bflk_beams_batch_dev(self._h, C.c_void_p(stream_dev_ptr), n_samples, n_frames,
+                                                 C.c_void_p(beams_dev_ptr), C.c_void_p(power_dev_ptr), C.c_void_p(cuda_stream)))
+
     def power_map_batch_dev_submit(self, stream_dev_ptr, n_samples, n_frames, power_dev_ptr, cuda_stream=0):
         """Continuous operation (bflk.h): consecutive batches overlap on the handle's two compute streams; complete after _dev_join."""
         self._check(self._L.bflk_power_map_batch_dev_submit(self._h, C.c_void_p(stream_dev_ptr), n_samples, n_frames,
@@ -510,6 +517,15 @@ class Beamformer:
         first, n = C.c_int64(), C.c_int32()
         self._check(self._L.bflk_stream_power_maps(self._h, max_frames, _ptr(out), C.byref(first), C.byref(n)))
         return first.value, out[:n.value].copy()
+
+    def stream_beams(self, max_frames=1):
+        """stream_power_maps with the frames' beams: (first_frame, beams [n][count][N], power [n][count]), n may be 0."""
+        count = self.n_directions()[2]
+        beams = np.zeros((max_frames, count, self.frame_len), np.float32)
+        out = np.zeros((max_frames, count), np.float32)
+        first, n = C.c_int64(), C.c_int32()
+        self._check(self._L.bflk_session_beams(self._h, max_frames, _ptr(beams), _ptr(out), C.byref(first), C.byref(n)))
+        return first.value, beams[:n.value].copy(), out[:n.value].copy()
 
     def stream_discard(self, keep=0):
         """Skip every ready frame but the newest `keep`."""

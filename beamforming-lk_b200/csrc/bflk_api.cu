@@ -676,7 +676,7 @@ int bflk::lanes_join(bflk_handle *h, int only) {
 }
 
 int bflk::power_map_dev(bflk_handle *h, const float *stream_dev, int64_t row_stride, int64_t n_samples, int32_t n_frames,
-                        float *power_dev, const Launch &launch) {
+                        float *power_dev, const Launch &launch, float *beams_dev) {
     if (!h) return BFLK_ERR_INVALID;
     if (!h->have_grid) return h->fail(BFLK_ERR_STATE, "bflk_power_map: set geometry and grid first");
     const int32_t *wire = launch.wire;   // wire-format call: stream_dev is null, the samples are wire[n_samples][C]
@@ -753,7 +753,7 @@ int bflk::power_map_dev(bflk_handle *h, const float *stream_dev, int64_t row_str
         a.usable = usable;
         a.n_dir = h->dir_count;
         a.power = power_dev;
-        a.audio = nullptr;
+        a.audio = beams_dev;
         a.norm = norm;
         if (fir) { a.fir = h->d_fir.p; a.fir_phases = h->fir_phases; a.fir_taps = h->fir_taps; }
         timing_hook(h, 0, true, st);
@@ -779,6 +779,7 @@ int bflk::power_map_dev(bflk_handle *h, const float *stream_dev, int64_t row_str
     f.n_dir = h->dir_count;
     f.index = h->d_index.p;
     f.power = power_dev;
+    f.beams = beams_dev;
     f.norm = norm;
     BFLK_CUDA(h, d_packed.reserve(packed_bytes(f, tiled ? h->tile_geom.row_bytes : h->bcast_geom.row_bytes)));
     f.packed = d_packed.p;
@@ -844,6 +845,13 @@ extern "C" {
 int bflk_power_map_batch_dev(bflk_handle *h, const float *stream_dev, int64_t n_samples, int32_t n_frames,
                              float *power_dev, void *cuda_stream) {
     return power_map_dev(h, stream_dev, n_samples, n_samples, n_frames, power_dev, Launch{(cudaStream_t)cuda_stream});
+}
+
+int bflk_beams_batch_dev(bflk_handle *h, const float *stream_dev, int64_t n_samples, int32_t n_frames, float *beams_dev,
+                         float *power_dev, void *cuda_stream) {
+    if (!h) return BFLK_ERR_INVALID;
+    if (!beams_dev || ((uintptr_t)beams_dev & 7)) return h->fail(BFLK_ERR_INVALID, "bflk_beams_batch_dev: beams_dev is null or not 8-byte aligned");
+    return power_map_dev(h, stream_dev, n_samples, n_samples, n_frames, power_dev, Launch{(cudaStream_t)cuda_stream}, beams_dev);
 }
 
 int bflk_power_map_batch_dev_submit(bflk_handle *h, const float *stream_dev, int64_t n_samples, int32_t n_frames,
@@ -1485,35 +1493,50 @@ int bflk_stream_push_i32(bflk_handle *h, const int32_t *rows, int32_t n) {
     return stream_push(h, rows, n, true, "bflk_stream_push_i32");
 }
 
-int bflk_stream_power_maps(bflk_handle *h, int32_t max_frames, float *power_out, int64_t *first_frame, int32_t *n_frames) {
+// bflk_stream_power_maps, and with_beams: bflk_session_beams -- the same frames, consumed the same way
+static int stream_maps(bflk_handle *h, int32_t max_frames, float *power_out, bool with_beams, float *beams_out,
+                       int64_t *first_frame, int32_t *n_frames, const char *who) {
     if (!h) return BFLK_ERR_INVALID;
-    Session *s = session_of(h, "bflk_stream_power_maps");
+    Session *s = session_of(h, who);
     if (!s) return BFLK_ERR_STATE;
-    if (!power_out || !first_frame || !n_frames || max_frames < 1)
-        return h->fail(BFLK_ERR_INVALID, "bflk_stream_power_maps: null output or max_frames = %d", max_frames);
-    if (!h->have_grid) return h->fail(BFLK_ERR_STATE, "bflk_stream_power_maps: set geometry and grid first");
+    if (!power_out || (with_beams && !beams_out) || !first_frame || !n_frames || max_frames < 1)
+        return h->fail(BFLK_ERR_INVALID, "%s: null output or max_frames = %d", who, max_frames);
+    if (!h->have_grid) return h->fail(BFLK_ERR_STATE, "%s: set geometry and grid first", who);
     const int64_t tail = frame_tail_samples(h);
     if (tail > s->tail)
-        return h->fail(BFLK_ERR_STATE, "bflk_stream_power_maps: a frame now reads %lld samples past its own, the session was opened for %lld (open it again)",
-                       (long long)tail, (long long)s->tail);
+        return h->fail(BFLK_ERR_STATE, "%s: a frame now reads %lld samples past its own, the session was opened for %lld (open it again)",
+                       who, (long long)tail, (long long)s->tail);
     *first_frame = s->next_frame;
     *n_frames = 0;
     const int k = (int)std::min<int64_t>(max_frames, ready_frames(h, s));
     if (k == 0) return BFLK_OK;
     const int N = h->cfg.frame_len;
+    const size_t n_beams = (size_t)k * h->dir_count * N;
     BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
     h->last_map_on_device = false;
     BFLK_CUDA(h, h->d_maps.reserve((size_t)k * h->dir_count));
+    if (with_beams) BFLK_CUDA(h, h->d_beams.reserve(n_beams));
     // the k frames and the tail of the last one: ready and still held, so at most cap samples, contiguous in the ring
     const float *window = s->ring.p + s->next_frame * N % s->cap;
-    int rc = power_map_dev(h, window, 2 * s->cap, (int64_t)k * N + tail, k, h->d_maps.p, Launch{h->stream});
+    int rc = power_map_dev(h, window, 2 * s->cap, (int64_t)k * N + tail, k, h->d_maps.p, Launch{h->stream},
+                           with_beams ? h->d_beams.p : nullptr);
     if (rc) return rc;
     BFLK_CUDA(h, cudaMemcpyAsync(power_out, h->d_maps.p, (size_t)k * h->dir_count * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+    if (with_beams) BFLK_CUDA(h, cudaMemcpyAsync(beams_out, h->d_beams.p, n_beams * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
     BFLK_CUDA(h, cudaStreamSynchronize(h->stream));
     s->next_frame += k;
     *n_frames = k;
     h->last_map_on_device = k == 1;   // d_maps[0 .. count) is the map: bflk_targets(NULL) / bflk_heatmap(NULL) use it
     return BFLK_OK;
+}
+
+int bflk_stream_power_maps(bflk_handle *h, int32_t max_frames, float *power_out, int64_t *first_frame, int32_t *n_frames) {
+    return stream_maps(h, max_frames, power_out, false, nullptr, first_frame, n_frames, "bflk_stream_power_maps");
+}
+
+int bflk_session_beams(bflk_handle *h, int32_t max_frames, float *beams_out, float *power_out, int64_t *first_frame,
+                       int32_t *n_frames) {
+    return stream_maps(h, max_frames, power_out, true, beams_out, first_frame, n_frames, "bflk_session_beams");
 }
 
 int bflk_stream_discard(bflk_handle *h, int32_t keep) {

@@ -265,6 +265,7 @@ struct bflk_handle {
     // maps of the synchronous host batches (bflk_power_map_batch, bflk_power_map_batch_i32); nothing else writes them
     bflk::DevBuf<float> d_maps;
     bool last_map_on_device = false;          // d_maps holds the [count] map of the last batch, which had one frame
+    bflk::DevBuf<float> d_beams;              // delayed sums of a session's maps call that returns them (bflk_session_beams)
     bflk::DevBuf<float> d_post;               // host map of bflk_heatmap / bflk_targets, channel powers of bflk_calibrate
     bflk::DevBuf<float> d_resident;
     bflk::DevBuf<float> d_miso_out;           // [flag | audio | power]: one D2H copy per call
@@ -406,6 +407,7 @@ struct FrameArgs {
     void *packed = nullptr;          // packed_bytes() of scratch
     float *power = nullptr;          // [B][n_dir]
     float *partial = nullptr;        // [B * blocks_per_frame][n_dir] when frame_len > 256
+    float *beams = nullptr;          // [B][n_dir][frame_len] delayed sums the power squares (8-byte aligned), or nullptr
     float norm = 0.f;
 };
 // bytes of the packed rows of a call: one row of row_bytes per (block pair, usable channel)
@@ -477,9 +479,10 @@ struct Launch {
     bool pipelined = false;          // on a lane: no caller_event wait or record; throughput CTA shape (tables built by lanes_fork)
     const int32_t *wire = nullptr;   // wire-format input [n_samples][C] instead of stream_dev
 };
-// stream_dev: first sample of frame 0; rows are row_stride floats apart and hold n_samples valid samples
+// stream_dev: first sample of frame 0; rows are row_stride floats apart and hold n_samples valid samples.  beams_dev: also
+// the delayed sums the maps square, [n_frames][count][frame_len] (8-byte aligned), or nullptr
 int power_map_dev(bflk_handle *h, const float *stream_dev, int64_t row_stride, int64_t n_samples, int32_t n_frames,
-                  float *power_dev, const Launch &launch);
+                  float *power_dev, const Launch &launch, float *beams_dev = nullptr);
 // Continuous operation: the same as power_map_dev, but enqueued on one of the handle's two lanes (alternating, each with its
 // own scratch) after `caller` has reached this point; *used = the stream the kernels are on.  Consecutive calls overlap: the
 // pack pre-pass of batch i + 1 runs under the kernel of batch i and its CTAs fill the SMs the last CTAs of batch i leave

@@ -17,7 +17,8 @@
 //  * rows and per-(channel, lane) {offset, fraction} tables are staged with cp.async.bulk (TMA bulk
 //    copy) into a 3-stage mbarrier pipeline, 8 channels per stage.
 //  * epilogue: 3-tap high-pass + squares (mimo.cpp:131-135); chunk-edge samples are exchanged through
-//    shared memory, per-direction sums reduced across the 16 warps in fixed order.
+//    shared memory, per-direction sums reduced across the 16 warps in fixed order; beams calls also store the
+//    delayed sums.
 #include "bflk_internal.h"
 #include "das_common.cuh"
 
@@ -65,8 +66,12 @@ struct KernelArgs {
     int n_items, nblk, frame_len, pair0;
     float *out;                 // power [frames][n_dir] (nblk == 1) or partial [items][n_dir]
     float norm;
+    float *beams;               // delayed sums [frames][n_dir][frame_len] (BEAMS instantiation only; FrameArgs::beams)
 };
 
+// BEAMS: the epilogue also stores the delayed sums (beams calls); a template flag, so that the power-only kernel is compiled
+// exactly as without it
+template <bool BEAMS>
 __global__ void __launch_bounds__(kThreads, 1) bcast_kernel(KernelArgs a) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int stage_rows = kCC * a.row_bytes;
@@ -159,6 +164,26 @@ __global__ void __launch_bounds__(kThreads, 1) bcast_kernel(KernelArgs a) {
         if (j >= jloA && j <= jhiA) pa = __fmaf_rn(ma, ma, pa);
         if (j >= jloB && j <= jhiB) pb = __fmaf_rn(mb, mb, pb);
     }
+    // beams calls: every block stores the frame samples it owns (item_beam_range), a lane its direction's 16 samples in
+    // 8-byte pairs (even bounds, rows start at even samples)
+    if constexpr (BEAMS) {
+        const int dir = a.tile_dirs[tile * 32 + lane];
+#pragma unroll
+        for (int h = 0; h < 2; h++) {
+            const int item = h ? itemB : itemA;
+            if (dir < 0 || item >= a.n_items) continue;
+            int blo, bhi;
+            item_beam_range(item, a.nblk, a.frame_len, blo, bhi);
+            const int b = item / a.nblk, q = item - b * a.nblk;
+            float *row = a.beams + ((size_t)b * a.n_dir + dir) * a.frame_len + block_first_sample(q, a.frame_len);
+#pragma unroll
+            for (int k = 0; k < kK; k += 2) {
+                const int j = kK * warp + k;
+                if (j >= blo && j < bhi)
+                    *reinterpret_cast<float2 *>(row + j) = h ? make_float2(hi(acc[k]), hi(acc[k + 1])) : make_float2(lo(acc[k]), lo(acc[k + 1]));
+            }
+        }
+    }
     part[warp * 32 + lane] = make_float2(pa, pb);
     __syncthreads();
     if (warp == 0) {
@@ -242,7 +267,8 @@ cudaError_t launch_das_bcast(const BcastArgs &a, cudaStream_t st, int *launches,
     if (f.frame_len < kBlock) return cudaErrorInvalidValue;
     const size_t smem = bcast_smem_bytes(a.geom);
     if (!das_bcast_fits(a.geom)) return cudaErrorInvalidConfiguration;
-    cudaError_t e = cudaFuncSetAttribute(bcast_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    void (*const kernel)(KernelArgs) = f.beams ? bcast_kernel<true> : bcast_kernel<false>;
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
 
     PackArgs p{};
@@ -270,6 +296,7 @@ cudaError_t launch_das_bcast(const BcastArgs &a, cudaStream_t st, int *launches,
     k.nblk = nblk;
     k.frame_len = f.frame_len;
     k.out = nblk == 1 ? f.power : f.partial;
+    k.beams = f.beams;
     k.norm = f.norm;
 
     const int max_slab = 32768;  // grid.y / grid.z limits
@@ -283,7 +310,7 @@ cudaError_t launch_das_bcast(const BcastArgs &a, cudaStream_t st, int *launches,
         if ((e = cudaGetLastError()) != cudaSuccess) return e;
         dim3 grid(a.n_tiles, np);
         if (hook) hook(hook_ctx, 0, true, st);
-        bcast_kernel<<<grid, kThreads, smem, st>>>(k);
+        kernel<<<grid, kThreads, smem, st>>>(k);
         if (hook) hook(hook_ctx, 0, false, st);
         if ((e = cudaGetLastError()) != cudaSuccess) return e;
         *launches += 2;

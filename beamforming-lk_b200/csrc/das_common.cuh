@@ -84,6 +84,14 @@ __device__ __forceinline__ void item_ma_range(int item, int nblk, int frame_len,
     jlo = 254 * q + 1 - s;
     jhi = min(254 * q + 254, frame_len - 2) - s;
 }
+// the delayed sums (beams) block q of a frame stores, so that every frame sample is written exactly once: frame samples
+// [254 q, 254 q + 254), the last block [254 q, N) -- as block samples [jlo, jhi), inside [0, 256), both bounds even
+__device__ __forceinline__ void item_beam_range(int item, int nblk, int frame_len, int &jlo, int &jhi) {
+    const int q = item % nblk;
+    const int s = block_first_sample(q, frame_len);
+    jlo = 254 * q - s;
+    jhi = (q == nblk - 1 ? frame_len : 254 * q + 254) - s;
+}
 
 }  // namespace
 }  // namespace bflk

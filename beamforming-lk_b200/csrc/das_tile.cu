@@ -22,7 +22,7 @@
 //        g = 1 - f from the table -- 16 FFMA2 per (direction, channel) and nothing else on the FP pipe,
 //        the whole pipeline stage in one generated PTX block (das_tile_fast_asm.inc).
 //  * epilogue: 3-tap high-pass + squares (mimo.cpp:131-135) with neighbour samples from lane +-1,
-//    warp-shuffle reduction, one store per (block, direction).
+//    warp-shuffle reduction, one store per (block, direction); beams calls also store the delayed sums.
 #include <algorithm>
 #include <array>
 #include <cstdlib>
@@ -155,6 +155,7 @@ struct KernelArgs {
     int launch_warps;            // warps per CTA of this launch (host side: <= the compiled variant's)
     float *out;                  // power [frames][n_dir] (blocks_per_frame == 1) or partial [items][n_dir]
     float norm;
+    float *beams;                // delayed sums [frames][n_dir][frame_len] (BEAMS instantiations only; FrameArgs::beams)
 };
 
 #include "das_tile_asm.inc"
@@ -167,7 +168,9 @@ struct KernelArgs {
 //       them and add their partial delayed sums through distributed shared memory, in rank order, before the epilogue.
 //       For calls too small to fill the SMs (a live worker's single frame: cfg3 is 16 CTAs): the serial channel loop gets
 //       shorter by the cluster size.  The channel sum is re-associated (rank sums added at the end), so FAST only.
-template <int NCH, int kWarps, bool DUAL = false, bool FAST = false, bool KSPLIT = false>
+// BEAMS: the epilogue also stores the delayed sums (beams calls).  A template flag, not a run-time test: even a branch the
+//       power-only calls never take changes how ptxas allocates registers around the channel loop (more moves inside it).
+template <int NCH, int kWarps, bool DUAL = false, bool FAST = false, bool KSPLIT = false, bool BEAMS = false>
 __global__ void __launch_bounds__(kWarps * 32, 1) das_tile_kernel(KernelArgs a) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     constexpr int kEnt = FAST ? (DUAL ? (int)sizeof(TileEntryFastDual) : (int)sizeof(TileEntryFast)) : (int)sizeof(TileEntry);
@@ -356,6 +359,29 @@ __global__ void __launch_bounds__(kWarps * 32, 1) das_tile_kernel(KernelArgs a) 
                 }
             }
         }
+        // beams calls: every block stores the frame samples it owns (item_beam_range); the bounds are even and rows start
+        // at even samples, so a lane's samples go out in 8-byte pairs
+        if (BEAMS && active) {
+            const int dir = a.tile_dirs[4 * my_tile + r];
+            if (dir >= 0) {
+#pragma unroll
+                for (int h = 0; h < 2; h++) {
+                    const int item = h ? itemB : itemA;
+                    if (item >= a.n_items) continue;
+                    int blo, bhi;
+                    item_beam_range(item, a.blocks_per_frame, a.frame_len, blo, bhi);
+                    const int b = item / a.blocks_per_frame, q = item - b * a.blocks_per_frame;
+                    float *row = a.beams + ((size_t)b * a.n_dir + dir) * a.frame_len + block_first_sample(q, a.frame_len);
+#pragma unroll
+                    for (int k = 0; k < kK; k += 2) {
+                        const int j = kK * lane + k;
+                        const u64 v0 = acc[r][k], v1 = acc[r][k + 1];
+                        if (j >= blo && j < bhi)
+                            *reinterpret_cast<float2 *>(row + j) = h ? make_float2(hi(v0), hi(v1)) : make_float2(lo(v0), lo(v1));
+                    }
+                }
+            }
+        }
     }
     }  // block pairs of this CTA
 }
@@ -512,14 +538,14 @@ size_t das_tile_entry_bytes(const TileGeometry &g) {
     return g.fast ? (g.mode ? sizeof(TileEntryFastDual) : sizeof(TileEntryFast)) : sizeof(TileEntry);
 }
 
-template <int NCH, int WARPS, bool DUAL = false, bool FAST = false, bool KSPLIT = false>
+template <int NCH, int WARPS, bool DUAL = false, bool FAST = false, bool KSPLIT = false, bool BEAMS = false>
 static cudaError_t launch_main(const KernelArgs &k, dim3 grid, size_t smem, cudaStream_t st) {
     // the attribute is per device and only ever grows: set it when a larger request appears there, not per launch
     static size_t configured[64] = {0};
     int dev = 0;
     cudaGetDevice(&dev);
     if (dev < 0 || dev >= 64 || smem > configured[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(das_tile_kernel<NCH, WARPS, DUAL, FAST, KSPLIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = cudaFuncSetAttribute(das_tile_kernel<NCH, WARPS, DUAL, FAST, KSPLIT, BEAMS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
         if (dev >= 0 && dev < 64) configured[dev] = smem;
     }
@@ -538,20 +564,22 @@ static cudaError_t launch_main(const KernelArgs &k, dim3 grid, size_t smem, cuda
         attr.val.clusterDim.z = grid.z;
         cfg.attrs = &attr;
         cfg.numAttrs = 1;
-        return cudaLaunchKernelEx(&cfg, das_tile_kernel<NCH, WARPS, DUAL, FAST, KSPLIT>, k);
+        return cudaLaunchKernelEx(&cfg, das_tile_kernel<NCH, WARPS, DUAL, FAST, KSPLIT, BEAMS>, k);
     }
-    das_tile_kernel<NCH, WARPS, DUAL, FAST, KSPLIT><<<grid, warps * 32, smem, st>>>(k);
+    das_tile_kernel<NCH, WARPS, DUAL, FAST, KSPLIT, BEAMS><<<grid, warps * 32, smem, st>>>(k);
     return cudaGetLastError();
 }
 
 using TileLauncher = cudaError_t (*)(const KernelArgs &, dim3, size_t, cudaStream_t);
-template <size_t... I>
+template <bool BEAMS, size_t... I>
 static constexpr std::array<TileLauncher, sizeof...(I)> tile_launchers(std::index_sequence<I...>) {
     return {launch_main<kTileVariants[I].nch, kTileVariants[I].warps, kTileVariants[I].dual, kTileVariants[I].fast,
-                        kTileVariants[I].ksplit>...};
+                        kTileVariants[I].ksplit, BEAMS>...};
 }
-// kTileLaunchers[i] launches kTileVariants[i]
-static constexpr auto kTileLaunchers = tile_launchers(std::make_index_sequence<kNumTileVariants>());
+// kTileLaunchers[beams][i] launches kTileVariants[i], the power-only or the beams instantiation
+static constexpr std::array<TileLauncher, kNumTileVariants> kTileLaunchers[2] = {
+    tile_launchers<false>(std::make_index_sequence<kNumTileVariants>()),
+    tile_launchers<true>(std::make_index_sequence<kNumTileVariants>())};
 
 cudaError_t launch_das_tile(const TileArgs &a, int sm_count, cudaStream_t st, int *launches, TileLaunchHook hook, void *hook_ctx) {
     (void)sm_count;
@@ -600,6 +628,7 @@ cudaError_t launch_das_tile(const TileArgs &a, int sm_count, cudaStream_t st, in
     k.frame_len = f.frame_len;
     k.pairs_per_cta = ksplit > 1 ? 1 : block_pairs_per_cta(a.geom.pairs_per_cta, f.usable);
     k.out = nblk == 1 ? f.power : f.partial;
+    k.beams = f.beams;
     k.norm = f.norm;
     k.stages = stages;
     k.launch_warps = kWarps;
@@ -636,7 +665,7 @@ cudaError_t launch_das_tile(const TileArgs &a, int sm_count, cudaStream_t st, in
         ks.n_pairs = np;
         dim3 grid((a.n_tiles + kWarps - 1) / kWarps, (np + ks.pairs_per_cta - 1) / ks.pairs_per_cta, ksplit);
         if (hook) hook(hook_ctx, 0, true, st);
-        e = kTileLaunchers[variant](ks, grid, smem, st);
+        e = kTileLaunchers[f.beams != nullptr][variant](ks, grid, smem, st);
         if (hook) hook(hook_ctx, 0, false, st);
         if (e != cudaSuccess) return e;
         *launches += 2;

@@ -17,6 +17,7 @@
  *   bflk_set_grid_tables            the same LUT supplied by the caller (offsetDelays / fractionalDelays, mimo.h:86-89)
  *   bflk_steer_tables               Particle::steer (src/dsp/particle.cpp:37-49)
  *   bflk_power_map*                 MIMOWorker::update (src/dsp/mimo.cpp:97-151) -> powerdB
+ *   bflk_beams_batch_dev, bflk_session_beams   the same, with the delayed sums out[] of every direction (mimo.cpp:121-130)
  *   bflk_power_map_batch*_submit / _wait / _join   the same in continuous operation (the reference's worker loop,
  *                                   src/dsp/worker.h:212-224, calls update() frame after frame): batches overlap their
  *                                   uploads, pre-passes and collectives with the kernels of their neighbours
@@ -135,6 +136,15 @@ int bflk_power_map_batch_i32_dev(bflk_handle *h, const int32_t *frames_dev, int6
 /* Same with DEVICE pointers, asynchronous on cuda_stream (a cudaStream_t, NULL = the handle's stream). */
 int bflk_power_map_batch_dev(bflk_handle *h, const float *stream_dev, int64_t n_samples, int32_t n_frames,
                              float *power_dev, void *cuda_stream);
+/* The beams with the maps: beams_dev[B][count][N] = for frame b and direction first + k of the range, the delayed sum
+ * out[i] (i < N) that its power squares (MIMOWorker::update, src/dsp/mimo.cpp:121-130, before the high-pass): the channels
+ * in mask order over stream[c][b*N + offset + i], interpolated as the kernel in use interpolates.  Kernels 1, 2 and 3 give
+ * the bits of the reference's delay(); kernel 4 (and the channel split) the two-FMA form's sums, within a few roundings
+ * per channel of them; with bflk_set_fir the FIR sums.  power_dev[B][count] holds the bits bflk_power_map_batch_dev gives
+ * on the same input.  stream_dev as there; beams_dev (8-byte aligned) and power_dev are required device buffers.
+ * Asynchronous on cuda_stream; argument checks and error codes as bflk_power_map_batch_dev. */
+int bflk_beams_batch_dev(bflk_handle *h, const float *stream_dev, int64_t n_samples, int32_t n_frames, float *beams_dev,
+                         float *power_dev, void *cuda_stream);
 /* Continuous operation on DEVICE-resident streams: _dev_submit enqueues the batch on one of the handle's two compute streams
  * (alternating, each with its own scratch) once cuda_stream has reached the call, and returns; consecutive batches overlap --
  * the pack pre-pass of batch i + 1 runs under the kernel of batch i and its CTAs fill the SMs the last CTAs of batch i leave
@@ -202,6 +212,9 @@ int bflk_kernel_time_ms(bflk_handle *h, float *das_ms, int32_t *das_launches, fl
  * in the latency shape -- into power_out[n][count] for the current direction range, reports the first frame and n, and
  * consumes them.  Nothing ready: *n_frames = 0, BFLK_OK, and nothing else changes.  Synchronous on the handle's stream;
  * after a call that returned one frame, bflk_targets / bflk_heatmap with a NULL map use it (as after bflk_power_map).
+ * bflk_session_beams is bflk_stream_power_maps that also returns the frames' beams (bflk_beams_batch_dev):
+ * beams_out[n][count][N] and power_out[n][count] on the host.  It takes and consumes frames exactly as the maps call does
+ * (the two may be interleaved), and after a one-frame call bflk_targets / bflk_heatmap with a NULL map use that frame's map.
  * bflk_stream_discard skips every ready frame but the newest `keep`.  bflk_stream_status: samples pushed per channel, the
  * next frame a maps call returns, frames ready, frames skipped so far.
  *
@@ -214,6 +227,8 @@ int bflk_stream_close(bflk_handle *h);
 int bflk_stream_push(bflk_handle *h, const float *samples, int32_t n);      /* [C][n], channel-major */
 int bflk_stream_push_i32(bflk_handle *h, const int32_t *rows, int32_t n);   /* [n][C], wire order */
 int bflk_stream_power_maps(bflk_handle *h, int32_t max_frames, float *power_out, int64_t *first_frame, int32_t *n_frames);
+int bflk_session_beams(bflk_handle *h, int32_t max_frames, float *beams_out, float *power_out, int64_t *first_frame,
+                       int32_t *n_frames);
 int bflk_stream_discard(bflk_handle *h, int32_t keep);
 int bflk_stream_status(const bflk_handle *h, int64_t *pushed, int64_t *next_frame, int32_t *ready, int64_t *skipped);
 int bflk_stream_window(bflk_handle *h, int64_t frame);
