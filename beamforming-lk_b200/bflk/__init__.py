@@ -658,14 +658,6 @@ class Group:
     def size(self):
         return int(self._L.bflk_group_size(self._g))
 
-    def power_map_batch_i32(self, frames, n_frames):
-        """frames [T][C] int32 wire samples (one row per time sample), frame b at row b*N -> power [B][count]."""
-        frames = _np(frames, np.int32)
-        assert frames.shape[1] == self.n_channels
-        out = np.zeros((n_frames, self.n_directions()[2]), np.float32)
-        self._check(self._L.bflk_power_map_batch_i32(self._h, _ptr(frames), frames.shape[0], n_frames, _ptr(out)))
-        return out
-
     def power_map_batch(self, stream, n_frames):
         stream = _np(stream, np.float32)
         out = np.zeros((n_frames, self.n_dir), np.float32)

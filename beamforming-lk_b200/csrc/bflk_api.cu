@@ -98,8 +98,7 @@ int bflk_destroy(bflk_handle *h) {
 // ---- geometry -----------------------------------------------------------------------------------------
 static void invalidate_tables(bflk_handle *h) {
     h->have_grid = false;
-    h->tiles_valid = false;
-    h->bcast_valid = false;
+    h->drop_kernel_tables();
     h->n_dir = 0;
     h->dir_first = h->dir_count = 0;
     h->last_map_on_device = false;
@@ -163,11 +162,10 @@ int bflk_set_channel_mask(bflk_handle *h, const int32_t *index, int32_t usable) 
     }
     BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
     h->index = idx;
-    h->bcast_valid = false;
+    h->drop_kernel_tables();
     BFLK_CUDA(h, h->d_index.reserve(idx.size()));
     BFLK_CUDA(h, cudaMemcpyAsync(h->d_index.p, h->index.data(), idx.size() * sizeof(int32_t), cudaMemcpyHostToDevice, h->stream));
     BFLK_CUDA(h, cudaStreamSynchronize(h->stream));
-    h->tiles_valid = false;
     return BFLK_OK;
 }
 
@@ -303,8 +301,7 @@ int bflk_set_grid_shape(bflk_handle *h, int32_t rows, int32_t cols) {
         return h->fail(BFLK_ERR_INVALID, "bflk_set_grid_shape: %d x %d is not the %d directions of the tables", rows, cols, h->n_dir);
     h->rows = rows;
     h->cols = cols;
-    h->tiles_valid = false;
-    h->bcast_valid = false;
+    h->drop_kernel_tables();
     return BFLK_OK;
 }
 
@@ -315,8 +312,7 @@ int bflk_set_direction_range(bflk_handle *h, int32_t first, int32_t count) {
         return h->fail(BFLK_ERR_INVALID, "bflk_set_direction_range: [%d, %d) outside grid of %d", first, first + count, h->n_dir);
     h->dir_first = first;
     h->dir_count = count;
-    h->tiles_valid = false;
-    h->bcast_valid = false;
+    h->drop_kernel_tables();
     h->last_map_on_device = false;   // the map left on the device covers the old range
     return BFLK_OK;
 }
@@ -369,8 +365,8 @@ int bflk_steer_tables(bflk_handle *h, const double *theta, const double *phi, in
 // ---- power map ---------------------------------------------------------------------------------------------
 int bflk_set_kernel(bflk_handle *h, int32_t which) {
     if (!h) return BFLK_ERR_INVALID;
-    if (which < 0 || which > 4) return h->fail(BFLK_ERR_INVALID, "bflk_set_kernel: %d", which);
-    h->kernel_choice = which;
+    if (which < kAuto || which > kTiledFma2) return h->fail(BFLK_ERR_INVALID, "bflk_set_kernel: %d", which);
+    h->kernel_choice = (Kernel)which;
     return BFLK_OK;
 }
 
@@ -396,8 +392,8 @@ int64_t bflk_launch_count(const bflk_handle *h) { return h ? h->launches : 0; }
 int bflk_get_kernel(const bflk_handle *h, int32_t *last_used, int32_t *tile_span, int32_t *window_chunks) {
     if (!h) return BFLK_ERR_INVALID;
     if (last_used) *last_used = h->kernel_last;
-    if (tile_span) *tile_span = h->tiles_valid ? h->tile_smax : -1;
-    if (window_chunks) *window_chunks = (h->tiles_valid && h->tiles_usable) ? h->tile_geom.nch : 0;
+    if (tile_span) *tile_span = h->tiles.valid ? h->tiles.smax : -1;
+    if (window_chunks) *window_chunks = (h->tiles.valid && h->tiles.usable) ? h->tiles.geom.nch : 0;
     return BFLK_OK;
 }
 
@@ -466,8 +462,17 @@ int bflk_kernel_time_ms(bflk_handle *h, float *das_ms, int32_t *das_launches, fl
 
 namespace bflk {
 
-int64_t min_stream_samples(const bflk_handle *h, int n_frames) {
+static int64_t min_stream_samples(const bflk_handle *h, int n_frames) {
     return (int64_t)(n_frames - 1) * h->cfg.frame_len + h->cfg.history + h->cfg.frame_len + 1;
+}
+
+int check_frames(bflk_handle *h, int64_t n_samples, int n_frames, const char *who) {
+    const int64_t need = min_stream_samples(h, n_frames);
+    if (n_samples < need)
+        return h->fail(BFLK_ERR_INVALID, "%s: %lld samples per channel cannot hold %d frames (need %lld)", who, (long long)n_samples, n_frames, (long long)need);
+    if (h->fir_phases > 0 && n_samples < need + h->fir_taps - 2)
+        return h->fail(BFLK_ERR_INVALID, "%s: the FIR reads %d samples past a frame's last tap", who, h->fir_taps - 2);
+    return BFLK_OK;
 }
 
 // 2x2 direction tiles of the handle's direction range (whole rows of the grid; the first is even)
@@ -477,23 +482,24 @@ static int tile_count(const bflk_handle *h) {
     return ((row1 - row0) / 2 + 1) * ((h->cols + 1) / 2);
 }
 
-// Builds (once per grid / mask / range) the packed tables of the register-tiled kernel.  tiles_valid is set only after
+// Builds (once per grid / mask / range) the packed tables of the register-tiled kernel.  tiles.valid is set only after
 // the last step has succeeded, so a failed build is retried (and reported again) by the next call.
-int ensure_tiles(bflk_handle *h, int fast, int want_warps) {
-    if (h->tiles_valid && h->tiles_fast == fast && h->tiles_want_warps == want_warps) return BFLK_OK;
+static int ensure_tiles(bflk_handle *h, int fast, int want_warps) {
+    bflk_handle::TileTables &t = h->tiles;
+    if (t.valid && t.fast == fast && t.want_warps == want_warps) return BFLK_OK;
     BFLK_CUDA(h, cudaEventSynchronize(h->caller_event));   // a queued kernel may still read the old tables
-    h->tiles_valid = false;
-    h->tiles_fast = fast;
-    h->tiles_want_warps = want_warps;
-    h->tiles_usable = false;
+    t.valid = false;
+    t.fast = fast;
+    t.want_warps = want_warps;
+    t.usable = false;
     if (h->rows <= 0 || h->cols <= 0) {  // caller-supplied LUT without a declared grid shape: nothing to tile
-        h->tiles_valid = true;
+        t.valid = true;
         return BFLK_OK;
     }
     const int cols = h->cols;
     const int n_tiles = tile_count(h);
     const int usable = (int)h->index.size();
-    BFLK_CUDA(h, h->d_tile_dirs.reserve((size_t)n_tiles * 4));
+    BFLK_CUDA(h, t.d_dirs.reserve((size_t)n_tiles * 4));
     BFLK_CUDA(h, h->d_misc.reserve(4));
     BFLK_CUDA(h, h->p_misc.reserve(4));
     const int stage_off = das_tile_geometry(h->cfg.history, h->max_delay, 0).stage_off;
@@ -519,39 +525,33 @@ int ensure_tiles(bflk_handle *h, int fast, int want_warps) {
     else if (span0 > 7 && pair_span <= 5) mode = pair_mode;   // two 7-chunk windows instead of one 10-chunk window
     const int forced = h->tuning.tile_mode;
     if (forced == 0 || ((forced == 1 || forced == 2) && h->p_misc.p[forced] <= 5)) mode = forced;
-    h->n_tiles = n_tiles;
-    h->tile_smax = h->p_misc.p[mode];
-    h->tile_geom = das_tile_geometry(h->cfg.history, h->max_delay, h->tile_smax, n_tiles, mode, fast, &h->tuning, want_warps);
+    t.n_tiles = n_tiles;
+    t.smax = h->p_misc.p[mode];
+    t.geom = das_tile_geometry(h->cfg.history, h->max_delay, t.smax, n_tiles, mode, fast, &h->tuning, want_warps);
     // usable: the spread fits a compiled variant, frames are whole blocks, AND the stage ring of some CTA shape fits
     // shared memory (packed rows grow with the largest delay: long arrays fall through to the other kernels)
-    h->tiles_usable = h->tile_smax <= das_tile_max_span() && h->cfg.frame_len >= 256 && h->cfg.frame_len % 2 == 0 &&
-                      h->tile_geom.stages >= 3;
-    if (!h->tiles_usable) {
-        h->tiles_valid = true;
+    t.usable = t.smax <= das_tile_max_span() && h->cfg.frame_len >= 256 && h->cfg.frame_len % 2 == 0 && t.geom.stages >= 3;
+    if (!t.usable) {
+        t.valid = true;
         return BFLK_OK;
     }
     // pass 2: the packed per-(tile, channel) entries, grouped for that variant's CTA shape
-    const size_t entries = tile_table_entries(n_tiles, usable, h->tile_geom.warps);
-    const size_t ent_bytes = das_tile_entry_bytes(h->tile_geom);
-    BFLK_CUDA(h, h->d_tiles.reserve(entries * ent_bytes));
-    BFLK_CUDA(h, cudaMemsetAsync(h->d_tiles.p, 0, entries * ent_bytes, h->stream));
+    const size_t entries = tile_table_entries(n_tiles, usable, t.geom.warps);
+    const size_t ent_bytes = das_tile_entry_bytes(t.geom);
+    BFLK_CUDA(h, t.d_tiles.reserve(entries * ent_bytes));
+    BFLK_CUDA(h, cudaMemsetAsync(t.d_tiles.p, 0, entries * ent_bytes, h->stream));
     BFLK_CUDA(h, launch_build_tiles(h->d_off.p, h->d_frac.p, h->cfg.n_channels, h->d_index.p, usable, h->rows, cols,
-                                    h->dir_first, h->dir_count, stage_off, h->tile_geom.copy_bytes, h->tile_geom.warps, mode,
-                                    2 * h->tile_geom.nch - 9, fast, h->d_tiles.p,
-                                    h->d_tile_dirs.p, n_tiles, h->d_misc.p, h->stream));
+                                    h->dir_first, h->dir_count, stage_off, t.geom.copy_bytes, t.geom.warps, mode,
+                                    2 * t.geom.nch - 9, fast, t.d_tiles.p, t.d_dirs.p, n_tiles, h->d_misc.p, h->stream));
     h->launches++;
     BFLK_CUDA(h, cudaStreamSynchronize(h->stream));
-    h->tiles_valid = true;
+    t.valid = true;
     return BFLK_OK;
 }
 
-}  // namespace bflk
-
-extern "C" {
-
 // Builds (once per grid / mask / range) the direction tiles and per-lane tables of the lane-broadcast kernel.
 static int ensure_bcast(bflk_handle *h) {
-    if (h->bcast_valid) return BFLK_OK;
+    if (h->bcast.valid) return BFLK_OK;
     BFLK_CUDA(h, cudaEventSynchronize(h->caller_event));   // a queued kernel may still read the old tables
     const int first = h->dir_first, count = h->dir_count;
     std::vector<int32_t> globals;
@@ -587,22 +587,22 @@ static int ensure_bcast(bflk_handle *h) {
     std::vector<int32_t> locals(globals.size());
     for (size_t i = 0; i < globals.size(); i++) locals[i] = globals[i] >= 0 ? globals[i] - first : -1;
     const int usable = (int)h->index.size();
-    h->bcast_geom = das_bcast_geometry(h->cfg.history, h->max_delay);
-    BFLK_CUDA(h, h->d_bcast_globals.reserve(globals.size()));
-    BFLK_CUDA(h, h->d_bcast_dirs.reserve(globals.size()));
-    BFLK_CUDA(h, h->d_bcast_table.reserve(das_bcast_table_entries(n_tiles, usable)));
-    BFLK_CUDA(h, cudaMemcpyAsync(h->d_bcast_globals.p, globals.data(), globals.size() * sizeof(int32_t), cudaMemcpyHostToDevice, h->stream));
-    BFLK_CUDA(h, cudaMemcpyAsync(h->d_bcast_dirs.p, locals.data(), locals.size() * sizeof(int32_t), cudaMemcpyHostToDevice, h->stream));
-    BFLK_CUDA(h, launch_bcast_table(h->d_off.p, h->d_frac.p, h->cfg.n_channels, h->d_index.p, usable, h->d_bcast_globals.p,
-                                    n_tiles, h->bcast_geom, h->d_bcast_table.p, h->stream));
+    h->bcast.geom = das_bcast_geometry(h->cfg.history, h->max_delay);
+    BFLK_CUDA(h, h->bcast.d_globals.reserve(globals.size()));
+    BFLK_CUDA(h, h->bcast.d_dirs.reserve(globals.size()));
+    BFLK_CUDA(h, h->bcast.d_table.reserve(das_bcast_table_entries(n_tiles, usable)));
+    BFLK_CUDA(h, cudaMemcpyAsync(h->bcast.d_globals.p, globals.data(), globals.size() * sizeof(int32_t), cudaMemcpyHostToDevice, h->stream));
+    BFLK_CUDA(h, cudaMemcpyAsync(h->bcast.d_dirs.p, locals.data(), locals.size() * sizeof(int32_t), cudaMemcpyHostToDevice, h->stream));
+    BFLK_CUDA(h, launch_bcast_table(h->d_off.p, h->d_frac.p, h->cfg.n_channels, h->d_index.p, usable, h->bcast.d_globals.p,
+                                    n_tiles, h->bcast.geom, h->bcast.d_table.p, h->stream));
     h->launches++;
     BFLK_CUDA(h, cudaStreamSynchronize(h->stream));  // the host vectors above go out of scope
-    h->bcast_tiles = n_tiles;
-    h->bcast_valid = true;
+    h->bcast.n_tiles = n_tiles;
+    h->bcast.valid = true;
     return BFLK_OK;
 }
 
-}  // extern "C"
+}  // namespace bflk
 
 // CTA shape of a call that cannot fill two waves of 16-warp CTAs (a live worker's single frame).  One CTA per SM (the stage
 // ring takes the shared memory), so the call takes waves x the time of one CTA = a fixed cost (launch, barrier set-up, first
@@ -638,9 +638,14 @@ void bflk::latency_shape(long long n_tiles, int n_frames, int frame_len, int usa
     if (*warps == 16 && *split == 1) *warps = 0;
 }
 
-int bflk::tiled_form(const bflk_handle *h) {
-    if (h->fir_phases > 0 || h->kernel_choice == 1 || h->kernel_choice == 3) return -1;
-    return h->kernel_choice != 2 ? 1 : 0;
+// *serve (serve may be null): the register-tiled kernels serve calls in the CTA shape of want_warps (0: throughput) from float
+// rows row_stride apart, or from wire rows (rows = nullptr).  Builds their tables for it unless FIR or kernel 1 / 3 rule them out.
+static int tiles_serve(bflk_handle *h, bool *serve, int want_warps = 0, const float *rows = nullptr, int64_t row_stride = 0) {
+    const bool form_ok = h->fir_phases == 0 && h->kernel_choice != kGeneric && h->kernel_choice != kBcast;
+    const int rc = form_ok ? ensure_tiles(h, h->kernel_choice != kTiledExact, want_warps) : BFLK_OK;
+    // the tiled kernels pack float rows with 8-byte loads: an even row stride from an 8-byte aligned start
+    if (serve) *serve = form_ok && rc == BFLK_OK && h->tiles.usable && (!rows || (!(row_stride & 1) && !((uintptr_t)rows & 7)));
+    return rc;
 }
 
 int bflk::note_use(bflk_handle *h, cudaStream_t st, bool overlapped) {
@@ -652,11 +657,8 @@ int bflk::note_use(bflk_handle *h, cudaStream_t st, bool overlapped) {
 
 int bflk::lanes_fork(bflk_handle *h, cudaEvent_t after, int only) {
     // tables first (ensure_tiles synchronises the handle's stream when it has to build them), before anything is queued
-    const int form = tiled_form(h);
-    if (form >= 0) {
-        int rc = ensure_tiles(h, form, 0);
-        if (rc) return rc;
-    }
+    int rc = tiles_serve(h, nullptr);
+    if (rc) return rc;
     const bool wait_caller = !(only >= 0 && h->caller_event_is_overlapped);
     for (int i = 0; i < 2; i++) {
         if (only >= 0 && i != only) continue;
@@ -675,15 +677,49 @@ int bflk::lanes_join(bflk_handle *h, int only) {
     return note_use(h, h->stream, only >= 0);
 }
 
+// route: the kernel of a call of n_frames frames from launch.wire or float rows (stream_dev, row_stride), the tiled kernels'
+// channel split (their warps are in the tables route builds), and whether wire samples go through ingest_kernel first.  A
+// chosen kernel that cannot serve the call is refused with BFLK_ERR_STATE.
+struct Route { Kernel kernel = kGeneric; int split = 1; bool ingest = false; };
+static int route(bflk_handle *h, const float *stream_dev, int64_t row_stride, int n_frames, const Launch &launch, Route *r) {
+    const int N = h->cfg.frame_len, usable = (int)h->index.size();
+    const bool fir = h->fir_phases > 0;   // FIR interpolation runs through the generic kernel only
+    if (fir && h->kernel_choice > kGeneric) return h->fail(BFLK_ERR_STATE, "bflk_power_map: FIR interpolation needs kernel 0 or 1");
+    // automatic choice = the two-FMA variant (power within the 1e-4 bar); 2 asks for bit-identical delayed sums
+    // a call with few block pairs cannot fill the SMs with 16-warp CTAs (one cfg3 frame: 16 CTAs, each walking 512
+    // channels with four warps per scheduler): smaller CTAs trade per-SM efficiency for latency.  The shape is part of
+    // the table layout, so a handle that alternates between single frames and large batches rebuilds its tables.
+    int want_warps = 0, want_split = 1;
+    if (h->rows > 0 && h->cols > 0 && h->tuning.tile_warps == 0)
+        latency_shape(tile_count(h), n_frames, N, usable, block_pairs_per_cta(h->tuning.tile_pairs, usable), h->sm_count,
+                      h->kernel_choice != kTiledExact && h->allow_ksplit && !h->tuning.no_ksplit, &want_warps, &want_split);
+    if (want_warps > 0 && h->tuning.lat_warps >= 2 && h->tuning.lat_warps <= 16) want_warps = h->tuning.lat_warps;   // experiments
+    if (want_warps > 0 && h->tuning.lat_split >= 1 && h->allow_ksplit) want_split = h->tuning.lat_split;
+    if (launch.pipelined) { want_warps = 0; want_split = 1; }   // lanes_fork built the throughput-shape tables
+    bool tiled;
+    int rc = tiles_serve(h, &tiled, want_warps, launch.wire ? nullptr : stream_dev, row_stride);
+    if (rc) return rc;
+    if ((h->kernel_choice == kTiledExact || h->kernel_choice == kTiledFma2) && !tiled)
+        return h->fail(BFLK_ERR_STATE, "bflk_power_map: the register-tiled kernel does not fit this grid (offset spread %d of at most %d, %d stage buffers fit shared memory)",
+                       h->tiles.smax, das_tile_max_span(), h->tiles.geom.stages);
+    const bool bcast_ok = N >= 256 && das_bcast_fits(das_bcast_geometry(h->cfg.history, h->max_delay));
+    if (h->kernel_choice == kBcast && !bcast_ok)
+        return h->fail(BFLK_ERR_STATE, "bflk_power_map: the lane-broadcast kernel needs frame_len >= 256 and a stage ring that fits shared memory");
+    r->split = tiled && das_tile_ksplit_ok(h->tiles.geom, want_split) ? want_split : 1;
+    r->ingest = launch.wire && !tiled;
+    if (tiled) r->kernel = h->tiles.geom.fast ? kTiledFma2 : kTiledExact;
+    else if (!fir && (h->kernel_choice == kAuto || h->kernel_choice == kBcast) && bcast_ok) r->kernel = kBcast;
+    return r->kernel == kBcast ? ensure_bcast(h) : BFLK_OK;
+}
+
 int bflk::power_map_dev(bflk_handle *h, const float *stream_dev, int64_t row_stride, int64_t n_samples, int32_t n_frames,
                         float *power_dev, const Launch &launch, float *beams_dev) {
     if (!h) return BFLK_ERR_INVALID;
     if (!h->have_grid) return h->fail(BFLK_ERR_STATE, "bflk_power_map: set geometry and grid first");
     const int32_t *wire = launch.wire;   // wire-format call: stream_dev is null, the samples are wire[n_samples][C]
     if ((!stream_dev && !wire) || !power_dev || n_frames <= 0) return h->fail(BFLK_ERR_INVALID, "bflk_power_map: null buffer or no frames");
-    if (n_samples < min_stream_samples(h, n_frames))
-        return h->fail(BFLK_ERR_INVALID, "bflk_power_map: %lld samples per channel cannot hold %d frames (need %lld)",
-                       (long long)n_samples, n_frames, (long long)min_stream_samples(h, n_frames));
+    int rc = check_frames(h, n_samples, n_frames, "bflk_power_map");
+    if (rc) return rc;
     BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
     cudaStream_t st = launch.st ? launch.st : h->stream;
     // the packed rows, partial sums and tables are the handle's: a call on another stream than the previous one waits for it
@@ -700,46 +736,17 @@ int bflk::power_map_dev(bflk_handle *h, const float *stream_dev, int64_t row_str
     const float norm = static_cast<float>(N * usable);  // power /= float(N_SAMPLES * count), mimo.cpp:137
     // automatic choice: register-tiled kernel when the grid tiles (2x2 direction tiles with small offset
     // spread), else the lane-broadcast kernel (any direction list), else the generic kernel (any frame length)
-    bool tiled = false;
-    const bool fir = h->fir_phases > 0;   // FIR interpolation runs through the generic kernel only
-    if (fir && h->kernel_choice > 1) return h->fail(BFLK_ERR_STATE, "bflk_power_map: FIR interpolation needs kernel 0 or 1");
-    if (fir && n_samples < min_stream_samples(h, n_frames) + h->fir_taps - 2)
-        return h->fail(BFLK_ERR_INVALID, "bflk_power_map: the FIR reads %d samples past a frame's last tap", h->fir_taps - 2);
-    const int form = tiled_form(h);
-    if (form >= 0) {
-        // automatic choice = the two-FMA variant (power within the 1e-4 bar); 2 asks for bit-identical delayed sums
-        // a call with few block pairs cannot fill the SMs with 16-warp CTAs (one cfg3 frame: 16 CTAs, each walking 512
-        // channels with four warps per scheduler): smaller CTAs trade per-SM efficiency for latency.  The shape is part of
-        // the table layout, so a handle that alternates between single frames and large batches rebuilds its tables.
-        int want_warps = 0, want_split = 1;
-        if (h->rows > 0 && h->cols > 0 && h->tuning.tile_warps == 0)
-            latency_shape(tile_count(h), n_frames, N, usable, block_pairs_per_cta(h->tuning.tile_pairs, usable), h->sm_count,
-                          h->kernel_choice != 2 && h->allow_ksplit && !h->tuning.no_ksplit, &want_warps, &want_split);
-        if (want_warps > 0 && h->tuning.lat_warps >= 2 && h->tuning.lat_warps <= 16) want_warps = h->tuning.lat_warps;   // experiments
-        if (want_warps > 0 && h->tuning.lat_split >= 1 && h->allow_ksplit) want_split = h->tuning.lat_split;
-        if (launch.pipelined) { want_warps = 0; want_split = 1; }   // lanes_fork built the throughput-shape tables
-        int rc = ensure_tiles(h, form, want_warps);
-        if (rc) return rc;
-        h->tile_geom.ksplit = das_tile_ksplit_ok(h->tile_geom, want_split) ? want_split : 1;
-        tiled = h->tiles_usable && (wire || (!(row_stride & 1) && !((uintptr_t)stream_dev & 7)));  // packed rows: 8-byte loads
-        if (h->kernel_choice != 0 && !tiled)
-            return h->fail(BFLK_ERR_STATE, "bflk_power_map: the register-tiled kernel does not fit this grid (offset spread %d of at most %d, %d stage buffers fit shared memory)",
-                           h->tile_smax, das_tile_max_span(), h->tile_geom.stages);
-    }
-    if (wire && !tiled) {
+    Route r;
+    if ((rc = route(h, stream_dev, row_stride, n_frames, launch, &r))) return rc;
+    if (r.ingest) {
         // the other kernels read channel-major float rows: convert the wire samples first (ingest_kernel), then carry on
         BFLK_CUDA(h, h->d_window.reserve((size_t)C * (n_samples + 1)));
         BFLK_CUDA(h, launch_ingest(wire, n_samples, C, h->d_window.p, st));
         h->launches++;
         stream_dev = h->d_window.p;
         row_stride = n_samples;
-        wire = nullptr;
     }
-    const bool bcast_ok = N >= 256 && das_bcast_fits(das_bcast_geometry(h->cfg.history, h->max_delay));
-    if (h->kernel_choice == 3 && !bcast_ok)
-        return h->fail(BFLK_ERR_STATE, "bflk_power_map: the lane-broadcast kernel needs frame_len >= 256 and a stage ring that fits shared memory");
-    const bool bcast = !fir && !tiled && (h->kernel_choice == 0 || h->kernel_choice == 3) && bcast_ok;
-    if (!tiled && !bcast) {
+    if (r.kernel == kGeneric) {
         GenericArgs a{};
         a.stream = stream_dev;
         a.row_stride = row_stride;
@@ -755,19 +762,15 @@ int bflk::power_map_dev(bflk_handle *h, const float *stream_dev, int64_t row_str
         a.power = power_dev;
         a.audio = beams_dev;
         a.norm = norm;
-        if (fir) { a.fir = h->d_fir.p; a.fir_phases = h->fir_phases; a.fir_taps = h->fir_taps; }
+        if (h->fir_phases > 0) { a.fir = h->d_fir.p; a.fir_phases = h->fir_phases; a.fir_taps = h->fir_taps; }
         timing_hook(h, 0, true, st);
         BFLK_CUDA(h, launch_das_generic(a, st));
         timing_hook(h, 0, false, st);
         h->launches++;
-        h->kernel_last = 1;
+        h->kernel_last = r.kernel;
         return BFLK_OK;
     }
     // the staged kernels: pack pre-pass, delay-and-sum, and for frames longer than one block finalize_kernel
-    if (bcast) {
-        int rc = ensure_bcast(h);
-        if (rc) return rc;
-    }
     FrameArgs f;
     f.stream = stream_dev;
     f.row_stride = row_stride;
@@ -781,35 +784,35 @@ int bflk::power_map_dev(bflk_handle *h, const float *stream_dev, int64_t row_str
     f.power = power_dev;
     f.beams = beams_dev;
     f.norm = norm;
-    BFLK_CUDA(h, d_packed.reserve(packed_bytes(f, tiled ? h->tile_geom.row_bytes : h->bcast_geom.row_bytes)));
+    BFLK_CUDA(h, d_packed.reserve(packed_bytes(f, r.kernel == kBcast ? h->bcast.geom.row_bytes : h->tiles.geom.row_bytes)));
     f.packed = d_packed.p;
     if (blocks_per_frame(N) > 1) {
         BFLK_CUDA(h, d_partial.reserve((size_t)n_frames * blocks_per_frame(N) * h->dir_count));
         f.partial = d_partial.p;
     }
     int launches = 0;
-    if (tiled) {
+    if (r.kernel != kBcast) {
         TileArgs a;
         a.f = f;
         a.wire = wire;
         a.wire_cols = C;
-        a.tiles = h->d_tiles.p;
-        a.tile_dirs = h->d_tile_dirs.p;
-        a.n_tiles = h->n_tiles;
-        a.geom = h->tile_geom;
+        a.tiles = h->tiles.d_tiles.p;
+        a.tile_dirs = h->tiles.d_dirs.p;
+        a.n_tiles = h->tiles.n_tiles;
+        a.geom = h->tiles.geom;
+        a.geom.ksplit = r.split;
         BFLK_CUDA(h, launch_das_tile(a, h->sm_count, st, &launches, timing_hook, h));
-        h->kernel_last = h->tile_geom.fast ? 4 : 2;
     } else {
         BcastArgs a;
         a.f = f;
-        a.table = h->d_bcast_table.p;
-        a.tile_dirs = h->d_bcast_dirs.p;
-        a.n_tiles = h->bcast_tiles;
-        a.geom = h->bcast_geom;
+        a.table = h->bcast.d_table.p;
+        a.tile_dirs = h->bcast.d_dirs.p;
+        a.n_tiles = h->bcast.n_tiles;
+        a.geom = h->bcast.geom;
         BFLK_CUDA(h, launch_das_bcast(a, st, &launches, timing_hook, h));
-        h->kernel_last = 3;
     }
     h->launches += launches;
+    h->kernel_last = r.kernel;
     return BFLK_OK;
 }
 
@@ -818,20 +821,16 @@ int bflk::power_map_dev_overlapped(bflk_handle *h, const float *stream_dev, int6
     *used = caller;
     if (!h->have_grid) return h->fail(BFLK_ERR_STATE, "bflk_power_map: set geometry and grid first");
     BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
-    const int form = tiled_form(h);
-    if (form >= 0) {
-        int rc = ensure_tiles(h, form, 0);
-        if (rc) return rc;
-    }
-    if (form < 0 || !h->tiles_usable || (row_stride & 1) || ((uintptr_t)stream_dev & 7))
-        return power_map_dev(h, stream_dev, row_stride, n_samples, n_frames, power_dev, Launch{caller});
+    bool tiled;
+    int rc = tiles_serve(h, &tiled, 0, stream_dev, row_stride);
+    if (rc) return rc;
+    if (!tiled) return power_map_dev(h, stream_dev, row_stride, n_samples, n_frames, power_dev, Launch{caller});
     const int slot = (int)(h->dev_seq++ & 1);
     // this batch's kernels wait for (a) the caller's stream having reached this call (its inputs), (b) whatever used the handle's
     // scratch on another stream before the overlapped batches began.  Earlier overlapped batches need no wait: the same
     // set's previous batch ran on this very lane, the other set's batch shares nothing with this one.
     BFLK_CUDA(h, cudaEventRecord(h->dev_in[slot], caller));
-    int rc = lanes_fork(h, h->dev_in[slot], slot);
-    if (rc) return rc;
+    if ((rc = lanes_fork(h, h->dev_in[slot], slot))) return rc;
     if ((rc = power_map_dev(h, stream_dev, row_stride, n_samples, n_frames, power_dev, Launch{h->lane[slot], slot, true})))
         return rc;
     // the handle's own stream collects the ends of all overlapped batches: caller_event then covers everything enqueued so far
@@ -889,13 +888,13 @@ int host_chunk_frames(bflk_handle *h, int n_frames, int *chunk_frames_out) {
     const int64_t frame_bytes = (int64_t)C * N * sizeof(float);
     int n_chunks = (int)std::max<int64_t>(1, ((int64_t)n_frames * frame_bytes + chunk_bytes / 2) / chunk_bytes);
     int chunk_frames = (n_frames + n_chunks - 1) / n_chunks;  // even split
-    const int form = tiled_form(h);
-    if (n_chunks > 1 && N == 256 && form >= 0 && h->sm_count > 0) {
+    if (n_chunks > 1 && N == 256 && h->sm_count > 0) {
         // the tiled kernel runs one CTA per (tile group, block pair): round the chunk to a whole number of CTA waves
-        int rc = ensure_tiles(h, form);
+        bool tiled;
+        int rc = tiles_serve(h, &tiled);
         if (rc) return rc;
-        if (h->tiles_usable) {
-            const int ctas_per_pair = (h->n_tiles + h->tile_geom.warps - 1) / h->tile_geom.warps;
+        if (tiled) {
+            const int ctas_per_pair = (h->tiles.n_tiles + h->tiles.geom.warps - 1) / h->tiles.geom.warps;
             int g = h->sm_count, b = ctas_per_pair;
             while (b) { const int t = g % b; g = b; b = t; }          // gcd
             const int quantum = 2 * (h->sm_count / g);                // frames per whole wave set
@@ -1014,10 +1013,7 @@ static int host_batch_enqueue(bflk_handle *h, const float *stream, int64_t n_sam
 static int host_batch_check(bflk_handle *h, const float *stream, int64_t n_samples, int32_t n_frames, const float *power_out) {
     if (!h->have_grid) return h->fail(BFLK_ERR_STATE, "bflk_power_map: set geometry and grid first");
     if (!stream || !power_out || n_frames <= 0 || n_samples <= 0) return h->fail(BFLK_ERR_INVALID, "bflk_power_map: null buffer or no frames");
-    if (n_samples < min_stream_samples(h, n_frames))
-        return h->fail(BFLK_ERR_INVALID, "bflk_power_map: %lld samples per channel cannot hold %d frames (need %lld)",
-                       (long long)n_samples, n_frames, (long long)min_stream_samples(h, n_frames));
-    return BFLK_OK;
+    return check_frames(h, n_samples, n_frames, "bflk_power_map");
 }
 
 int bflk_power_map_batch_wait(bflk_handle *h) {
@@ -1086,11 +1082,9 @@ int bflk_power_map_batch_i32(bflk_handle *h, const int32_t *frames, int64_t n_sa
     if (!h) return BFLK_ERR_INVALID;
     if (!h->have_grid) return h->fail(BFLK_ERR_STATE, "bflk_power_map_batch_i32: set geometry and grid first");
     if (!frames || !power_out || n_frames <= 0) return h->fail(BFLK_ERR_INVALID, "bflk_power_map_batch_i32: null buffer or no frames");
-    if (n_samples < min_stream_samples(h, n_frames))
-        return h->fail(BFLK_ERR_INVALID, "bflk_power_map_batch_i32: %lld samples cannot hold %d frames (need %lld)",
-                       (long long)n_samples, n_frames, (long long)min_stream_samples(h, n_frames));
-    int rc = wire_check(h, n_samples);
+    int rc = check_frames(h, n_samples, n_frames, "bflk_power_map_batch_i32");
     if (rc) return rc;
+    if ((rc = wire_check(h, n_samples))) return rc;
     BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
     const int C = h->cfg.n_channels, N = h->cfg.frame_len;
     BFLK_CUDA(h, h->d_wire.reserve((size_t)C * n_samples));
@@ -1104,11 +1098,7 @@ int bflk_power_map_batch_i32(bflk_handle *h, const int32_t *frames, int64_t n_sa
     in.last = n_samples;
     // two lanes only when the register-tiled kernel takes the wire samples directly: the other kernels convert them into
     // the handle's one float window first (ingest_kernel)
-    const int form = tiled_form(h);
-    if (chunk_frames < n_frames && form >= 0) {
-        if ((rc = ensure_tiles(h, form, 0))) return rc;
-        in.lanes = h->tiles_usable;
-    }
+    if (chunk_frames < n_frames && (rc = tiles_serve(h, &in.lanes))) return rc;
     int32_t *dev = h->d_wire.p;
     in.upload = [=](int64_t t0, int64_t t1, cudaStream_t st) {
         return cudaMemcpyAsync(dev + (size_t)t0 * C, frames + (size_t)t0 * C, (size_t)(t1 - t0) * C * sizeof(int32_t),

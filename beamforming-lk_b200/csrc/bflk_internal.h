@@ -103,6 +103,8 @@ struct TileGeometry {
     int ksplit = 1;      // 2 / 4: a thread-block cluster of that size splits the channels of a block pair (small calls, two-FMA form)
 };
 
+enum Kernel : int32_t { kAuto = 0, kGeneric = 1, kTiledExact = 2, kBcast = 3, kTiledFma2 = 4 };   // as in bflk_set_kernel
+
 // ---- lane-broadcast kernel (das_bcast.cu) -----------------------------------------------------------------
 constexpr int kBcastCC = 8;  // channels per pipeline stage
 struct BcastEntry {
@@ -207,8 +209,8 @@ struct bflk_handle {
     int sm_count = 0;
     std::string error;
     int64_t launches = 0;
-    int kernel_choice = 0;  // 0 auto, 1 generic, 2 tiled
-    int kernel_last = 0;    // what the last power-map call ran
+    bflk::Kernel kernel_choice = bflk::kAuto;
+    bflk::Kernel kernel_last = bflk::kAuto;   // what the last power-map call ran (kAuto: none yet)
     bool allow_ksplit = false;  // bflk_set_channel_split: small two-FMA calls may split the channels across a thread-block cluster
 
     // geometry + mask (host copies are the source of truth; device copies feed the table kernels)
@@ -229,23 +231,28 @@ struct bflk_handle {
     bflk::DevBuf<float> d_frac;   // [D][C]
 
     // register-tiled kernel tables (built lazily for the current grid / mask / range)
-    bool tiles_valid = false;
-    bool tiles_usable = false;   // false: grid shape / spreads do not fit the tiled kernel
-    int tiles_fast = 0;          // the tables were built for the two-FMA variant
-    int tiles_want_warps = 0;    // ... and for this CTA shape (0: throughput shape; 2..15: latency shape of small calls, latency_warps())
-    int32_t n_tiles = 0;
-    int32_t tile_smax = 0;       // compiled window slack the tables need
-    bflk::DevBuf<char> d_tiles;             // tile_table_entries(n_tiles, usable) TileEntry / TileEntryFast, layout above
-    bflk::DevBuf<int32_t> d_tile_dirs;      // [n_tiles][4] local direction index (or -1)
-    bflk::TileGeometry tile_geom;
+    struct TileTables {
+        bool valid = false;
+        bool usable = false;   // false: grid shape / spreads do not fit the tiled kernel
+        int fast = 0;          // the tables were built for the two-FMA variant
+        int want_warps = 0;    // ... and for this CTA shape (0: throughput shape; 2..15: latency shape of small calls, latency_warps())
+        int32_t n_tiles = 0;
+        int32_t smax = 0;      // compiled window slack the tables need
+        bflk::DevBuf<char> d_tiles;        // tile_table_entries(n_tiles, usable) TileEntry / TileEntryFast, layout above
+        bflk::DevBuf<int32_t> d_dirs;      // [n_tiles][4] local direction index (or -1)
+        bflk::TileGeometry geom;
+    } tiles;
 
     // lane-broadcast kernel tables (built lazily for the current grid / mask / range)
-    bool bcast_valid = false;
-    int32_t bcast_tiles = 0;
-    bflk::BcastGeometry bcast_geom;
-    bflk::DevBuf<bflk::BcastEntry> d_bcast_table;  // [tile][stage][kBcastCC][32]
-    bflk::DevBuf<int32_t> d_bcast_dirs;            // [tile][32] local direction index or -1
-    bflk::DevBuf<int32_t> d_bcast_globals;         // [tile][32] grid direction index or -1
+    struct BcastTables {
+        bool valid = false;
+        int32_t n_tiles = 0;
+        bflk::BcastGeometry geom;
+        bflk::DevBuf<bflk::BcastEntry> d_table;  // [tile][stage][kBcastCC][32]
+        bflk::DevBuf<int32_t> d_dirs;            // [tile][32] local direction index or -1
+        bflk::DevBuf<int32_t> d_globals;         // [tile][32] grid direction index or -1
+    } bcast;
+    void drop_kernel_tables() { tiles.valid = bcast.valid = false; }   // every change of grid, mask or direction range
 
     // optional FIR interpolation (bflk_set_fir): coefficient table on the device
     bflk::DevBuf<float> d_fir;
@@ -498,13 +505,11 @@ int note_use(bflk_handle *h, cudaStream_t st, bool overlapped);
 // device batch), which skips caller_event when it covers overlapped batches only (the lane's own are in its stream order).
 int lanes_fork(bflk_handle *h, cudaEvent_t after, int only = -1);
 int lanes_join(bflk_handle *h, int only = -1);
-// -1 when the register-tiled kernels cannot serve a call (FIR, or kernel 1 / 3), else the `fast` flag for ensure_tiles
-int tiled_form(const bflk_handle *h);
-int ensure_tiles(bflk_handle *h, int fast, int want_warps = 0);
 // CTA shape of a tiled call over n_tiles direction tiles and n_frames frames: warps = 0 (throughput shape) or 2..16
 void latency_shape(long long n_tiles, int n_frames, int frame_len, int usable, int pairs_per_cta, int sms, bool may_split,
                    int *warps, int *split);
-int64_t min_stream_samples(const bflk_handle *h, int n_frames);
+// BFLK_ERR_INVALID (reported as who's) unless n_samples per channel hold n_frames frames and what the FIR reads past them
+int check_frames(bflk_handle *h, int64_t n_samples, int n_frames, const char *who);
 // frames per chunk of a host batch of n_frames (whole CTA waves of the tiled kernel where it applies) and the samples a
 // frame needs beyond its own N
 int host_chunk_frames(bflk_handle *h, int n_frames, int *chunk_frames);

@@ -289,8 +289,7 @@ int sharded_dev(const std::vector<bflk_handle *> &hs, const std::vector<const fl
         int rc = check_sharded(h, "bflk_power_map_batch_sharded_dev");
         if (rc) return rc;
         if (!stream_dev[i] || !power_all_dev[i] || n_frames <= 0) return h->fail(BFLK_ERR_INVALID, "bflk_power_map_batch_sharded_dev: null buffer or no frames");
-        if (n_samples < min_stream_samples(h, n_frames))
-            return h->fail(BFLK_ERR_INVALID, "bflk_power_map_batch_sharded_dev: %lld samples per channel cannot hold %d frames", (long long)n_samples, n_frames);
+        if ((rc = check_frames(h, n_samples, n_frames, "bflk_power_map_batch_sharded_dev"))) return rc;
         BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
         bflk_comm *c = h->comm;
         if (pipelined) {
@@ -384,8 +383,7 @@ int sharded_host(const std::vector<bflk_handle *> &hs, const float *stream, int6
         int rc = check_sharded(h, "bflk_power_map_batch_sharded");
         if (rc) return rc;
         if (!stream || n_frames <= 0) return h->fail(BFLK_ERR_INVALID, "bflk_power_map_batch_sharded: null buffer or no frames");
-        if (n_samples < min_stream_samples(h, n_frames))
-            return h->fail(BFLK_ERR_INVALID, "bflk_power_map_batch_sharded: %lld samples per channel cannot hold %d frames", (long long)n_samples, n_frames);
+        if ((rc = check_frames(h, n_samples, n_frames, "bflk_power_map_batch_sharded"))) return rc;
         BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
         bflk_comm *c = h->comm;
         sets[i] = &c->sets[0];
