@@ -32,9 +32,9 @@ SYMBOLS = [
     "bflk_power_map_batch", "bflk_power_map_batch_submit", "bflk_power_map_batch_wait", "bflk_power_map_batch_i32", "bflk_power_map_batch_i32_dev",
     "bflk_power_map_batch_dev", "bflk_beams_batch_dev", "bflk_power_map_batch_dev_submit", "bflk_power_map_batch_dev_join", "bflk_set_kernel", "bflk_set_channel_split", "bflk_launch_shape", "bflk_get_kernel", "bflk_launch_count", "bflk_enable_timing",
     "bflk_kernel_time_ms", "bflk_fp32_peak_tflops", "bflk_set_window", "bflk_set_window_dev", "bflk_miso", "bflk_miso_dev", "bflk_monopulse", "bflk_set_fir",
-    "bflk_pin_host", "bflk_unpin_host", "bflk_heatmap", "bflk_resize_u8", "bflk_targets", "bflk_calibrate", "bflk_ingest_i32",
+    "bflk_pin_host", "bflk_unpin_host", "bflk_heatmap", "bflk_resize_u8", "bflk_targets", "bflk_targets_batch_dev", "bflk_calibrate", "bflk_ingest_i32",
     "bflk_stream_open", "bflk_stream_close", "bflk_stream_push", "bflk_stream_push_i32", "bflk_stream_power_maps",
-    "bflk_stream_discard", "bflk_stream_status", "bflk_stream_window", "bflk_session_beams",
+    "bflk_stream_discard", "bflk_stream_status", "bflk_stream_window", "bflk_session_beams", "bflk_session_targets",
     "bflk_comm_unique_id", "bflk_comm_init_rank", "bflk_comm_info", "bflk_shard_plan",
     "bflk_power_map_batch_sharded_dev", "bflk_power_map_batch_sharded_dev_submit", "bflk_power_map_batch_sharded_dev_join", "bflk_power_map_batch_sharded", "bflk_power_map_batch_sharded_submit", "bflk_power_map_batch_sharded_wait",
     "bflk_group_create", "bflk_group_destroy", "bflk_group_size", "bflk_group_handle", "bflk_group_last_error",
@@ -53,6 +53,22 @@ class Target(C.Structure):
     """struct bflk_target (Target of src/dsp/worker.h:32-61 for a peak of the MIMO map)."""
     _fields_ = [("theta", C.c_double), ("phi", C.c_double), ("power", C.c_float), ("probability", C.c_float),
                 ("direction", C.c_int32), ("row", C.c_int32), ("col", C.c_int32), ("reserved", C.c_int32)]
+
+
+# the same 40-byte record as a numpy dtype: decodes targets copied back from a device buffer (Beamformer.targets_batch_dev)
+TARGET_DTYPE = np.dtype([("theta", np.float64), ("phi", np.float64), ("power", np.float32), ("probability", np.float32),
+                         ("direction", np.int32), ("row", np.int32), ("col", np.int32), ("reserved", np.int32)])
+assert TARGET_DTYPE.itemsize == C.sizeof(Target)
+
+
+def decode_targets(raw, counts):
+    """Records of a [n_maps][max_targets] buffer of bflk_target (raw bytes or a uint8 / TARGET_DTYPE array of that size) and
+    counts [n_maps] -> one list of target dicts per map, as Beamformer.targets returns them."""
+    counts = np.asarray(counts).ravel()
+    rec = np.frombuffer(np.ascontiguousarray(raw).tobytes() if not isinstance(raw, bytes) else raw, TARGET_DTYPE)
+    rec = rec.reshape(counts.shape[0], -1)
+    keys = ("theta", "phi", "power", "probability", "direction", "row", "col")
+    return [[{k: t[k].item() for k in keys} for t in rec[b, :counts[b]]] for b in range(counts.shape[0])]
 
 
 class BflkError(RuntimeError):
@@ -124,6 +140,7 @@ def load_library():
     L.bflk_unpin_host.argtypes = [vp]
     L.bflk_resize_u8.argtypes = [vp, vp, i32, i32, i32, i32, vp]
     L.bflk_targets.argtypes = [vp, vp, i32, f32, vp, C.POINTER(i32)]
+    L.bflk_targets_batch_dev.argtypes = [vp, vp, i32, i32, f32, vp, vp, vp]
     L.bflk_calibrate.argtypes = [vp, vp, i32, f32, vp, vp, C.POINTER(i32), C.POINTER(f32), C.POINTER(f32)]
     L.bflk_ingest_i32.argtypes = [vp, vp, i32, i32, vp]
     L.bflk_stream_open.argtypes = [vp, i32]
@@ -132,6 +149,7 @@ def load_library():
     L.bflk_stream_push_i32.argtypes = [vp, vp, i32]
     L.bflk_stream_power_maps.argtypes = [vp, i32, vp, C.POINTER(i64), C.POINTER(i32)]
     L.bflk_session_beams.argtypes = [vp, i32, vp, vp, C.POINTER(i64), C.POINTER(i32)]
+    L.bflk_session_targets.argtypes = [vp, i32, i32, f32, vp, vp, vp, C.POINTER(i64), C.POINTER(i32)]
     L.bflk_stream_discard.argtypes = [vp, i32]
     L.bflk_stream_status.argtypes = [vp, C.POINTER(i64), C.POINTER(i64), C.POINTER(i32), C.POINTER(i64)]
     L.bflk_stream_window.argtypes = [vp, i64]
@@ -527,6 +545,18 @@ class Beamformer:
         self._check(self._L.bflk_session_beams(self._h, max_frames, _ptr(beams), _ptr(out), C.byref(first), C.byref(n)))
         return first.value, beams[:n.value].copy(), out[:n.value].copy()
 
+    def stream_targets(self, max_frames=1, max_targets=8, min_rel_power=0.5):
+        """stream_power_maps with the Targets of every map: (first_frame, power [n][count], [list of target dicts per frame]),
+        n may be 0."""
+        count = self.n_directions()[2]
+        out = np.zeros((max_frames, count), np.float32)
+        recs = (Target * (max_frames * max_targets))()
+        counts = np.zeros(max_frames, np.int32)
+        first, n = C.c_int64(), C.c_int32()
+        self._check(self._L.bflk_session_targets(self._h, max_frames, max_targets, float(min_rel_power), _ptr(out), recs,
+                                                 _ptr(counts), C.byref(first), C.byref(n)))
+        return first.value, out[:n.value].copy(), decode_targets(bytes(recs), counts)[:n.value]
+
     def stream_discard(self, keep=0):
         """Skip every ready frame but the newest `keep`."""
         self._check(self._L.bflk_stream_discard(self._h, keep))
@@ -565,6 +595,14 @@ class Beamformer:
         self._check(self._L.bflk_targets(self._h, _ptr(power) if power is not None else None, max_targets, float(min_rel_power), arr, C.byref(n)))
         return [dict(theta=t.theta, phi=t.phi, power=t.power, probability=t.probability, direction=t.direction, row=t.row, col=t.col)
                 for t in arr[:n.value]]
+
+    def targets_batch_dev(self, power_dev_ptr, n_maps, targets_dev_ptr, n_dev_ptr, max_targets=8, min_rel_power=0.5,
+                          cuda_stream=0):
+        """Targets of n_maps whole-grid maps [n_maps][D] on the device, one launch, asynchronous on cuda_stream:
+        targets_dev [n_maps][max_targets] bflk_target records (40 bytes each; decode_targets / TARGET_DTYPE read them back),
+        n_dev [n_maps] int32 counts."""
+        self._check(self._L.bflk_targets_batch_dev(self._h, C.c_void_p(power_dev_ptr), n_maps, max_targets, float(min_rel_power),
+                                                   C.c_void_p(targets_dev_ptr), C.c_void_p(n_dev_ptr), C.c_void_p(cuda_stream)))
 
     def calibrate(self, signals, reference_power_level=1e-5):
         signals = _np(signals, np.float32)

@@ -247,6 +247,13 @@ int bflk_set_grid_fov(bflk_handle *h, int32_t rows, int32_t cols, float fov_deg)
     if (rc) return rc;
     invalidate_tables(h);
     if ((rc = check_delay_range(h, max_delay, "bflk_set_grid_fov"))) return rc;
+    // the angles of the Targets records, on the device
+    BFLK_CUDA(h, cudaEventSynchronize(h->caller_event));   // a caller's stream may still read the old ones
+    BFLK_CUDA(h, h->d_theta.reserve(D));
+    BFLK_CUDA(h, h->d_phi.reserve(D));
+    BFLK_CUDA(h, cudaMemcpyAsync(h->d_theta.p, theta.data(), D * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    BFLK_CUDA(h, cudaMemcpyAsync(h->d_phi.p, phi.data(), D * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    BFLK_CUDA(h, cudaStreamSynchronize(h->stream));
     h->theta.swap(theta);
     h->phi.swap(phi);
     h->rows = rows;
@@ -283,7 +290,7 @@ int bflk_set_grid_tables(bflk_handle *h, const int32_t *offsets, const float *fr
         return h->fail(BFLK_ERR_RANGE, "bflk_set_grid_tables: offsets must lie in [0, history = %d]; got [%d, %d]",
                        h->cfg.history, min_off, max_off);
     const int max_delay = h->cfg.history - min_off;
-    h->theta.clear();
+    h->theta.clear();   // no angles: the Targets calls refuse these tables
     h->phi.clear();
     h->rows = h->cols = 0;
     h->n_dir = n_directions;
@@ -1398,6 +1405,51 @@ int bflk_monopulse(bflk_handle *h, double *theta, const double *phi, int32_t n_p
     return BFLK_OK;
 }
 
+// ---- Targets of the maps ------------------------------------------------------------------------------------------
+// Targets carry the grid's angles: they need a bflk_set_grid_fov grid (caller tables have none, with or without a shape).
+static bool fov_grid(const bflk_handle *h) { return h->have_grid && h->rows > 0 && h->cols > 0 && !h->theta.empty(); }
+
+// Targets of k whole-grid maps d_maps[k][D] on the handle's stream, synchronously: out[k][max_targets] (records past a map's
+// count are not written) and counts[k] on the host.  Work the caller enqueued on the handle's stream before is done too.
+static int host_targets(bflk_handle *h, const float *d_maps, int k, int max_targets, float min_rel, bflk_target *out,
+                        int32_t *counts) {
+    const size_t n_rec = (size_t)k * max_targets;
+    BFLK_CUDA(h, h->d_targets.reserve(n_rec));
+    BFLK_CUDA(h, h->d_target_counts.reserve(k));
+    BFLK_CUDA(h, h->p_targets.reserve(n_rec));
+    BFLK_CUDA(h, h->p_target_counts.reserve(k));
+    BFLK_CUDA(h, launch_map_targets(d_maps, k, h->rows, h->cols, max_targets, min_rel, h->d_theta.p, h->d_phi.p,
+                                    h->d_targets.p, h->d_target_counts.p, h->sm_count, h->stream));
+    h->launches++;
+    BFLK_CUDA(h, cudaMemcpyAsync(h->p_targets.p, h->d_targets.p, n_rec * sizeof(bflk_target), cudaMemcpyDeviceToHost, h->stream));
+    BFLK_CUDA(h, cudaMemcpyAsync(h->p_target_counts.p, h->d_target_counts.p, k * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+    BFLK_CUDA(h, cudaStreamSynchronize(h->stream));
+    for (int b = 0; b < k; b++) {
+        const int32_t n = h->p_target_counts.p[b];
+        std::memcpy(out + (size_t)b * max_targets, h->p_targets.p + (size_t)b * max_targets, n * sizeof(bflk_target));
+        counts[b] = n;
+    }
+    return BFLK_OK;
+}
+
+int bflk_targets_batch_dev(bflk_handle *h, const float *power_dev, int32_t n_maps, int32_t max_targets, float min_rel_power,
+                           bflk_target *targets_dev, int32_t *n_dev, void *cuda_stream) {
+    if (!h) return BFLK_ERR_INVALID;
+    if (!power_dev || !targets_dev || !n_dev || n_maps < 1 || max_targets < 1 || max_targets > 256)
+        return h->fail(BFLK_ERR_INVALID, "bflk_targets_batch_dev: null buffer, n_maps = %d or max_targets = %d (1..256)", n_maps, max_targets);
+    if (!fov_grid(h)) return h->fail(BFLK_ERR_STATE, "bflk_targets_batch_dev: needs a rows x cols grid (bflk_set_grid_fov)");
+    BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
+    cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : h->stream;
+    // ordered like power_map_dev: after the handle's work on another stream (its maps, its angles), and recorded for the next
+    if (h->last_stream != st) BFLK_CUDA(h, cudaStreamWaitEvent(st, h->caller_event, 0));
+    const cudaError_t e = launch_map_targets(power_dev, n_maps, h->rows, h->cols, max_targets, min_rel_power, h->d_theta.p,
+                                             h->d_phi.p, targets_dev, n_dev, h->sm_count, st);
+    const int rc = note_use(h, st, false);
+    BFLK_CUDA(h, e);
+    h->launches++;
+    return rc;
+}
+
 // ---- streaming session (bflk_internal.h: Session) ---------------------------------------------------------------
 static Session *session_of(bflk_handle *h, const char *who) {
     if (!h->session) h->fail(BFLK_ERR_STATE, "%s: no session open (bflk_stream_open)", who);
@@ -1483,15 +1535,30 @@ int bflk_stream_push_i32(bflk_handle *h, const int32_t *rows, int32_t n) {
     return stream_push(h, rows, n, true, "bflk_stream_push_i32");
 }
 
-// bflk_stream_power_maps, and with_beams: bflk_session_beams -- the same frames, consumed the same way
-static int stream_maps(bflk_handle *h, int32_t max_frames, float *power_out, bool with_beams, float *beams_out,
-                       int64_t *first_frame, int32_t *n_frames, const char *who) {
+// What a session maps call returns besides the maps: nothing (bflk_stream_power_maps), the beams (bflk_session_beams) or
+// the Targets of every map (bflk_session_targets).  All three take and consume the same frames the same way.
+struct SessionOut {
+    enum { kMaps, kBeams, kTargets } mode = kMaps;
+    float *beams = nullptr;          // kBeams: [n][count][N]
+    bflk_target *targets = nullptr;  // kTargets: [n][max_targets], with the counts [n]
+    int32_t *n_targets = nullptr;
+    int32_t max_targets = 0;
+    float min_rel = 0.f;
+};
+
+static int stream_maps(bflk_handle *h, int32_t max_frames, float *power_out, const SessionOut &o, int64_t *first_frame,
+                       int32_t *n_frames, const char *who) {
     if (!h) return BFLK_ERR_INVALID;
     Session *s = session_of(h, who);
     if (!s) return BFLK_ERR_STATE;
-    if (!power_out || (with_beams && !beams_out) || !first_frame || !n_frames || max_frames < 1)
+    const bool with_beams = o.mode == SessionOut::kBeams, with_targets = o.mode == SessionOut::kTargets;
+    if (!power_out || (with_beams && !o.beams) || (with_targets && (!o.targets || !o.n_targets)) || !first_frame || !n_frames || max_frames < 1)
         return h->fail(BFLK_ERR_INVALID, "%s: null output or max_frames = %d", who, max_frames);
+    if (with_targets && (o.max_targets < 1 || o.max_targets > 256))
+        return h->fail(BFLK_ERR_INVALID, "%s: max_targets = %d (1..256)", who, o.max_targets);
     if (!h->have_grid) return h->fail(BFLK_ERR_STATE, "%s: set geometry and grid first", who);
+    if (with_targets && (!fov_grid(h) || h->dir_count != h->n_dir))
+        return h->fail(BFLK_ERR_STATE, "%s: needs a rows x cols grid (bflk_set_grid_fov) and the whole map on this handle", who);
     const int64_t tail = frame_tail_samples(h);
     if (tail > s->tail)
         return h->fail(BFLK_ERR_STATE, "%s: a frame now reads %lld samples past its own, the session was opened for %lld (open it again)",
@@ -1512,8 +1579,10 @@ static int stream_maps(bflk_handle *h, int32_t max_frames, float *power_out, boo
                            with_beams ? h->d_beams.p : nullptr);
     if (rc) return rc;
     BFLK_CUDA(h, cudaMemcpyAsync(power_out, h->d_maps.p, (size_t)k * h->dir_count * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
-    if (with_beams) BFLK_CUDA(h, cudaMemcpyAsync(beams_out, h->d_beams.p, n_beams * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
-    BFLK_CUDA(h, cudaStreamSynchronize(h->stream));
+    if (with_beams) BFLK_CUDA(h, cudaMemcpyAsync(o.beams, h->d_beams.p, n_beams * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+    if (with_targets) rc = host_targets(h, h->d_maps.p, k, o.max_targets, o.min_rel, o.targets, o.n_targets);
+    else BFLK_CUDA(h, cudaStreamSynchronize(h->stream));
+    if (rc) return rc;
     s->next_frame += k;
     *n_frames = k;
     h->last_map_on_device = k == 1;   // d_maps[0 .. count) is the map: bflk_targets(NULL) / bflk_heatmap(NULL) use it
@@ -1521,12 +1590,26 @@ static int stream_maps(bflk_handle *h, int32_t max_frames, float *power_out, boo
 }
 
 int bflk_stream_power_maps(bflk_handle *h, int32_t max_frames, float *power_out, int64_t *first_frame, int32_t *n_frames) {
-    return stream_maps(h, max_frames, power_out, false, nullptr, first_frame, n_frames, "bflk_stream_power_maps");
+    return stream_maps(h, max_frames, power_out, SessionOut{}, first_frame, n_frames, "bflk_stream_power_maps");
 }
 
 int bflk_session_beams(bflk_handle *h, int32_t max_frames, float *beams_out, float *power_out, int64_t *first_frame,
                        int32_t *n_frames) {
-    return stream_maps(h, max_frames, power_out, true, beams_out, first_frame, n_frames, "bflk_session_beams");
+    SessionOut o;
+    o.mode = SessionOut::kBeams;
+    o.beams = beams_out;
+    return stream_maps(h, max_frames, power_out, o, first_frame, n_frames, "bflk_session_beams");
+}
+
+int bflk_session_targets(bflk_handle *h, int32_t max_frames, int32_t max_targets, float min_rel_power, float *power_out,
+                         bflk_target *targets_out, int32_t *n_targets, int64_t *first_frame, int32_t *n_frames) {
+    SessionOut o;
+    o.mode = SessionOut::kTargets;
+    o.targets = targets_out;
+    o.n_targets = n_targets;
+    o.max_targets = max_targets;
+    o.min_rel = min_rel_power;
+    return stream_maps(h, max_frames, power_out, o, first_frame, n_frames, "bflk_session_targets");
 }
 
 int bflk_stream_discard(bflk_handle *h, int32_t keep) {
@@ -1640,36 +1723,14 @@ int bflk_resize_u8(bflk_handle *h, const uint8_t *src, int32_t rows, int32_t col
 int bflk_targets(bflk_handle *h, const float *power, int32_t max_targets, float min_rel_power, bflk_target *out, int32_t *n_out) {
     if (!h) return BFLK_ERR_INVALID;
     if (!out || !n_out || max_targets <= 0 || max_targets > 256) return h->fail(BFLK_ERR_INVALID, "bflk_targets: need 1..256 output slots");
-    if (!h->have_grid || h->rows <= 0 || h->cols <= 0 || h->dir_first != 0 || h->dir_count != h->n_dir)
+    if (!fov_grid(h) || h->dir_first != 0 || h->dir_count != h->n_dir)
         return h->fail(BFLK_ERR_STATE, "bflk_targets: needs a rows x cols grid (bflk_set_grid_fov) and the whole map on this handle");
     if (!power && !h->last_map_on_device) return h->fail(BFLK_ERR_STATE, "bflk_targets: no map given and none left on the device by bflk_power_map");
     BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
     const int D = h->n_dir;
     if (power) BFLK_CUDA(h, h->d_post.reserve(D));
-    BFLK_CUDA(h, h->d_bytes.reserve(D));
-    BFLK_CUDA(h, h->d_misc.reserve(3 * (size_t)max_targets + 1));
-    BFLK_CUDA(h, h->p_misc.reserve(3 * (size_t)max_targets + 1));
     if (power) BFLK_CUDA(h, cudaMemcpyAsync(h->d_post.p, power, D * sizeof(float), cudaMemcpyHostToDevice, h->stream));
-    int32_t *d_index = h->d_misc.p, *d_n = h->d_misc.p + 3 * max_targets;
-    float *d_pw = reinterpret_cast<float *>(h->d_misc.p + max_targets), *d_prob = reinterpret_cast<float *>(h->d_misc.p + 2 * max_targets);
-    BFLK_CUDA(h, launch_map_targets(power ? h->d_post.p : h->d_maps.p, h->rows, h->cols, max_targets, min_rel_power, h->d_bytes.p, d_index, d_pw, d_prob, d_n, h->stream));
-    h->launches++;
-    BFLK_CUDA(h, cudaMemcpyAsync(h->p_misc.p, h->d_misc.p, (3 * (size_t)max_targets + 1) * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-    BFLK_CUDA(h, cudaStreamSynchronize(h->stream));
-    const int n = h->p_misc.p[3 * max_targets];
-    for (int i = 0; i < n; i++) {
-        bflk_target &t = out[i];
-        t.direction = h->p_misc.p[i];
-        t.row = t.direction / h->cols;
-        t.col = t.direction % h->cols;
-        t.theta = h->theta[t.direction];
-        t.phi = h->phi[t.direction];
-        std::memcpy(&t.power, &h->p_misc.p[max_targets + i], sizeof(float));
-        std::memcpy(&t.probability, &h->p_misc.p[2 * max_targets + i], sizeof(float));
-        t.reserved = 0;
-    }
-    *n_out = n;
-    return BFLK_OK;
+    return host_targets(h, power ? h->d_post.p : h->d_maps.p, 1, max_targets, min_rel_power, out, n_out);
 }
 
 int bflk_calibrate(bflk_handle *h, const float *signals, int32_t window_len, float reference_power_level, int32_t *index,

@@ -226,7 +226,8 @@ struct bflk_handle {
     int32_t n_dir = 0;           // D (whole grid)
     int32_t dir_first = 0, dir_count = 0;
     int32_t max_delay = 0;       // largest integer delay in the LUT
-    std::vector<double> theta, phi;
+    std::vector<double> theta, phi;   // [D] of a bflk_set_grid_fov grid, empty for caller tables
+    bflk::DevBuf<double> d_theta, d_phi;   // device copies of theta / phi (the records of the targets kernel)
     bflk::DevBuf<int32_t> d_off;  // [D][C]
     bflk::DevBuf<float> d_frac;   // [D][C]
 
@@ -263,7 +264,11 @@ struct bflk_handle {
     int64_t resident_stride = 0;              // its row stride: window_len, or 2 * cap of the session's ring
     std::unique_ptr<bflk::Session> session;   // bflk_stream_open .. bflk_stream_close
     bflk::DevBuf<int32_t> d_wire;
-    bflk::DevBuf<uint8_t> d_bytes;            // heat-map / resize / peak-candidate scratch
+    bflk::DevBuf<uint8_t> d_bytes;            // resize scratch
+    bflk::DevBuf<bflk_target> d_targets;      // records of bflk_targets / bflk_session_targets ...
+    bflk::DevBuf<int32_t> d_target_counts;    // ... and their counts per map
+    bflk::PinBuf<bflk_target> p_targets;
+    bflk::PinBuf<int32_t> p_target_counts;
     // bflk_power_map_batch_submit / _wait: two batches in flight, each with its own device buffers
     bflk::DevBuf<float> d_async_in[2], d_async_out[2];
     bflk::Event async_done[2];
@@ -474,8 +479,11 @@ cudaError_t launch_history_push(const float *d_block, const int32_t *d_wire, int
                                 cudaStream_t st);
 cudaError_t launch_ffma2_peak(float *d_out, int n_blocks, int iters, cudaStream_t st);
 cudaError_t launch_resize_u8(const uint8_t *d_src, int ih, int iw, uint8_t *d_dst, int oh, int ow, const int32_t *d_tab, cudaStream_t st);
-cudaError_t launch_map_targets(const float *d_power, int rows, int cols, int max_targets, float min_rel, uint8_t *d_cand,
-                               int32_t *d_index, float *d_pw, float *d_prob, int32_t *d_n, cudaStream_t st);
+// Targets of n_maps whole-grid maps d_maps[n_maps][rows * cols], one CTA each: d_targets[n_maps][max_targets] (records past a
+// map's count are not written), d_counts[n_maps]; d_theta / d_phi [rows * cols] are the grid's angles
+cudaError_t launch_map_targets(const float *d_maps, int n_maps, int rows, int cols, int max_targets, float min_rel,
+                               const double *d_theta, const double *d_phi, bflk_target *d_targets, int32_t *d_counts,
+                               int sm_count, cudaStream_t st);
 
 // ---- bflk_api.cu internals used by multi.cu ---------------------------------------------------------------
 // How power_map_dev runs.  A plain call orders itself against the handle's earlier calls through caller_event; a pipelined

@@ -179,92 +179,138 @@ cudaError_t launch_resize_u8(const uint8_t *d_src, int ih, int iw, uint8_t *d_ds
     return cudaGetLastError();
 }
 
-// ---- peaks of the map as Targets (src/dsp/worker.h:32-61) -----------------------------------------------------------
-// One CTA.  Pass 1 marks the directions that are the maximum of their 3x3 neighbourhood (ties: lowest index) and carry at
-// least min_rel of the map's maximum; pass 2 picks the max_targets strongest of them in order (power descending, index
-// ascending) and forms the tracker-style probability 1 / gradientError from the four grid neighbours
+// ---- peaks of the maps as Targets (src/dsp/worker.h:32-61) ----------------------------------------------------------
+// One CTA per map (blockIdx.x).  A direction is a candidate when it carries at least min_rel of the map's maximum and is the
+// maximum of its 3x3 neighbourhood (ties: lowest index); the max_targets strongest candidates come out in order (power
+// descending, index ascending), each with the tracker-style probability 1 / gradientError from the four grid neighbours
 // (src/dsp/gradient_ascend.cpp:62-76).  Same definition as oracle.c orc_map_targets.
-__global__ void __launch_bounds__(1024) map_targets_kernel(const float *__restrict__ power, int rows, int cols, int max_targets,
-                                                          float min_rel, uint8_t *__restrict__ cand, int32_t *__restrict__ out_index,
-                                                          float *__restrict__ out_power, float *__restrict__ out_prob,
-                                                          int32_t *__restrict__ out_n) {
+//
+// Candidates have power > 0, so key(i) = power bits << 32 | ~i orders them exactly as the selection does, and pick n + 1 is
+// the largest key below pick n: nothing is marked taken, and the CTA needs no global scratch.  The candidates are kept as a
+// bitmask in dynamic shared memory (one bit per direction) when the launch provides it, else re-evaluated on every pick.
+__device__ __forceinline__ bool is_peak(const float *__restrict__ power, int rows, int cols, int i, float thr) {
+    const float p = power[i];
+    if (!(p >= thr && p > 0.0f)) return false;
+    const int r = i / cols, c = i - r * cols;
+    for (int dr = -1; dr <= 1; dr++)
+        for (int dc = -1; dc <= 1; dc++) {
+            const int rr = r + dr, cc = c + dc;
+            if ((dr == 0 && dc == 0) || rr < 0 || rr >= rows || cc < 0 || cc >= cols) continue;
+            const int j = rr * cols + cc;
+            const float q = power[j];
+            if (q > p || (q == p && j < i)) return false;
+        }
+    return true;
+}
+
+__device__ __forceinline__ unsigned long long peak_key(float p, int i) {
+    return (unsigned long long)__float_as_uint(p) << 32 | (unsigned)~i;
+}
+
+__global__ void __launch_bounds__(1024) map_targets_kernel(const float *__restrict__ maps, int rows, int cols, int max_targets,
+                                                          float min_rel, bool use_mask, const double *__restrict__ theta,
+                                                          const double *__restrict__ phi, bflk_target *__restrict__ targets,
+                                                          int32_t *__restrict__ counts) {
+    extern __shared__ uint32_t s_mask[];   // [ceil(D / 32)] when use_mask
     __shared__ float s_v[32];
-    __shared__ int s_i[32];
-    __shared__ float s_max;
-    __shared__ int s_best;
-    const int D = rows * cols;
+    __shared__ unsigned long long s_k[32];
+    __shared__ unsigned long long s_pick;
+    const int D = rows * cols, words = (D + 31) / 32;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, n_warps = blockDim.x >> 5;
+    const float *__restrict__ power = maps + (size_t)blockIdx.x * D;
+    bflk_target *out = targets + (size_t)blockIdx.x * max_targets;
+
     float mx = 0.0f;
     for (int i = threadIdx.x; i < D; i += blockDim.x) mx = fmaxf(mx, power[i]);
     for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-    if ((threadIdx.x & 31) == 0) s_v[threadIdx.x >> 5] = mx;
+    if (lane == 0) s_v[warp] = mx;
     __syncthreads();
-    if (threadIdx.x == 0) {
-        float m = 0.0f;
-        for (int w = 0; w < (int)(blockDim.x >> 5); w++) m = fmaxf(m, s_v[w]);
-        s_max = m;
-    }
-    __syncthreads();
-    const float thr = __fmul_rn(min_rel, s_max);
-    for (int i = threadIdx.x; i < D; i += blockDim.x) {
-        const float p = power[i];
-        bool is_max = p >= thr && p > 0.0f;
-        if (is_max) {
-            const int r = i / cols, c = i - r * cols;
-            for (int dr = -1; dr <= 1 && is_max; dr++)
-                for (int dc = -1; dc <= 1; dc++) {
-                    const int rr = r + dr, cc = c + dc;
-                    if ((dr == 0 && dc == 0) || rr < 0 || rr >= rows || cc < 0 || cc >= cols) continue;
-                    const int j = rr * cols + cc;
-                    const float q = power[j];
-                    if (q > p || (q == p && j < i)) { is_max = false; break; }
-                }
+    mx = 0.0f;
+    for (int w = 0; w < n_warps; w++) mx = fmaxf(mx, s_v[w]);
+    const float thr = __fmul_rn(min_rel, mx);
+    if (use_mask) {
+        for (int w = warp; w < words; w += n_warps) {   // one word per warp: lane b tests direction 32 w + b
+            const int i = w * 32 + lane;
+            const unsigned bits = __ballot_sync(0xffffffffu, i < D && is_peak(power, rows, cols, i, thr));
+            if (lane == 0) s_mask[w] = bits;
         }
-        cand[i] = is_max ? 1 : 0;
+        __syncthreads();
     }
-    __syncthreads();
+    unsigned long long prev = ~0ull;
     int n = 0;
     for (; n < max_targets; n++) {
-        float best = -1.0f;
-        int besti = 0x7fffffff;
-        for (int i = threadIdx.x; i < D; i += blockDim.x)
-            if (cand[i]) {
-                const float p = power[i];
-                if (p > best || (p == best && i < besti)) { best = p; besti = i; }
-            }
-        for (int o = 16; o > 0; o >>= 1) {
-            const float ov = __shfl_xor_sync(0xffffffffu, best, o);
-            const int oi = __shfl_xor_sync(0xffffffffu, besti, o);
-            if (ov > best || (ov == best && oi < besti)) { best = ov; besti = oi; }
+        unsigned long long best = 0;   // 0: no candidate below prev
+        if (use_mask) {
+            for (int w = threadIdx.x; w < words; w += blockDim.x)
+                for (unsigned bits = s_mask[w]; bits; bits &= bits - 1) {
+                    const int i = w * 32 + __ffs(bits) - 1;
+                    const unsigned long long k = peak_key(power[i], i);
+                    if (k < prev && k > best) best = k;
+                }
+        } else {
+            for (int i = threadIdx.x; i < D; i += blockDim.x)
+                if (is_peak(power, rows, cols, i, thr)) {
+                    const unsigned long long k = peak_key(power[i], i);
+                    if (k < prev && k > best) best = k;
+                }
         }
-        if ((threadIdx.x & 31) == 0) { s_v[threadIdx.x >> 5] = best; s_i[threadIdx.x >> 5] = besti; }
+        for (int o = 16; o > 0; o >>= 1) best = max(best, __shfl_xor_sync(0xffffffffu, best, o));
+        if (lane == 0) s_k[warp] = best;
         __syncthreads();
-        if (threadIdx.x == 0) {
-            for (int w = 1; w < (int)(blockDim.x >> 5); w++)
-                if (s_v[w] > best || (s_v[w] == best && s_i[w] < besti)) { best = s_v[w]; besti = s_i[w]; }
-            s_best = best >= 0.0f ? besti : -1;
-            if (s_best >= 0) {
-                const int i = s_best, r = i / cols, c = i - r * cols;
-                const float p = power[i];
-                const double ql = c > 0 ? power[i - 1] : p, qr = c < cols - 1 ? power[i + 1] : p;
-                const double qu = r > 0 ? power[i - cols] : p, qd = r < rows - 1 ? power[i + cols] : p;
-                const double err = (fabs(qr - ql) + fabs(qd - qu)) / (((ql + qr) + qu) + qd);
-                double pr = 1.0 / err;
-                if (!(pr < 3.4028234663852886e38)) pr = 3.4028234663852886e38;
-                out_index[n] = i;
-                out_power[n] = p;
-                out_prob[n] = (float)pr;
-                cand[i] = 0;
+        if (warp == 0) {
+            best = lane < n_warps ? s_k[lane] : 0;
+            for (int o = 16; o > 0; o >>= 1) best = max(best, __shfl_xor_sync(0xffffffffu, best, o));
+            if (lane == 0) {
+                s_pick = best;
+                if (best) {
+                    const int i = (int)~(unsigned)best, r = i / cols, c = i - r * cols;
+                    const float p = power[i];
+                    const double ql = c > 0 ? power[i - 1] : p, qr = c < cols - 1 ? power[i + 1] : p;
+                    const double qu = r > 0 ? power[i - cols] : p, qd = r < rows - 1 ? power[i + cols] : p;
+                    const double err = (fabs(qr - ql) + fabs(qd - qu)) / (((ql + qr) + qu) + qd);
+                    double pr = 1.0 / err;
+                    if (!(pr < 3.4028234663852886e38)) pr = 3.4028234663852886e38;
+                    bflk_target t;
+                    t.theta = theta[i];
+                    t.phi = phi[i];
+                    t.power = p;
+                    t.probability = (float)pr;
+                    t.direction = i;
+                    t.row = r;
+                    t.col = c;
+                    t.reserved = 0;
+                    out[n] = t;
+                }
             }
         }
         __syncthreads();
-        if (s_best < 0) break;
+        prev = s_pick;
+        if (!prev) break;
     }
-    if (threadIdx.x == 0) *out_n = n;
+    if (threadIdx.x == 0) counts[blockIdx.x] = n;
 }
 
-cudaError_t launch_map_targets(const float *d_power, int rows, int cols, int max_targets, float min_rel, uint8_t *d_cand,
-                               int32_t *d_index, float *d_pw, float *d_prob, int32_t *d_n, cudaStream_t st) {
-    map_targets_kernel<<<1, 1024, 0, st>>>(d_power, rows, cols, max_targets, min_rel, d_cand, d_index, d_pw, d_prob, d_n);
+cudaError_t launch_map_targets(const float *d_maps, int n_maps, int rows, int cols, int max_targets, float min_rel,
+                               const double *d_theta, const double *d_phi, bflk_target *d_targets, int32_t *d_counts,
+                               int sm_count, cudaStream_t st) {
+    // the candidate bitmask takes whatever shared memory a block may opt into beside the kernel's static arrays (on a B200
+    // 227 KB: grids of up to 1.85 M directions); beyond the kernel's current dynamic limit (48 KB less the static arrays
+    // until raised) it is raised first -- per device, so checked per launch
+    int dev = 0, optin = 0;
+    cudaFuncAttributes fa;
+    cudaError_t e;
+    if ((e = cudaGetDevice(&dev)) != cudaSuccess) return e;
+    if ((e = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev)) != cudaSuccess) return e;
+    if ((e = cudaFuncGetAttributes(&fa, map_targets_kernel)) != cudaSuccess) return e;
+    const size_t mask_bytes = ((size_t)rows * cols + 31) / 32 * sizeof(uint32_t);
+    const bool use_mask = mask_bytes + fa.sharedSizeBytes <= (size_t)optin;
+    if (use_mask && mask_bytes > (size_t)fa.maxDynamicSharedSizeBytes &&
+        (e = cudaFuncSetAttribute(map_targets_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mask_bytes)) != cudaSuccess)
+        return e;
+    // a map per CTA: few maps get the whole SM each, a backlog smaller CTAs so that several maps share an SM
+    const int threads = n_maps < sm_count ? 1024 : 256;
+    map_targets_kernel<<<n_maps, threads, use_mask ? mask_bytes : 0, st>>>(d_maps, rows, cols, max_targets, min_rel, use_mask,
+                                                                           d_theta, d_phi, d_targets, d_counts);
     return cudaGetLastError();
 }
 

@@ -28,6 +28,7 @@
  *   bflk_heatmap                    MIMOWorker::populateHeatmap (src/dsp/mimo.cpp:61-95)
  *   bflk_resize_u8                  cv::resize(..., INTER_LINEAR) in AWProcessingUnit::draw (aw_processing_unit.cpp:245-259)
  *   bflk_targets                    Worker::tracking / getTargets (src/dsp/worker.h:32-61,136-142) for the MIMO map
+ *   bflk_targets_batch_dev, bflk_session_targets   the same for every map of a device batch or a session backlog, in one launch
  *   bflk_calibrate                  AWProcessingUnit::calibrate mask (aw_processing_unit.cpp:126-200)
  *   bflk_ingest_i32, bflk_power_map_i32   Pipeline::receive_exposure conversion (src/fpga/pipeline.cpp:260-297)
  *   bflk_stream_*                   Streams (src/fpga/streams.hpp:152-182) + the worker loop (src/dsp/worker.h:212-224),
@@ -215,6 +216,11 @@ int bflk_kernel_time_ms(bflk_handle *h, float *das_ms, int32_t *das_launches, fl
  * bflk_session_beams is bflk_stream_power_maps that also returns the frames' beams (bflk_beams_batch_dev):
  * beams_out[n][count][N] and power_out[n][count] on the host.  It takes and consumes frames exactly as the maps call does
  * (the two may be interleaved), and after a one-frame call bflk_targets / bflk_heatmap with a NULL map use that frame's map.
+ * bflk_session_targets is bflk_stream_power_maps that also returns the Targets of every frame it maps (bflk_targets_batch_dev,
+ * one launch for all of them): power_out[n][count], targets_out[n][max_targets] and n_targets[n] on the host; records past a
+ * frame's count are not written.  It takes and consumes frames exactly as the other two (all three may be interleaved), and
+ * after a one-frame call bflk_targets / bflk_heatmap with a NULL map use that frame's map.  It needs a bflk_set_grid_fov
+ * grid and the whole grid on the handle (BFLK_ERR_STATE otherwise); a refused call consumes no frame.
  * bflk_stream_discard skips every ready frame but the newest `keep`.  bflk_stream_status: samples pushed per channel, the
  * next frame a maps call returns, frames ready, frames skipped so far.
  *
@@ -229,6 +235,9 @@ int bflk_stream_push_i32(bflk_handle *h, const int32_t *rows, int32_t n);   /* [
 int bflk_stream_power_maps(bflk_handle *h, int32_t max_frames, float *power_out, int64_t *first_frame, int32_t *n_frames);
 int bflk_session_beams(bflk_handle *h, int32_t max_frames, float *beams_out, float *power_out, int64_t *first_frame,
                        int32_t *n_frames);
+typedef struct bflk_target bflk_target;
+int bflk_session_targets(bflk_handle *h, int32_t max_frames, int32_t max_targets, float min_rel_power, float *power_out,
+                         bflk_target *targets_out, int32_t *n_targets, int64_t *first_frame, int32_t *n_frames);
 int bflk_stream_discard(bflk_handle *h, int32_t keep);
 int bflk_stream_status(const bflk_handle *h, int64_t *pushed, int64_t *next_frame, int32_t *ready, int64_t *skipped);
 int bflk_stream_window(bflk_handle *h, int64_t frame);
@@ -351,16 +360,25 @@ int bflk_resize_u8(bflk_handle *h, const uint8_t *src, int32_t rows, int32_t col
  * (ties: lowest index) and carries at least min_rel_power of the map's maximum; strongest first.  power = the map
  * value; probability = 1 / gradientError as the gradient tracker reports it (src/dsp/gradient_ascend.cpp:62-76,406),
  * with the four grid neighbours in place of the four quadrant beams.  power == NULL: the map the last bflk_power_map
- * call left on the device (no upload).  Needs a bflk_set_grid_fov grid and the whole map on this handle. */
-typedef struct bflk_target {
+ * call left on the device (no upload).  Needs a bflk_set_grid_fov grid and the whole map on this handle: caller tables,
+ * with or without bflk_set_grid_shape, or a direction range give BFLK_ERR_STATE.  max_targets: 1..256. */
+struct bflk_target {         /* 40 bytes (typedef above) */
     double theta, phi;      /* Spherical direction of the grid cell (bflk_get_grid) */
     float power;
     float probability;
     int32_t direction;      /* r * cols + c */
     int32_t row, col;
-    int32_t reserved;
-} bflk_target;
+    int32_t reserved;       /* 0 */
+};
 int bflk_targets(bflk_handle *h, const float *power, int32_t max_targets, float min_rel_power, bflk_target *out, int32_t *n_out);
+/* The same for n_maps whole-grid maps on the DEVICE, one launch: power_dev[n_maps][D] (D = rows * cols; the handle's direction
+ * range is not consulted, so a rank of a sharded job can pass its power_all_dev) -> targets_dev[n_maps][max_targets] (records
+ * past a map's count are not written) and n_dev[n_maps], device buffers.  Each map's records are those bflk_targets gives for
+ * it.  Asynchronous on cuda_stream (NULL = the handle's stream), ordered against the handle's earlier calls on other streams
+ * as bflk_power_map_batch_dev is; the map bflk_targets / bflk_heatmap use with NULL is not touched.  Any n_maps >= 1;
+ * max_targets 1..256.  Needs a bflk_set_grid_fov grid (BFLK_ERR_STATE otherwise). */
+int bflk_targets_batch_dev(bflk_handle *h, const float *power_dev, int32_t n_maps, int32_t max_targets, float min_rel_power,
+                           bflk_target *targets_dev, int32_t *n_dev, void *cuda_stream);
 /* calibrate(): signals[64][W] of one array -> index[<=64], correction[<=64]; *usable = count. */
 int bflk_calibrate(bflk_handle *h, const float *signals, int32_t window_len, float reference_power_level,
                    int32_t *index, float *correction, int32_t *usable, float *median, float *mean);
