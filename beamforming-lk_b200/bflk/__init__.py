@@ -487,6 +487,19 @@ class Beamformer:
                                       _ptr(audio) if want_audio else None, _ptr(power) if want_power else None))
         return audio, power
 
+    def set_window_dev(self, window_dev_ptr):
+        """Borrow a device window [C][W] float32 (e.g. a torch tensor's data_ptr()) as the resident one; 0 / None forgets it.
+        The buffer must outlive its use: the handle does not copy it."""
+        self._check(self._L.bflk_set_window_dev(self._h, C.c_void_p(window_dev_ptr) if window_dev_ptr else None))
+
+    def miso_dev(self, theta, phi, window_dev_ptr, audio_dev_ptr, power_dev_ptr, cuda_stream=0):
+        """miso() on device buffers, asynchronous on cuda_stream: window [C][W] (None: the resident window), audio [T][N]
+        and power [T] (either may be 0 / None).  A delay beyond the history is clamped to it, not reported (bflk.h)."""
+        theta, phi = _np(theta, np.float64).ravel(), _np(phi, np.float64).ravel()
+        ptr = lambda p: C.c_void_p(p) if p else None
+        self._check(self._L.bflk_miso_dev(self._h, _ptr(theta), _ptr(phi), theta.shape[0], ptr(window_dev_ptr),
+                                          ptr(audio_dev_ptr), ptr(power_dev_ptr), C.c_void_p(cuda_stream)))
+
     def set_fir(self, coeffs):
         """FIR interpolation of the reference's USE_FILTER build (delay.cpp:28-40): coeffs [n_phases][taps], None = 2-tap form."""
         if coeffs is None:

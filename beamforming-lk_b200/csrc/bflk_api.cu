@@ -1173,6 +1173,8 @@ int bflk_set_window_dev(bflk_handle *h, const float *window_dev) {
 static int miso_launch(bflk_handle *h, const double *theta, const double *phi, int n_targets, const float *window_dev,
                        int64_t row_stride, float *audio_dev, float *power_dev, int32_t *flag_dev, cudaStream_t st) {
     const int C = h->cfg.n_channels, N = h->cfg.frame_len;
+    // the partial sums, counters and range flag are the handle's: a call on another stream than the previous one waits for it
+    if (h->last_stream != st) BFLK_CUDA(h, cudaStreamWaitEvent(st, h->caller_event, 0));
     MisoArgs a{};
     if (n_targets <= kMisoInline) {
         for (int i = 0; i < n_targets; i++) a.trig_inline[i] = make_trig(theta[i], phi[i]);
@@ -1259,6 +1261,7 @@ static int miso_dev(bflk_handle *h, const double *theta, const double *phi, int3
     a.audio = audio_dev;
     a.norm = static_cast<float>(N);
     a.fir = h->d_fir.p; a.fir_phases = h->fir_phases; a.fir_taps = h->fir_taps;
+    if (h->last_stream != st) BFLK_CUDA(h, cudaStreamWaitEvent(st, h->caller_event, 0));
     BFLK_CUDA(h, launch_das_generic(a, st));
     h->launches++;
     return note_use(h, st, false);

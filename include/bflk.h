@@ -311,12 +311,16 @@ int bflk_set_window_dev(bflk_handle *h, const float *window_dev);
 /* For each target t: steer(theta[t], phi[t]); audio_out[t][N] = Particle::das; power_out[t] = Particle::beam.
  * Either output may be NULL. window[C][W] as in bflk_power_map, or NULL = the resident window.  One kernel launch:
  * the steering tables are built inside it (same bits as bflk_steer_tables); a delay beyond the history makes the
- * call return BFLK_ERR_RANGE. */
+ * call return BFLK_ERR_RANGE.  Only the channels of the mask are checked: a microphone outside it may lie beyond the
+ * history (its delay still counts for the minimum every delay is measured from), whereas bflk_steer_tables and
+ * bflk_set_grid_fov check every channel. */
 int bflk_miso(bflk_handle *h, const double *theta, const double *phi, int32_t n_targets, const float *window,
               float *audio_out, float *power_out);
 /* Device pointers, asynchronous on cuda_stream (NULL = the handle's stream); window_dev == NULL = the resident window.
  * Being asynchronous it cannot return BFLK_ERR_RANGE: a delay beyond the history is clamped to it (validate the
- * directions once with bflk_steer_tables, or use bflk_miso). */
+ * directions once with bflk_steer_tables, or use bflk_miso).  With FIR interpolation set it builds its tables
+ * synchronously and does return BFLK_ERR_RANGE.  It is ordered after the handle's earlier calls on other streams (and
+ * bflk_miso after it), since all MISO calls share the handle's partial sums. */
 int bflk_miso_dev(bflk_handle *h, const double *theta, const double *phi, int32_t n_targets,
                   const float *window_dev, float *audio_dev, float *power_dev, void *cuda_stream);
 

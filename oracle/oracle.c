@@ -33,6 +33,10 @@ void orc_create_tiled_antenna(float *xyz, int n_tiles, const float *origins) {
 
 /* ---- a2-a5 -------------------------------------------------------------------------------- */
 void orc_steering_vector_spherical(const float *xyz, int C, double theta, double phi, float *delays) {
+    orc_steering_vector_spherical_k(xyz, C, theta, phi, (float)(ORC_SAMPLE_RATE / ORC_PROPAGATION_SPEED), delays);
+}
+
+void orc_steering_vector_spherical_k(const float *xyz, int C, double theta, double phi, float k, float *delays) {
     /* steer(): rotateY(-float(theta)) * (rotateZ(float(phi)) * points), antenna.cpp:99-107.
      * Matrix entries: float(cos/sin((double)angle)), geometry.cpp:219-233.
      * Product evaluation order (Eigen 3.4 GEMM path, FMA-contracted, k = 0,1,2 from a zero
@@ -43,9 +47,8 @@ void orc_steering_vector_spherical(const float *xyz, int C, double theta, double
     const float cy = (float)cos((double)ay), sy = (float)sin((double)ay);
     const float Rz[3][3] = {{cz, -sz, 0.0f}, {sz, cz, 0.0f}, {0.0f, 0.0f, 1.0f}};
     const float Ry[3][3] = {{cy, 0.0f, sy}, {0.0f, 1.0f, 0.0f}, {-sy, 0.0f, cy}};
-    /* compute_delays(): row(Z) * (SAMPLE_RATE / PROPAGATION_SPEED) as float x float, then
-     * subtract the minimum, antenna.cpp:89-97. */
-    const float k = (float)(ORC_SAMPLE_RATE / ORC_PROPAGATION_SPEED);
+    /* compute_delays(): row(Z) * k as float x float, k = float(SAMPLE_RATE / PROPAGATION_SPEED), then subtract the
+     * minimum, antenna.cpp:89-97. */
     float mn = INFINITY;
     for (int c = 0; c < C; c++) {
         const float *p = &xyz[3 * c];
@@ -98,13 +101,18 @@ void orc_mimo_grid(int rows, int cols, double fov_deg, double *theta, double *ph
 
 void orc_mimo_lut(const float *xyz, int C, int rows, int cols, double fov_deg, int history,
                   int32_t *offsets, float *fractions) {
+    orc_mimo_lut_k(xyz, C, rows, cols, fov_deg, history, (float)(ORC_SAMPLE_RATE / ORC_PROPAGATION_SPEED), offsets, fractions);
+}
+
+void orc_mimo_lut_k(const float *xyz, int C, int rows, int cols, double fov_deg, int history, float k,
+                    int32_t *offsets, float *fractions) {
     int D = rows * cols;
     double *theta = (double *)malloc(sizeof(double) * D), *phi = (double *)malloc(sizeof(double) * D);
     float *del = (float *)malloc(sizeof(float) * C);
     orc_mimo_grid(rows, cols, fov_deg, theta, phi);
-    for (int k = 0; k < D; k++) {
-        orc_steering_vector_spherical(xyz, C, theta[k], phi[k], del);
-        orc_split_delays(del, C, history, &offsets[(size_t)k * C], &fractions[(size_t)k * C]);
+    for (int d = 0; d < D; d++) {
+        orc_steering_vector_spherical_k(xyz, C, theta[d], phi[d], k, del);
+        orc_split_delays(del, C, history, &offsets[(size_t)d * C], &fractions[(size_t)d * C]);
     }
     free(theta); free(phi); free(del);
 }
@@ -300,6 +308,16 @@ void orc_delay_fir(float *out, const float *signal, float fraction, int n, const
     if (delay_int > n_phases - 1) delay_int = n_phases - 1;
     for (int k = 0; k < n; k++)
         for (int i = 0; i < taps; i++) out[k] = out[k] + coeffs[(size_t)delay_int * taps + i] * signal[k + i];
+}
+
+/* Particle::das with the FIR delay(): the delayed sum of one direction, channels in mask order */
+void orc_particle_das_fir(const float *window, int W, int n, const int *index, int usable, const int32_t *offsets,
+                          const float *fractions, const float *coeffs, int n_phases, int taps, float *out) {
+    memset(out, 0, sizeof(float) * n);
+    for (int s = 0; s < usable; s++) {
+        int i = index[s];
+        orc_delay_fir(out, &window[(size_t)i * W + offsets[i]], fractions[i], n, coeffs, n_phases, taps);
+    }
 }
 
 void orc_mimo_update_fir(const float *window, int C, int W, int n, const int *index, int usable,

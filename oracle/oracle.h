@@ -41,6 +41,9 @@ void orc_create_tiled_antenna(float *xyz, int n_tiles, const float *origins);
 /* a2-a5: steering_vector_spherical, src/geometry/antenna.cpp:89-107,126-134 and
  * src/geometry/geometry.cpp:219-233.  delays[C] in samples, min-subtracted. */
 void orc_steering_vector_spherical(const float *xyz, int C, double theta, double phi, float *delays);
+/* the same with the delay scale k (samples per metre, float(sample_rate / propagation_speed)) given; the entry point
+ * above passes float(ORC_SAMPLE_RATE / ORC_PROPAGATION_SPEED) */
+void orc_steering_vector_spherical_k(const float *xyz, int C, double theta, double phi, float k, float *delays);
 
 /* a6/a7 split: fraction = (float)modf((double)del, &ip); offset = history - (int)ip
  * (src/dsp/mimo.cpp:46-54, src/dsp/particle.cpp:37-49; history == N_SAMPLES == 256 there). */
@@ -54,6 +57,8 @@ void orc_mimo_grid(int rows, int cols, double fov_deg, double *theta, double *ph
 /* a6: full LUT, offsets/fractions [D][C] row-major, D = rows*cols, k = r*cols + c. */
 void orc_mimo_lut(const float *xyz, int C, int rows, int cols, double fov_deg, int history,
                   int32_t *offsets, float *fractions);
+void orc_mimo_lut_k(const float *xyz, int C, int rows, int cols, double fov_deg, int history, float k,
+                    int32_t *offsets, float *fractions);
 
 /* a9: delay(), src/dsp/delay.cpp:16-26 (AVX2 variant) == scalar twin :44-48 with the FMA pinned:
  * out[i] = out[i] + fma(fraction, signal[i] - signal[i+1], signal[i+1]), i in [0, n). */
@@ -96,6 +101,9 @@ void orc_delay_fir(float *out, const float *signal, float fraction, int n, const
 void orc_mimo_update_fir(const float *window, int C, int W, int n, const int *index, int usable,
                          const int32_t *offsets, const float *fractions, int D, const float *coeffs, int n_phases,
                          int taps, float *power);
+/* Particle::das around the FIR delay(): out[n] of one direction (window rows W apart, offset + n + taps - 1 <= W) */
+void orc_particle_das_fir(const float *window, int W, int n, const int *index, int usable, const int32_t *offsets,
+                          const float *fractions, const float *coeffs, int n_phases, int taps, float *out);
 
 #ifdef __cplusplus
 }

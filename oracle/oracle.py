@@ -13,6 +13,8 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 N_SAMPLES = 256
 WINDOW = 1024
 ELEMENTS = 64
+SAMPLE_RATE = 48828.0         # src/geometry/antenna.h:17
+PROPAGATION_SPEED = 340.0     # src/geometry/antenna.h:16
 
 _f32p = np.ctypeslib.ndpointer(np.float32, flags="C_CONTIGUOUS")
 _f64p = np.ctypeslib.ndpointer(np.float64, flags="C_CONTIGUOUS")
@@ -43,9 +45,11 @@ def lib():
         L.orc_create_antenna.argtypes = [_f32p, C.c_int, C.c_int, C.c_float]
         L.orc_create_tiled_antenna.argtypes = [_f32p, C.c_int, _f32p]
         L.orc_steering_vector_spherical.argtypes = [_f32p, C.c_int, C.c_double, C.c_double, _f32p]
+        L.orc_steering_vector_spherical_k.argtypes = [_f32p, C.c_int, C.c_double, C.c_double, C.c_float, _f32p]
         L.orc_split_delays.argtypes = [_f32p, C.c_int, C.c_int, _i32p, _f32p]
         L.orc_mimo_grid.argtypes = [C.c_int, C.c_int, C.c_double, _f64p, _f64p]
         L.orc_mimo_lut.argtypes = [_f32p, C.c_int, C.c_int, C.c_int, C.c_double, C.c_int, _i32p, _f32p]
+        L.orc_mimo_lut_k.argtypes = [_f32p, C.c_int, C.c_int, C.c_int, C.c_double, C.c_int, C.c_float, _i32p, _f32p]
         L.orc_delay.argtypes = [_f32p, _f32p, C.c_float, C.c_int]
         L.orc_mimo_update.argtypes = [_f32p, C.c_int, C.c_int, C.c_int, _i32p, C.c_int, _i32p, _f32p, C.c_int, _f32p]
         L.orc_mimo_das.argtypes = [_f32p, C.c_int, C.c_int, C.c_int, _i32p, C.c_int, _i32p, _f32p, C.c_int, _f32p]
@@ -56,6 +60,9 @@ def lib():
         L.orc_mimo_update_fir.restype = None
         L.orc_delay_fir.argtypes = [_f32p, _f32p, C.c_float, C.c_int, _f32p, C.c_int, C.c_int]
         L.orc_delay_fir.restype = None
+        L.orc_particle_das_fir.argtypes = [_f32p, C.c_int, C.c_int, _i32p, C.c_int, _i32p, _f32p, _f32p, C.c_int, C.c_int,
+                                           _f32p]
+        L.orc_particle_das_fir.restype = None
         L.orc_quadrant.argtypes = [_f64p, C.c_double, C.c_double, C.c_double, _f64p, _f64p]
         L.orc_quadrant.restype = None
         L.orc_monopulse_gradient.argtypes = [_f64p, C.c_double, _f64p, _f64p]
@@ -147,9 +154,20 @@ def create_tiled_antenna(origins):
     return xyz
 
 
-def steering_vector_spherical(xyz, theta, phi):
+def delay_scale(sample_rate=SAMPLE_RATE, propagation_speed=PROPAGATION_SPEED):
+    """Samples per metre of path difference, float(sample_rate / propagation_speed) as compute_delays() scales
+    (antenna.cpp:90-92) and the library derives it from its config."""
+    return float(np.float32(float(sample_rate) / float(propagation_speed)))
+
+
+def steering_vector_spherical(xyz, theta, phi, scale=None):
+    """Delays [C] in samples, min-subtracted; scale (delay_scale()) defaults to the reference's constants."""
     d = np.zeros(xyz.shape[0], np.float32)
-    lib().orc_steering_vector_spherical(np.ascontiguousarray(xyz, np.float32), xyz.shape[0], float(theta), float(phi), d)
+    xyz = np.ascontiguousarray(xyz, np.float32)
+    if scale is None:
+        lib().orc_steering_vector_spherical(xyz, xyz.shape[0], float(theta), float(phi), d)
+    else:
+        lib().orc_steering_vector_spherical_k(xyz, xyz.shape[0], float(theta), float(phi), float(scale), d)
     return d
 
 
@@ -168,21 +186,25 @@ def mimo_grid(rows, cols, fov_deg):
     return th, ph
 
 
-def mimo_lut(xyz, rows, cols, fov_deg, history=N_SAMPLES):
+def mimo_lut(xyz, rows, cols, fov_deg, history=N_SAMPLES, scale=None):
     Cn = xyz.shape[0]
     off = np.zeros((rows * cols, Cn), np.int32)
     fr = np.zeros((rows * cols, Cn), np.float32)
-    lib().orc_mimo_lut(np.ascontiguousarray(xyz, np.float32), Cn, rows, cols, float(fov_deg), history, off, fr)
+    xyz = np.ascontiguousarray(xyz, np.float32)
+    if scale is None:
+        lib().orc_mimo_lut(xyz, Cn, rows, cols, float(fov_deg), history, off, fr)
+    else:
+        lib().orc_mimo_lut_k(xyz, Cn, rows, cols, float(fov_deg), history, float(scale), off, fr)
     return off, fr
 
 
-def steer_tables(xyz, thetas, phis, history=N_SAMPLES):
+def steer_tables(xyz, thetas, phis, history=N_SAMPLES, scale=None):
     """Particle::steer for a list of directions -> offsets/fractions [T][C]."""
     T = len(thetas)
     off = np.zeros((T, xyz.shape[0]), np.int32)
     fr = np.zeros((T, xyz.shape[0]), np.float32)
     for t in range(T):
-        off[t], fr[t] = split_delays(steering_vector_spherical(xyz, thetas[t], phis[t]), history)
+        off[t], fr[t] = split_delays(steering_vector_spherical(xyz, thetas[t], phis[t], scale), history)
     return off, fr
 
 
@@ -285,7 +307,8 @@ def quadrant(theta, phi, spread, theta_limit):
     return float(t[0]), nt, nph
 
 
-def monopulse(xyz, theta, phi, window, spread, theta_limit, reference=0.0, index=None):
+def monopulse(xyz, theta, phi, window, spread, theta_limit, reference=0.0, index=None, history=N_SAMPLES, scale=None,
+              n=N_SAMPLES):
     """GradientParticle::findNearby + step() up to the gradient (gradient_ascend.cpp:18-81) for each particle, with the
     oracle's steer / beam: (theta', near_theta, near_phi, q, gradient, error)."""
     theta = np.asarray(theta, np.float64).ravel().copy()
@@ -295,13 +318,27 @@ def monopulse(xyz, theta, phi, window, spread, theta_limit, reference=0.0, index
     grad, err = np.zeros((P, 3)), np.zeros(P)
     for p in range(P):
         theta[p], nth[p], nph[p] = quadrant(theta[p], phi[p], spread, theta_limit)
-        off, fr = steer_tables(xyz, nth[p], nph[p])
+        off, fr = steer_tables(xyz, nth[p], nph[p], history, scale)
         for k in range(4):
-            q[p, k] = particle_beam(window, off[k], fr[k], index=index)
+            q[p, k] = particle_beam(window, off[k], fr[k], index=index, n=n)
         e = np.zeros(1)
         lib().orc_monopulse_gradient(np.ascontiguousarray(q[p]), float(reference), grad[p], e)
         err[p] = e[0]
     return theta, nth, nph, q, grad, err
+
+
+def particle_das_fir(window, offsets, fractions, coeffs, index=None, n=N_SAMPLES):
+    """Particle::das around the FIR variant of delay() (delay.cpp:28-40) for one direction: out [n]; coeffs [n_phases][taps]."""
+    window = np.ascontiguousarray(window, np.float32)
+    coeffs = np.ascontiguousarray(coeffs, np.float32)
+    Cn, W = window.shape
+    index = _idx(index, Cn)
+    offsets = np.ascontiguousarray(offsets, np.int32)
+    assert int(offsets[index].max()) + n + coeffs.shape[1] - 1 <= W, "the window is too short for the FIR taps"
+    out = np.zeros(n, np.float32)
+    lib().orc_particle_das_fir(window, W, n, index, len(index), offsets, np.ascontiguousarray(fractions, np.float32), coeffs,
+                               coeffs.shape[0], coeffs.shape[1], out)
+    return out
 
 
 def mimo_update_fir(window, offsets, fractions, coeffs, index=None, n=N_SAMPLES):
