@@ -28,7 +28,7 @@ SYMBOLS = [
     "bflk_default_config", "bflk_version", "bflk_create", "bflk_destroy", "bflk_last_error",
     "bflk_set_geometry", "bflk_set_tiled_geometry", "bflk_get_geometry", "bflk_set_channel_mask",
     "bflk_set_grid_fov", "bflk_set_grid_tables", "bflk_set_grid_shape", "bflk_set_direction_range", "bflk_get_n_directions",
-    "bflk_get_grid", "bflk_get_tables", "bflk_steer_tables", "bflk_power_map", "bflk_power_map_i32",
+    "bflk_get_grid", "bflk_get_tables", "bflk_steer_tables", "bflk_set_focus", "bflk_power_map", "bflk_power_map_i32",
     "bflk_power_map_batch", "bflk_power_map_batch_submit", "bflk_power_map_batch_wait", "bflk_power_map_batch_i32", "bflk_power_map_batch_i32_dev",
     "bflk_power_map_batch_dev", "bflk_beams_batch_dev", "bflk_power_map_batch_dev_submit", "bflk_power_map_batch_dev_join", "bflk_set_kernel", "bflk_set_channel_split", "bflk_launch_shape", "bflk_get_kernel", "bflk_launch_count", "bflk_enable_timing",
     "bflk_kernel_time_ms", "bflk_fp32_peak_tflops", "bflk_set_window", "bflk_set_window_dev", "bflk_miso", "bflk_miso_dev", "bflk_monopulse", "bflk_set_fir",
@@ -39,7 +39,7 @@ SYMBOLS = [
     "bflk_power_map_batch_sharded_dev", "bflk_power_map_batch_sharded_dev_submit", "bflk_power_map_batch_sharded_dev_join", "bflk_power_map_batch_sharded", "bflk_power_map_batch_sharded_submit", "bflk_power_map_batch_sharded_wait",
     "bflk_group_create", "bflk_group_destroy", "bflk_group_size", "bflk_group_handle", "bflk_group_last_error",
     "bflk_group_set_geometry", "bflk_group_set_tiled_geometry", "bflk_group_set_channel_mask", "bflk_group_set_grid_fov",
-    "bflk_group_set_kernel", "bflk_group_power_map_batch", "bflk_group_power_map_batch_dev", "bflk_group_synchronize",
+    "bflk_group_set_kernel", "bflk_group_set_focus", "bflk_group_power_map_batch", "bflk_group_power_map_batch_dev", "bflk_group_synchronize",
 ]
 
 
@@ -109,6 +109,7 @@ def load_library():
     L.bflk_get_grid.argtypes = [vp, vp, vp]
     L.bflk_get_tables.argtypes = [vp, vp, vp]
     L.bflk_steer_tables.argtypes = [vp, vp, vp, i32, vp, vp]
+    L.bflk_set_focus.argtypes = [vp, f64]
     L.bflk_power_map.argtypes = [vp, vp, vp]
     L.bflk_power_map_i32.argtypes = [vp, vp, vp]
     L.bflk_power_map_batch.argtypes = [vp, vp, i64, i32, vp]
@@ -176,6 +177,7 @@ def load_library():
     L.bflk_group_set_channel_mask.argtypes = [vp, vp, i32]
     L.bflk_group_set_grid_fov.argtypes = [vp, i32, i32, f32]
     L.bflk_group_set_kernel.argtypes = [vp, i32]
+    L.bflk_group_set_focus.argtypes = [vp, f64]
     L.bflk_group_power_map_batch.argtypes = [vp, vp, i64, i32, vp]
     L.bflk_group_power_map_batch_dev.argtypes = [vp, vp, i64, i32, vp]
     L.bflk_group_synchronize.argtypes = [vp]
@@ -388,6 +390,11 @@ class Beamformer:
         fr = np.zeros((T, self.n_channels), np.float32)
         self._check(self._L.bflk_steer_tables(self._h, _ptr(theta), _ptr(phi), T, _ptr(off), _ptr(fr)))
         return off, fr
+
+    def set_focus(self, distance):
+        """Steer every table built from angles (the set_grid_fov grid, steer_tables, miso, monopulse) at the point `distance`
+        metres away in each direction instead of at a plane wave; 0 = far field (bflk_set_focus)."""
+        self._check(self._L.bflk_set_focus(self._h, float(distance)))
 
     def set_kernel(self, which):
         self._check(self._L.bflk_set_kernel(self._h, which))
@@ -708,6 +715,10 @@ class Group:
 
     def size(self):
         return int(self._L.bflk_group_size(self._g))
+
+    def set_focus(self, distance):
+        """Beamformer.set_focus on every device of the group."""
+        self._check(self._L.bflk_group_set_focus(self._g, float(distance)))
 
     def power_map_batch(self, stream, n_frames):
         stream = _np(stream, np.float32)

@@ -49,6 +49,33 @@ def make_stream(xyz, n_samples, sources=DEFAULT_SOURCES, sigma=1e-3, seed=SEED, 
     return out.astype(dtype)
 
 
+def point_source_delays(xyz, theta, phi, r, sample_rate=SAMPLE_RATE, speed=PROPAGATION_SPEED):
+    """Per-element delay in samples of a point source r metres from the origin in direction (theta, phi),
+    (r - |s - p|) * fs / c with s = r u, min-subtracted (float64): the near-field counterpart of arrival_delays, whose
+    plane-wave delay is u.p * fs / c with the same u = (sin theta cos phi, -sin theta sin phi, cos theta)."""
+    xyz = np.asarray(xyz, np.float64)
+    s = r * np.array([np.sin(theta) * np.cos(phi), -np.sin(theta) * np.sin(phi), np.cos(theta)])
+    d = (r - np.linalg.norm(s[None, :] - xyz, axis=1)) * (sample_rate / speed)
+    return d - d.min()
+
+
+def point_source_stream(xyz, n_samples, sources, sigma=1e-3, seed=SEED, t0=0, sample_rate=SAMPLE_RATE,
+                        speed=PROPAGATION_SPEED, dtype=np.float32):
+    """stream[C][n_samples] of point sources (theta, phi, r, f, A) r metres away: sum_j A_j sin(2 pi f_j (t + tau_jc) / fs)
+    + sigma * n_c(t), tau_jc = point_source_delays (the same amplitude at every element)."""
+    xyz = np.asarray(xyz, np.float64)
+    C = xyz.shape[0]
+    t = np.arange(t0, t0 + n_samples, dtype=np.float64)
+    out = np.zeros((C, n_samples), np.float64)
+    for theta, phi, r, f, A in sources:
+        tau = point_source_delays(xyz, theta, phi, r, sample_rate, speed)
+        out += A * np.sin(2.0 * np.pi * f * (t[None, :] + tau[:, None]) / sample_rate)
+    if sigma > 0:
+        rng = np.random.Generator(np.random.Philox(seed))
+        out += sigma * rng.standard_normal((C, n_samples))
+    return out.astype(dtype)
+
+
 def to_wire_i32(stream):
     """float stream[C][n] -> wire frames[n][C] int32 (round(x * 2^23)) with the serpentine column flip
     the FPGA applies (inverse of src/fpga/pipeline.cpp:273-287)."""

@@ -110,6 +110,11 @@ int bflk_set_geometry(bflk_handle *h, const float *xyz, int32_t n_channels) {
         return h->fail(BFLK_ERR_INVALID, "bflk_set_geometry: expected %d channels, got %d", h->cfg.n_channels, n_channels);
     BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
     h->xyz.assign(xyz, xyz + 3 * (size_t)n_channels);
+    h->max_radius = 0.0;
+    for (int c = 0; c < n_channels; c++) {
+        const double x = xyz[3 * c], y = xyz[3 * c + 1], z = xyz[3 * c + 2];
+        h->max_radius = std::max(h->max_radius, std::sqrt((x * x + y * y) + z * z));
+    }
     BFLK_CUDA(h, h->d_xyz.reserve(3 * (size_t)n_channels));
     BFLK_CUDA(h, cudaMemcpyAsync(h->d_xyz.p, h->xyz.data(), h->xyz.size() * sizeof(float), cudaMemcpyHostToDevice, h->stream));
     BFLK_CUDA(h, cudaStreamSynchronize(h->stream));
@@ -184,9 +189,10 @@ static DirTrig make_trig(double theta, double phi) {
 
 static float delay_scale(const bflk_handle *h) { return (float)(h->cfg.sample_rate / h->cfg.propagation_speed); }
 
-// Runs the device table kernel for n directions; results land in d_off/d_frac; *max_delay updated.
+// Runs the device table kernel for n directions, focused at `focus` (0: far field); results land in d_off/d_frac;
+// *max_delay updated.
 static int run_steer_tables(bflk_handle *h, const double *theta, const double *phi, int n, int32_t *d_off, float *d_frac,
-                            int32_t *max_delay) {
+                            int32_t *max_delay, double focus) {
     BFLK_CUDA(h, h->p_trig.reserve(n));
     BFLK_CUDA(h, h->d_trig.reserve(n));
     BFLK_CUDA(h, h->d_misc.reserve(4));
@@ -195,7 +201,7 @@ static int run_steer_tables(bflk_handle *h, const double *theta, const double *p
     BFLK_CUDA(h, cudaMemcpyAsync(h->d_trig.p, h->p_trig.p, n * sizeof(DirTrig), cudaMemcpyHostToDevice, h->stream));
     BFLK_CUDA(h, cudaMemsetAsync(h->d_misc.p, 0, 4 * sizeof(int32_t), h->stream));
     BFLK_CUDA(h, launch_steer_tables(h->d_trig.p, n, h->d_xyz.p, h->cfg.n_channels, delay_scale(h), h->cfg.history, d_off,
-                                     d_frac, h->d_misc.p, h->stream));
+                                     d_frac, h->d_misc.p, focus, h->stream));
     h->launches++;
     BFLK_CUDA(h, cudaMemcpyAsync(h->p_misc.p, h->d_misc.p, sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
     BFLK_CUDA(h, cudaStreamSynchronize(h->stream));
@@ -209,11 +215,20 @@ static int check_delay_range(bflk_handle *h, int max_delay, const char *who) {
     return BFLK_OK;
 }
 
+// A focus point must lie outside the array: every element nearer to the origin than `focus` (0: far field, always fine).
+static int check_focus(bflk_handle *h, double focus, const char *who) {
+    if (focus > 0.0 && h->have_geometry && !(focus > h->max_radius))
+        return h->fail(BFLK_ERR_INVALID, "%s: focus distance %g m is not beyond the array (an element lies %g m from the origin)",
+                       who, focus, h->max_radius);
+    return BFLK_OK;
+}
+
 int bflk_set_grid_fov(bflk_handle *h, int32_t rows, int32_t cols, float fov_deg) {
     if (!h) return BFLK_ERR_INVALID;
     if (!h->have_geometry) return h->fail(BFLK_ERR_STATE, "bflk_set_grid_fov: set the geometry first");
     if (rows <= 0 || cols <= 0 || !(fov_deg > 0.f) || fov_deg > 180.f)
         return h->fail(BFLK_ERR_INVALID, "bflk_set_grid_fov: invalid grid %d x %d fov %g", rows, cols, (double)fov_deg);
+    if (int rc = check_focus(h, h->focus, "bflk_set_grid_fov")) return rc;
     BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
     const int D = rows * cols;
     std::vector<double> theta(D), phi(D);
@@ -243,7 +258,7 @@ int bflk_set_grid_fov(bflk_handle *h, int32_t rows, int32_t cols, float fov_deg)
     BFLK_CUDA(h, h->d_off.reserve(DC));
     BFLK_CUDA(h, h->d_frac.reserve(DC));
     int32_t max_delay = 0;
-    int rc = run_steer_tables(h, theta.data(), phi.data(), D, h->d_off.p, h->d_frac.p, &max_delay);
+    int rc = run_steer_tables(h, theta.data(), phi.data(), D, h->d_off.p, h->d_frac.p, &max_delay, h->focus);
     if (rc) return rc;
     invalidate_tables(h);
     if ((rc = check_delay_range(h, max_delay, "bflk_set_grid_fov"))) return rc;
@@ -356,17 +371,46 @@ int bflk_steer_tables(bflk_handle *h, const double *theta, const double *phi, in
     if (!h) return BFLK_ERR_INVALID;
     if (!h->have_geometry) return h->fail(BFLK_ERR_STATE, "bflk_steer_tables: set the geometry first");
     if (!theta || !phi || n_targets <= 0) return h->fail(BFLK_ERR_INVALID, "bflk_steer_tables: null / empty direction list");
+    if (int rc = check_focus(h, h->focus, "bflk_steer_tables")) return rc;
     BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
     const size_t TC = (size_t)n_targets * h->cfg.n_channels;
     BFLK_CUDA(h, h->d_soff.reserve(TC));
     BFLK_CUDA(h, h->d_sfrac.reserve(TC));
     int32_t max_delay = 0;
-    int rc = run_steer_tables(h, theta, phi, n_targets, h->d_soff.p, h->d_sfrac.p, &max_delay);
+    int rc = run_steer_tables(h, theta, phi, n_targets, h->d_soff.p, h->d_sfrac.p, &max_delay, h->focus);
     if (rc) return rc;
     if (offsets) BFLK_CUDA(h, cudaMemcpyAsync(offsets, h->d_soff.p, TC * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
     if (fractions) BFLK_CUDA(h, cudaMemcpyAsync(fractions, h->d_sfrac.p, TC * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
     BFLK_CUDA(h, cudaStreamSynchronize(h->stream));
     return check_delay_range(h, max_delay, "bflk_steer_tables");
+}
+
+int bflk_set_focus(bflk_handle *h, double distance_m) {
+    if (!h) return BFLK_ERR_INVALID;
+    if (!(distance_m >= 0.0) || std::isinf(distance_m))
+        return h->fail(BFLK_ERR_INVALID, "bflk_set_focus: distance %g m (0 = far field, else a finite distance)", distance_m);
+    if (int rc = check_focus(h, distance_m, "bflk_set_focus")) return rc;
+    if (h->have_grid && !h->theta.empty()) {
+        // a bflk_set_grid_fov grid: its tables again, at the new focus, built aside so that a refusal leaves the old ones
+        BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
+        const size_t DC = (size_t)h->n_dir * h->cfg.n_channels;
+        DevBuf<int32_t> off;
+        DevBuf<float> frac;
+        BFLK_CUDA(h, off.reserve(DC));
+        BFLK_CUDA(h, frac.reserve(DC));
+        int32_t max_delay = 0;
+        int rc = run_steer_tables(h, h->theta.data(), h->phi.data(), h->n_dir, off.p, frac.p, &max_delay, distance_m);
+        if (rc) return rc;
+        if ((rc = check_delay_range(h, max_delay, "bflk_set_focus"))) return rc;
+        BFLK_CUDA(h, cudaEventSynchronize(h->caller_event));   // a caller's stream may still read the old tables
+        std::swap(h->d_off, off);
+        std::swap(h->d_frac, frac);
+        h->max_delay = max_delay;
+        h->drop_kernel_tables();
+        h->last_map_on_device = false;
+    }
+    h->focus = distance_m;
+    return BFLK_OK;
 }
 
 // ---- power map ---------------------------------------------------------------------------------------------
@@ -1215,6 +1259,7 @@ static int miso_launch(bflk_handle *h, const double *theta, const double *phi, i
     a.power = power_dev;
     a.norm = static_cast<float>(N);  // Particle::beam: power_accumulator /= N_SAMPLES, particle.cpp:79
     a.error_flag = flag_dev;
+    a.focus = h->focus;
     a.epoch = ++h->miso_epoch;
     if (h->miso_epoch == 0x7fffffff) h->miso_epoch = 0;
     BFLK_CUDA(h, launch_das_miso(a, st));
@@ -1240,7 +1285,7 @@ static int miso_dev(bflk_handle *h, const double *theta, const double *phi, int3
     BFLK_CUDA(h, h->d_sfrac.reserve(TC));
     BFLK_CUDA(h, cudaEventSynchronize(h->caller_event));
     int32_t max_delay = 0;
-    int rc = run_steer_tables(h, theta, phi, n_targets, h->d_soff.p, h->d_sfrac.p, &max_delay);  // Particle::steer
+    int rc = run_steer_tables(h, theta, phi, n_targets, h->d_soff.p, h->d_sfrac.p, &max_delay, h->focus);  // Particle::steer
     if (rc) return rc;
     if ((rc = check_delay_range(h, max_delay, "bflk_miso"))) return rc;
     if (n_samples < h->cfg.history + N + h->fir_taps - 1)
@@ -1273,6 +1318,7 @@ int bflk_miso_dev(bflk_handle *h, const double *theta, const double *phi, int32_
     if (!h->have_geometry) return h->fail(BFLK_ERR_STATE, "bflk_miso: set the geometry first");
     if (!theta || !phi || n_targets <= 0 || (!window_dev && !h->resident_window))
         return h->fail(BFLK_ERR_INVALID, "bflk_miso: null / empty arguments (no window given and none resident)");
+    if (int rc = check_focus(h, h->focus, "bflk_miso")) return rc;
     BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
     cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : h->stream;
     if (window_dev) return miso_dev(h, theta, phi, n_targets, window_dev, h->cfg.window_len, h->cfg.window_len, audio_dev, power_dev, st);
@@ -1285,6 +1331,7 @@ int bflk_miso(bflk_handle *h, const double *theta, const double *phi, int32_t n_
     if (!h->have_geometry) return h->fail(BFLK_ERR_STATE, "bflk_miso: set the geometry first");
     if (!theta || !phi || n_targets <= 0 || (!window && !h->resident_window))
         return h->fail(BFLK_ERR_INVALID, "bflk_miso: null / empty arguments (no window given and none resident)");
+    if (int rc = check_focus(h, h->focus, "bflk_miso")) return rc;
     BFLK_CUDA(h, cudaSetDevice(h->cfg.device));
     const int N = h->cfg.frame_len;
     const size_t n_in = (size_t)h->cfg.n_channels * h->cfg.window_len;

@@ -216,6 +216,8 @@ struct bflk_handle {
     // geometry + mask (host copies are the source of truth; device copies feed the table kernels)
     bool have_geometry = false;
     std::vector<float> xyz;      // [C][3]
+    double max_radius = 0.0;     // largest |p| of the geometry: a focus must lie beyond it
+    double focus = 0.0;          // bflk_set_focus: distance of the point every angle-built table steers at, 0 = far field
     std::vector<int32_t> index;  // [usable]
     bflk::DevBuf<float> d_xyz;
     bflk::DevBuf<int32_t> d_index;
@@ -347,8 +349,9 @@ namespace bflk {
 // ---- tables.cu --------------------------------------------------------------------------------------
 // delays -> (offset, fraction) for n_dir directions given their trig; also returns the largest integer
 // delay through d_maxdelay (device int, atomically maxed).  off / frac are [n_dir][C].
+// focus > 0: the delays of a point source at that distance (bflk_set_focus) instead of a plane wave
 cudaError_t launch_steer_tables(const DirTrig *d_trig, int n_dir, const float *d_xyz, int C, float k_scale,
-                                int history, int32_t *d_off, float *d_frac, int32_t *d_maxdelay, cudaStream_t st);
+                                int history, int32_t *d_off, float *d_frac, int32_t *d_maxdelay, double focus, cudaStream_t st);
 cudaError_t launch_offset_range(const int32_t *d_off, size_t n, int32_t *d_maxoff, int32_t *d_minoff, cudaStream_t st);
 // tile tables for directions [first, first+count) of a rows x cols grid, 2x2 direction tiles.
 cudaError_t launch_build_tiles(const int32_t *d_off, const float *d_frac, int C, const int32_t *d_index, int usable,
@@ -402,6 +405,7 @@ struct MisoArgs {
     float *frac_out;
     int n_inline;            // n_targets when the directions are in trig_inline, else 0
     DirTrig trig_inline[kMisoInline];
+    double focus;            // > 0: tables of a point source at this distance (bflk_set_focus), 0: far field
 };
 cudaError_t launch_das_miso(const MisoArgs &a, cudaStream_t st);
 int das_miso_slices(int frame_len);

@@ -27,6 +27,8 @@ constexpr int kMisoThreads = 64;            // samples per CTA: 62 high-pass out
 constexpr int kMisoOut = kMisoThreads - 2;
 constexpr int kBatch = 32;                  // channels per register set
 
+// FOCUS: the tables of a point source at a.focus (focus_z); the far-field instantiation is the kernel as it was before
+template <bool FOCUS>
 __global__ void __launch_bounds__(kMisoThreads) miso_kernel(MisoArgs a) {
     extern __shared__ __align__(8) unsigned char s_raw[];
     __shared__ float s_red[kMisoThreads / 32];
@@ -42,7 +44,7 @@ __global__ void __launch_bounds__(kMisoThreads) miso_kernel(MisoArgs a) {
     // ---- Particle::steer: steering_vector_spherical + split (particle.cpp:37-49), all C elements for the minimum ----
     float mn = INFINITY;
     for (int c = threadIdx.x; c < a.C; c += kMisoThreads) {
-        const float del = steer_delay(trig, a.xyz, c, a.k_scale);
+        const float del = steer_delay<FOCUS>(trig, a.xyz, c, a.k_scale, a.focus);
         s_del[c] = del;
         mn = fminf(mn, del);
     }
@@ -138,8 +140,9 @@ cudaError_t launch_das_miso(const MisoArgs &a, cudaStream_t st) {
     if (a.n_targets <= 0 || a.n_frames <= 0) return cudaSuccess;
     const size_t smem = (size_t)a.usable * (sizeof(long long) + sizeof(float)) + (size_t)a.C * sizeof(float);
     if (smem > 200 * 1024) return cudaErrorInvalidConfiguration;
+    auto kernel = a.focus > 0.0 ? miso_kernel<true> : miso_kernel<false>;
     if (smem > 48 * 1024) {   // beyond the default limit (thousands of channels): per device, so set per launch
-        cudaError_t e = cudaFuncSetAttribute(miso_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
     }
     const int n_slices = das_miso_slices(a.frame_len);
@@ -152,7 +155,7 @@ cudaError_t launch_das_miso(const MisoArgs &a, cudaStream_t st) {
         if (a.partial) s.partial = a.partial + (size_t)b0 * a.n_targets * n_slices;
         if (a.counters) s.counters = a.counters + (size_t)b0 * a.n_targets;
         dim3 grid(a.n_targets, n_slices, s.n_frames);
-        miso_kernel<<<grid, kMisoThreads, smem, st>>>(s);
+        kernel<<<grid, kMisoThreads, smem, st>>>(s);
         cudaError_t e = cudaGetLastError();
         if (e != cudaSuccess) return e;
     }

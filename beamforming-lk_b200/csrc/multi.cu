@@ -732,6 +732,7 @@ int bflk_group_set_tiled_geometry(bflk_group *g, int32_t n_tiles, const float *o
 int bflk_group_set_channel_mask(bflk_group *g, const int32_t *index, int32_t usable) { BFLK_FORALL(g, bflk_set_channel_mask(h, index, usable)); }
 int bflk_group_set_grid_fov(bflk_group *g, int32_t rows, int32_t cols, float fov_deg) { BFLK_FORALL(g, bflk_set_grid_fov(h, rows, cols, fov_deg)); }
 int bflk_group_set_kernel(bflk_group *g, int32_t which) { BFLK_FORALL(g, bflk_set_kernel(h, which)); }
+int bflk_group_set_focus(bflk_group *g, double distance_m) { BFLK_FORALL(g, bflk_set_focus(h, distance_m)); }
 
 int bflk_group_power_map_batch(bflk_group *g, const float *stream, int64_t n_samples, int32_t n_frames, float *power_out) {
     if (!g || g->hs.empty()) return BFLK_ERR_INVALID;

@@ -11,17 +11,19 @@
 
 namespace bflk {
 
+// FOCUS: the delays of a point source at distance `focus` (focus_z) instead of a plane wave (steer_z)
+template <bool FOCUS>
 __global__ void __launch_bounds__(128) steer_tables_kernel(const DirTrig *__restrict__ trig, const float *__restrict__ xyz,
                                                            int C, float k_scale, int history, int32_t *__restrict__ off,
-                                                           float *__restrict__ frac, int32_t *__restrict__ maxdelay) {
+                                                           float *__restrict__ frac, int32_t *__restrict__ maxdelay,
+                                                           double focus) {
     extern __shared__ float s_del[];
     __shared__ float s_red[4];
     const int d = blockIdx.x;
     const DirTrig t = trig[d];
     float mn = INFINITY;
     for (int c = threadIdx.x; c < C; c += blockDim.x) {
-        float z = steer_z(t, xyz[3 * c + 0], xyz[3 * c + 1], xyz[3 * c + 2]);
-        float del = __fmul_rn(z, k_scale);  // compute_delays: row(Z) * float(SAMPLE_RATE / PROPAGATION_SPEED)
+        float del = steer_delay<FOCUS>(t, xyz, c, k_scale, focus);  // compute_delays: row(Z) * float(SAMPLE_RATE / PROPAGATION_SPEED)
         s_del[c] = del;
         mn = fminf(mn, del);
     }
@@ -44,9 +46,10 @@ __global__ void __launch_bounds__(128) steer_tables_kernel(const DirTrig *__rest
 }
 
 cudaError_t launch_steer_tables(const DirTrig *d_trig, int n_dir, const float *d_xyz, int C, float k_scale, int history,
-                                int32_t *d_off, float *d_frac, int32_t *d_maxdelay, cudaStream_t st) {
+                                int32_t *d_off, float *d_frac, int32_t *d_maxdelay, double focus, cudaStream_t st) {
     if (n_dir <= 0) return cudaSuccess;
-    steer_tables_kernel<<<n_dir, 128, C * sizeof(float), st>>>(d_trig, d_xyz, C, k_scale, history, d_off, d_frac, d_maxdelay);
+    auto kernel = focus > 0.0 ? steer_tables_kernel<true> : steer_tables_kernel<false>;
+    kernel<<<n_dir, 128, C * sizeof(float), st>>>(d_trig, d_xyz, C, k_scale, history, d_off, d_frac, d_maxdelay, focus);
     return cudaGetLastError();
 }
 

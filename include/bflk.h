@@ -16,6 +16,8 @@
  *   bflk_set_grid_fov               MIMOWorker::computeDelayLUT (src/dsp/mimo.cpp:20-59)
  *   bflk_set_grid_tables            the same LUT supplied by the caller (offsetDelays / fractionalDelays, mimo.h:86-89)
  *   bflk_steer_tables               Particle::steer (src/dsp/particle.cpp:37-49)
+ *   bflk_set_focus                  (no reference counterpart: the reference steers at plane waves only) the tables of
+ *                                   all of the above focused at a point at a given distance
  *   bflk_power_map*                 MIMOWorker::update (src/dsp/mimo.cpp:97-151) -> powerdB
  *   bflk_beams_batch_dev, bflk_session_beams   the same, with the delayed sums out[] of every direction (mimo.cpp:121-130)
  *   bflk_power_map_batch*_submit / _wait / _join   the same in continuous operation (the reference's worker loop,
@@ -106,6 +108,22 @@ int bflk_get_tables(const bflk_handle *h, int32_t *offsets, float *fractions);  
 /* Particle::steer for T directions: offsets / fractions [T][C], computed by the device table kernel. */
 int bflk_steer_tables(bflk_handle *h, const double *theta, const double *phi, int32_t n_targets,
                       int32_t *offsets, float *fractions);
+/* Near-field steering: every table the handle builds from angles steers at the point distance_m metres from the origin of
+ * the geometry's frame in that direction, instead of at a plane wave from it.  For direction (theta, phi), with cz, sz,
+ * cy, sy the floats of the far-field rotation (cos / sin of float(phi) and of -float(theta)), u = (-sy cz, sy sz, cy) in
+ * double and element p promoted to double, the element's z'' becomes
+ *     z = (2 r u.p - p.p) / (r + |r u - p|)    (= r - |r u - p|, without the cancellation),
+ * every double operation rounded where it is written ((a0 b0 + a1 b1) + a2 b2 for dot products), then zf = float(z);
+ * from zf on the float path is the far-field one (times the delay scale, minus the minimum, integer and fraction split).
+ * As distance_m grows the tables tend to the far-field ones.  distance_m = 0 is the far field (the default): the tables
+ * are then bit-identical to those of a handle that never called this.
+ * The focus applies to: the bflk_set_grid_fov grid (rebuilt at once when one is set; later bflk_set_grid_fov calls use
+ * the focus), bflk_steer_tables, bflk_miso and bflk_miso_dev (FIR form included) and bflk_monopulse.  Tables the caller
+ * supplies (bflk_set_grid_tables) are not touched, and grid angles (bflk_get_grid, Target records) do not change.
+ * BFLK_ERR_INVALID: distance_m negative, NaN or infinite, or not larger than the largest |p| of the geometry (the point
+ * would lie inside the array); the table calls above check that again after a geometry change.  BFLK_ERR_RANGE: a
+ * focused delay of the grid exceeds the history.  A refused call changes nothing: the previous focus and tables stay. */
+int bflk_set_focus(bflk_handle *h, double distance_m);
 
 /* ---- full-grid power map (MIMO) ------------------------------------------------------------------- */
 /* window[C][W] channel-major snapshot exactly as read_stream() produces it (oldest sample first);
@@ -294,6 +312,7 @@ int bflk_group_set_tiled_geometry(bflk_group *g, int32_t n_tiles, const float *o
 int bflk_group_set_channel_mask(bflk_group *g, const int32_t *index, int32_t usable);
 int bflk_group_set_grid_fov(bflk_group *g, int32_t rows, int32_t cols, float fov_deg);
 int bflk_group_set_kernel(bflk_group *g, int32_t which);
+int bflk_group_set_focus(bflk_group *g, double distance_m);
 /* stream[C][n_samples] on the host -> power_out[B][D] on the host; all devices of the group work on it. */
 int bflk_group_power_map_batch(bflk_group *g, const float *stream, int64_t n_samples, int32_t n_frames, float *power_out);
 /* stream_dev[i] / power_all_dev[i]: the batch and the [B][D] result on device i.  Asynchronous on each member's stream. */
